@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU, torchrun for N > 1)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port)
+    python bench.py --gpus 1 --steps K --dump-outputs DIR    # + the last timed step's codebook and loss as DIR/*.npy
 
 Headline workload at every N (BASELINE.json `metric` = patches/sec BMU+update; configs[3], C4): ONE SOM training step
 of /root/reference/train_codebook.py:225-249 -- BMU search + neighbourhood-weighted update + Adam -- at P=4 (D=64),
@@ -184,7 +185,8 @@ def _max_over_ranks(ms, dev, world):
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# the reference arm: the reference's own CPU implementation of the step (oracle port), bounded sample
+# the reference arm: the reference's own CPU implementation of the step (oracle port) on a 128-fmap sample of the
+# batch, for as many steps as --steps asks
 # ---------------------------------------------------------------------------------------------------------------
 def _cpu_reference_step(steps, warmup, sample_fmaps=128, min_seconds=0.0):
     """train_codebook.py:225-249 on the host cores at the C4 shape, 8192 patches per step (the reference's dense N x K
@@ -216,7 +218,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 40))
+    steps = args.steps
     base, s_per_step = _cpu_reference_step(steps, args.warmup)
     line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT,
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": s_per_step * 1e3,
@@ -282,6 +284,10 @@ def run_headline(args, dev, world, rank, peaks):
     ms_step = _max_over_ranks(e0.elapsed_time(e1), dev, world) / args.steps
     n_global = C4["n_fmaps"] * C4["seq"]
     value = n_global / (ms_step * 1e-3)
+    # what a caller holds after the last timed step: the codebook it updated in place and the loss it returned (read
+    # here, before the end-to-end run below trains the same codebook further)
+    outputs = {"codebook_weight": cb.codebook.weight.detach().cpu().numpy(),
+               "loss": loss.detach().reshape(1).cpu().numpy()} if args.dump_outputs else None
     loss = float(loss)
     assert loss == loss and 0.0 < loss < float("inf"), f"implausible loss {loss}"
 
@@ -426,7 +432,7 @@ def run_headline(args, dev, world, rank, peaks):
                 "algorithmic_flops_per_patch": 2 * k * d, "algorithmic_bytes_per_patch": 4 * d + 8,
                 "hbm_frac": (4 * d + 8) * n_local / (parts["bmu"] * 1e-3) / 1e9 / peaks["hbm_gbs"],
                 "tensor_pipe_active_pct_ncu": pipe_pct, "note": mode or None}
-    head = {"value": value, "ms_per_step": ms_step, "loss": loss, "clocks": clk.summary(), "e2e": e2e,
+    head = {"value": value, "ms_per_step": ms_step, "loss": loss, "outputs": outputs, "clocks": clk.summary(), "e2e": e2e,
             "gpu_launches": launches_per_step * args.steps, "roofline": roofline, "breakdown": breakdown,
             "details": {"fmaps_per_rank": share, "patches_per_rank": n_local, "rotation_buffers": n_rot,
                         "launches_per_step": launches_per_step,
@@ -603,10 +609,17 @@ def main():
                     help="peer tail: W~ = T @ W per slice + multicast, or the whole filter on every rank")
     ap.add_argument("--tail", default="auto", choices=["auto", "peer", "nccl"],
                     help="data-parallel tail: sharded over NVSwitch multicast peer memory, or NCCL all-reduce + replicated")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed (the codebook it updated and "
+                         "its loss) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of our arm's step; --impl reference has none to write")
         run_reference(args)
         return
 
@@ -632,6 +645,12 @@ def main():
 
     head, tr, cb, xs = run_headline(args, dev, world, rank, peaks)
     _log("headline + breakdown done")
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in head["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
+        _log(f"outputs of the last timed step written to {args.dump_outputs}")
 
     extra = {}
     if not args.no_extra:

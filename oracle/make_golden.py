@@ -39,6 +39,39 @@ def _build(Codebook, weight, patch_dim, image_dim, channels, rng):
     return cb
 
 
+# reference outputs that are stored as a sample of their rows when a record would not fit GOLDEN_BYTES
+CASE_OUTPUTS = ("patches", "quant_gauss", "quant_hard", "forward_gauss", "quant_image", "grad", "weight_after_step")
+GOLDEN_BYTES = 900_000
+
+
+def keep_sampled_rows(rec, names, seed=0):
+    """Fit a record under GOLDEN_BYTES of tensor data.  Inputs and small outputs stay whole; each output in ``names``
+    (a tensor, or a dict of same-shaped tensors) keeps a fixed, seeded sample of the rows of t.reshape(-1, t.shape[-1]),
+    as many as fit beside the rest.  The rows go to rec["sampled_rows"][name], the full shape to rec["shapes"][name]
+    (tests/_helpers.golden_rows compares on those rows)."""
+    def parts(v):
+        return list(v.values()) if isinstance(v, dict) else [v]
+
+    def nbytes(v):
+        return sum(t.numel() * t.element_size() for t in parts(v) if isinstance(t, torch.Tensor))
+    fixed = sum(nbytes(v) for k, v in rec.items() if k not in names and isinstance(v, (torch.Tensor, dict)))
+    frac = (GOLDEN_BYTES - fixed) / sum(nbytes(rec[n]) for n in names)
+    if frac >= 1.0:
+        return rec
+    rec = dict(rec, sampled_rows={}, shapes={})
+    for n in names:
+        shape = tuple(parts(rec[n])[0].shape)
+        n_rows = parts(rec[n])[0].numel() // shape[-1]
+        rows = torch.randperm(n_rows, generator=torch.Generator().manual_seed(seed))[:max(1, int(n_rows * frac))]
+        rows = rows.sort().values
+
+        def pick(t):
+            return t.reshape(-1, shape[-1])[rows].clone()
+        rec[n] = {k: pick(t) for k, t in rec[n].items()} if isinstance(rec[n], dict) else pick(rec[n])
+        rec["sampled_rows"][n], rec["shapes"][n] = rows, shape
+    return rec
+
+
 def fresh_weight(k, d, seed=0):
     """The reference init U(-1/K, 1/K) (models/Codebook.py:44-46) under a fixed seed."""
     torch.manual_seed(seed)
@@ -90,7 +123,7 @@ def main():
         opt.step()
         rec["loss"] = loss.detach().clone()
         rec["weight_after_step"] = cb.codebook.weight.detach().clone()
-        torch.save(rec, os.path.join(out_dir, f"case_{name}.pt"))
+        torch.save(keep_sampled_rows(rec, CASE_OUTPUTS), os.path.join(out_dir, f"case_{name}.pt"))
         print(name, "patches", rec["bmu"].numel(), "loss", float(loss.detach()))
 
     # ---- tie-break: duplicated rows must resolve to the lowest index --------------------
@@ -126,10 +159,11 @@ def main():
         ranges.append(cb.neighbourhood_range)
         if step + 1 in (1, 10, 50, 100):
             snaps[step + 1] = cb.codebook.weight.detach().clone()
-    torch.save({"weight0": wt, "patch_dim": pd, "image_dim": (32, 32), "channels": 4,
-                "range0": rng, "lr": 1e-4, "neighbourhood_step": neighbourhood_step,
-                "losses": torch.tensor(losses, dtype=torch.float64), "ranges": ranges,
-                "weights": snaps}, os.path.join(out_dir, "run_c1_trained_100.pt"))
+    torch.save(keep_sampled_rows({"weight0": wt, "patch_dim": pd, "image_dim": (32, 32), "channels": 4,
+                                  "range0": rng, "lr": 1e-4, "neighbourhood_step": neighbourhood_step,
+                                  "losses": torch.tensor(losses, dtype=torch.float64), "ranges": ranges,
+                                  "weights": snaps}, ("weights",)),
+               os.path.join(out_dir, "run_c1_trained_100.pt"))
     print("100-step run: loss", losses[0], "->", losses[-1], "range", ranges[-1])
 
     # ---- histogram + prune (prune_codebook.py:129-162) ----------------------------------

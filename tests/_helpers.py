@@ -20,6 +20,20 @@ def load_golden(fname):
     return torch.load(os.path.join(GOLDEN, fname), weights_only=True)
 
 
+def golden_rows(rec, name, *got):
+    """The given tensors, each shaped like the reference output ``name``, and that stored output, on the rows the
+    golden file keeps: a large output is stored as a fixed, seeded sample of the rows of t.reshape(-1, t.shape[-1])
+    (oracle/make_golden.keep_sampled_rows), a small one whole.  Returns (*got, want)."""
+    rows = rec.get("sampled_rows", {}).get(name)
+    if rows is None:
+        return (*got, rec[name])
+    out = []
+    for t in got:
+        assert tuple(t.shape) == tuple(rec["shapes"][name]), f"{name}: shape {tuple(t.shape)}"
+        out.append(t.reshape(-1, t.shape[-1])[rows.to(t.device)])
+    return (*out, rec[name])
+
+
 def flat_patches(x, patch_dim):
     p = patchify(x, patch_dim)
     return p.reshape(-1, p.shape[-1])

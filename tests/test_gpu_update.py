@@ -10,7 +10,7 @@ from somcb import ops
 from oracle import neighbourhood_two_var
 from oracle.step_oracle import synthetic_fmaps
 from _helpers import (CASES, assert_bmu_parity, assert_close_norm, assert_weights_parity, flat_patches,
-                      fp64_truth_step, load_case, load_golden, rel_fro)
+                      fp64_truth_step, golden_rows, load_case, load_golden, rel_fro)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -206,12 +206,12 @@ def test_quantize_paths_match_reference(name, monkeypatch):
         if not torch.equal(bmu.cpu(), rec["bmu"]):
             assert_bmu_parity(bmu, rec["bmu"], flat_patches(rec["x"], rec["patch_dim"]), rec["weight"])
             _teacher_force(monkeypatch, rec)
-        assert torch.equal(cb.get_quantized_patches(x, use_gaussian=False).cpu(), rec["quant_hard"])
-        assert torch.equal(cb.get_quantized_image(rec["bmu_reshaped"].to(DEV)).cpu(), rec["quant_image"])
+        assert torch.equal(*golden_rows(rec, "quant_hard", cb.get_quantized_patches(x, use_gaussian=False).cpu()))
+        assert torch.equal(*golden_rows(rec, "quant_image", cb.get_quantized_image(rec["bmu_reshaped"].to(DEV)).cpu()))
         qi = cb.get_quantized_image(rec["bmu_reshaped"].to(DEV), unpatchify_input=False)
-        assert torch.equal(qi.cpu(), rec["quant_hard"])
-        assert_close_norm(cb.get_quantized_patches(x).cpu(), rec["quant_gauss"], 1e-5, "quant_gauss")
-        assert_close_norm(cb(x).cpu(), rec["forward_gauss"], 1e-5, "forward")
+        assert torch.equal(*golden_rows(rec, "quant_hard", qi.cpu()))
+        assert_close_norm(*golden_rows(rec, "quant_gauss", cb.get_quantized_patches(x).cpu()), 1e-5, "quant_gauss")
+        assert_close_norm(*golden_rows(rec, "forward_gauss", cb(x).cpu()), 1e-5, "forward")
 
 
 @pytest.mark.parametrize("name", CASES)
@@ -234,12 +234,15 @@ def test_dropin_autograd_step_matches_reference(name, monkeypatch):
     assert not torch.isnan(loss)
     loss.backward()
     grad = cb.codebook.weight.grad
-    assert grad is not None and grad.shape == rec["grad"].shape
+    assert grad is not None
+    g, g_ref = golden_rows(rec, "grad", grad)
+    assert g.shape == g_ref.shape
     opt.step()
     assert_close_norm(loss, rec["loss"], 1e-5, "loss")
-    assert_close_norm(grad, rec["grad"], 1e-5, "grad")
+    assert_close_norm(g, g_ref, 1e-5, "grad")
     w_truth, _, _ = fp64_truth_step(rec)
-    assert_weights_parity(cb.codebook.weight.detach(), rec["weight_after_step"], w_truth)
+    w, w_truth, w_ref = golden_rows(rec, "weight_after_step", cb.codebook.weight.detach(), w_truth)
+    assert_weights_parity(w, w_ref, w_truth)
 
 
 @pytest.mark.parametrize("name", CASES)
@@ -251,7 +254,8 @@ def test_fused_trainer_step_teacher_forced(name):
     loss = tr.step(rec["x"].to(DEV), bmu=rec["bmu"].to(DEV))
     assert_close_norm(loss, rec["loss"], 1e-5, "loss")
     w_truth, _, _ = fp64_truth_step(rec)
-    assert_weights_parity(cb.codebook.weight.detach(), rec["weight_after_step"], w_truth)
+    w, w_truth, w_ref = golden_rows(rec, "weight_after_step", cb.codebook.weight.detach(), w_truth)
+    assert_weights_parity(w, w_ref, w_truth)
 
 
 @pytest.mark.parametrize("path", ["fused", "dropin"])
@@ -282,8 +286,8 @@ def test_free_run_100_steps_c1(path):
         assert abs(float(loss) - ref_loss) <= 1e-5 * abs(ref_loss), f"loss at step {step}"
         assert cb.neighbourhood_range == run["ranges"][step]
         if step + 1 in run["weights"]:
-            assert_close_norm(cb.codebook.weight.detach(), run["weights"][step + 1], 1e-5,
-                              f"weights@{step + 1}")
+            w, snaps = golden_rows(run, "weights", cb.codebook.weight.detach())
+            assert_close_norm(w, snaps[step + 1], 1e-5, f"weights@{step + 1}")
 
 
 def test_adam_kernel_matches_torch_adam():

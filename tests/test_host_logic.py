@@ -6,7 +6,7 @@ import torch
 import oracle
 import somcb
 from somcb import ops
-from _helpers import (CASES, assert_close_norm, assert_weights_parity, fp64_truth_step, load_case,
+from _helpers import (CASES, assert_close_norm, assert_weights_parity, fp64_truth_step, golden_rows, load_case,
                       load_golden)
 import _oracle_ops
 
@@ -114,7 +114,8 @@ def test_trainer_orchestration_matches_reference_step(name):
     loss = tr.step(rec["x"], bmu=rec["bmu"])
     assert_close_norm(loss, rec["loss"], 1e-6, "loss")
     w_truth, _, _ = fp64_truth_step(rec)
-    assert_weights_parity(cb.codebook.weight.detach(), rec["weight_after_step"], w_truth)
+    w, w_truth, w_ref = golden_rows(rec, "weight_after_step", cb.codebook.weight.detach(), w_truth)
+    assert_weights_parity(w, w_ref, w_truth)
     assert tr.global_steps == 1 and tr.t == 1
 
 

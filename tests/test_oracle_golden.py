@@ -7,7 +7,8 @@ import oracle
 from oracle.step_oracle import (AdamState, closed_form_step, factorised_grad, histogram_prune,
                                 make_oracle_codebook, make_reference_optimizer, reference_step,
                                 synthetic_fmaps, trained_like_codebook)
-from _helpers import CASES, assert_bmu_parity, assert_close_norm, flat_patches, load_case, load_golden
+from _helpers import (CASES, assert_bmu_parity, assert_close_norm, flat_patches, golden_rows, load_case,
+                      load_golden)
 
 
 def _cb(rec):
@@ -22,18 +23,19 @@ def test_oracle_forward_matches_reference(name):
     x = rec["x"]
     flat = flat_patches(x, rec["patch_dim"])
     with torch.no_grad():
-        assert torch.equal(oracle.patchify(x, rec["patch_dim"]), rec["patches"])
-        assert torch.equal(oracle.unpatchify(rec["patches"], rec["image_dim"], rec["patch_dim"]), x)
+        patches = oracle.patchify(x, rec["patch_dim"])
+        assert torch.equal(*golden_rows(rec, "patches", patches))
+        assert torch.equal(oracle.unpatchify(patches, rec["image_dim"], rec["patch_dim"]), x)
         bmu = cb.get_patches_bmu(x)
         # same torch build -> normally bit-identical; a different BLAS thread count may move a
         # near-tie, which the parity rule still bounds
         assert_bmu_parity(bmu, rec["bmu"], flat, rec["weight"])
         assert cb.get_patches_bmu(x, reshape=True).shape == rec["bmu_reshaped"].shape
         if torch.equal(bmu, rec["bmu"]):
-            assert_close_norm(cb.get_quantized_patches(x, True), rec["quant_gauss"], 1e-6, "quant_gauss")
-            assert torch.equal(cb.get_quantized_patches(x, False), rec["quant_hard"])
-            assert_close_norm(cb(x), rec["forward_gauss"], 1e-6, "forward")
-            assert torch.equal(cb.get_quantized_image(rec["bmu_reshaped"]), rec["quant_image"])
+            assert_close_norm(*golden_rows(rec, "quant_gauss", cb.get_quantized_patches(x, True)), 1e-6, "quant_gauss")
+            assert torch.equal(*golden_rows(rec, "quant_hard", cb.get_quantized_patches(x, False)))
+            assert_close_norm(*golden_rows(rec, "forward_gauss", cb(x)), 1e-6, "forward")
+            assert torch.equal(*golden_rows(rec, "quant_image", cb.get_quantized_image(rec["bmu_reshaped"])))
 
 
 @pytest.mark.parametrize("name", CASES)
@@ -43,8 +45,8 @@ def test_oracle_step_matches_reference(name):
     opt = make_reference_optimizer(cb, 1e-4)
     loss = reference_step(cb, opt, rec["x"])
     assert_close_norm(loss, rec["loss"], 1e-6, "loss")
-    assert_close_norm(cb.codebook.weight.grad, rec["grad"], 1e-6, "grad")
-    assert_close_norm(cb.codebook.weight.detach(), rec["weight_after_step"], 1e-6, "weight")
+    assert_close_norm(*golden_rows(rec, "grad", cb.codebook.weight.grad), 1e-6, "grad")
+    assert_close_norm(*golden_rows(rec, "weight_after_step", cb.codebook.weight.detach()), 1e-6, "weight")
 
 
 @pytest.mark.parametrize("name", CASES)
@@ -54,14 +56,14 @@ def test_closed_form_and_factorised_match_reference(name):
     st = AdamState.zeros_like(w)
     loss, bmu, grad = closed_form_step(w, st, rec["x"], rec["patch_dim"], rec["neighbourhood_range"],
                                        1e-4, bmu=rec["bmu"])
-    assert_close_norm(grad, rec["grad"], 2e-6, "closed-form grad")
-    assert_close_norm(w, rec["weight_after_step"], 1e-6, "closed-form weight")
+    assert_close_norm(*golden_rows(rec, "grad", grad), 2e-6, "closed-form grad")
+    assert_close_norm(*golden_rows(rec, "weight_after_step", w), 1e-6, "closed-form weight")
     assert_close_norm(loss, rec["loss"], 1e-6, "closed-form loss")
     flat = flat_patches(rec["x"], rec["patch_dim"])
     _, _, counts, sse, g = factorised_grad(rec["weight"], flat, rec["bmu"], rec["neighbourhood_range"],
                                            rec["x"].numel())
     assert int(counts.sum()) == flat.shape[0]
-    assert_close_norm(g, rec["grad"], 2e-6, "factorised grad")
+    assert_close_norm(*golden_rows(rec, "grad", g), 2e-6, "factorised grad")
     assert_close_norm(sse / rec["x"].numel(), rec["loss"], 1e-6, "factorised loss")
 
 
@@ -88,8 +90,8 @@ def test_oracle_free_run_100_steps():
             cb.decrease_neighbourhood(steps=1)
         assert cb.neighbourhood_range == run["ranges"][step]
         if step + 1 in run["weights"]:
-            assert_close_norm(cb.codebook.weight.detach(), run["weights"][step + 1], 1e-5,
-                              f"weights@{step + 1}")
+            w, snaps = golden_rows(run, "weights", cb.codebook.weight.detach())
+            assert_close_norm(w, snaps[step + 1], 1e-5, f"weights@{step + 1}")
 
 
 def test_oracle_prune_matches_reference():
