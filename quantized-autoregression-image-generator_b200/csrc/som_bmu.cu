@@ -15,6 +15,10 @@ bool tc_can_stage(int64_t n_patches, int D, int K, int arith);
 int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn, int K,
                   int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
                   int arith, cudaStream_t st);
+bool tc_f16_native(int64_t n_patches, int D, int K, int arith);
+int launch_bmu_tc_f16(const void* x, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
+                      int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes, int arith,
+                      cudaStream_t st);
 }  // namespace som
 
 using namespace som;
@@ -87,6 +91,29 @@ extern "C" int som_bmu_stage_nchw_f32(const float* x, int64_t n_img, int C, int 
     SOM_REQUIRE(stage_rows == nullptr, SOM_E_UNSUPPORTED, "bmu: the FFMA variant does not emit a staging copy");
     return launch_bmu_ffma(x, g, W, c_norm2, K, unit_offset, out_idx, out_rd, ws, ws_bytes,
                            (cudaStream_t)stream);
+}
+
+extern "C" int som_bmu_f16_native(int64_t n_patches, int D, int K, int variant) {
+    if (n_patches <= 0 || D <= 0 || K <= 0) return 0;
+    if (variant == SOM_BMU_AUTO) variant = som_bmu_pick_variant(n_patches, D, K);
+    return is_tc(variant) && tc_f16_native(n_patches, D, K, arith_of(variant)) ? 1 : 0;
+}
+
+extern "C" int som_bmu_stage_nchw_f16(const void* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                      const float* W, const float* c_norm2, int K, int64_t unit_offset,
+                                      int64_t* out_idx, float* out_rd, float* stage_rows,
+                                      void* ws, size_t ws_bytes, int variant, void* stream) {
+    SOM_REQUIRE(W && c_norm2 && ((x && out_idx) || n_img == 0), SOM_E_BADARG, "bmu(f16): null pointer");
+    SOM_REQUIRE(K > 0, SOM_E_BADARG, "bmu(f16): K=%d", K);
+    SOM_REQUIRE(variant >= SOM_BMU_AUTO && variant <= SOM_BMU_TC_F16, SOM_E_BADARG, "bmu(f16): variant=%d", variant);
+    Geom g;
+    int rc = make_geom(&g, x, n_img, C, H, Wd, pH, pW, 2);
+    if (rc) return rc;
+    if (g.n_patches == 0) return SOM_OK;
+    if (variant == SOM_BMU_AUTO) variant = som_bmu_pick_variant(g.n_patches, g.D, K);
+    SOM_REQUIRE(is_tc(variant), SOM_E_UNSUPPORTED, "bmu(f16): the FFMA variant does not read fp16 input");
+    return launch_bmu_tc_f16(x, g, W, c_norm2, K, unit_offset, out_idx, out_rd, stage_rows, ws, ws_bytes,
+                             arith_of(variant), (cudaStream_t)stream);
 }
 
 extern "C" int som_bmu_flat_f32(const float* patches, int64_t n, int D, const float* W, const float* c_norm2, int K,

@@ -30,6 +30,13 @@
 //   warps 6-13  epilogue    : tcgen05.ld of their TMEM lane quarter / column half, exact running (min, index) per
 //                             patch row; the N x K distance matrix never leaves TMEM
 // Bound: tensor pipe (FP16 rate / 3).
+//
+// FP16 input (T = __half, som_bmu_stage_nchw_f16): the builders read halves and upcast them exactly, so everything
+// from the row scale on sees the values x.float() would give.  When s_p x is itself exact in FP16 (fp16 data and a
+// row scale of at least 1 that no clamp lowered), lo(s_p x) is zero: every builder warp reports whether any lo of
+// its rows in a 64-feature block is non-zero, and the issuer drops the A_lo x B_hi group of that block when none is
+// (9 instead of 13 MMAs per tile at D = 64).  The dropped products are exact zeros; the fp32 instantiation never reads
+// the flag and keeps its MMA sequence.
 #include "som_common.cuh"
 #include "som_tc_ptx.cuh"
 
@@ -63,7 +70,7 @@ struct Params {
     int64_t unit_offset;
     int64_t* out_idx;
     float* out_rd;
-    const float* x;
+    const void* x;          // float or __half, per the kernel's T
     Geom g;
     const float* scale;     // [s_c, t_c] written by cb_scale_l_kernel earlier on the stream
     float* stage;           // optional patch-major copy of the patch rows (n_patches x D), written by the builders
@@ -83,6 +90,8 @@ struct Aux {
     float mrg_val[2][TM];
     int mrg_idx[2][TM];
     int row_exp[2][TM];
+    // FP16 input: per A slot one byte per builder warp (CG x 4, all in the leader CTA): "a lo of my rows is non-zero"
+    alignas(8) uint8_t lo_nz[NA_MAX][8];
 };
 constexpr uint32_t SMEM_BYTES = 1024 + TILES_BYTES + sizeof(Aux);
 
@@ -105,9 +114,32 @@ __device__ long long g_prof16[8];             // CTA 0's MMA loop: cycles, tiles
 // (block 0) the norm tail -- so the issuing thread pays ONE barrier wait and ONE commit per block instead of three.
 // With 13 MMAs per tile the issuing thread, not the tensor pipe, sets the pace otherwise (~48 cycles per MMA issue,
 // ~100 per barrier check, ~120 per commit).
-template <int CG, bool MERGED>
+// exact fp32 values of 4 / 2 / 1 consecutive input elements (float or __half)
+__device__ __forceinline__ void ld4(const float* p, float* o) {
+    const float4 f = __ldg(reinterpret_cast<const float4*>(p));
+    o[0] = f.x; o[1] = f.y; o[2] = f.z; o[3] = f.w;
+}
+__device__ __forceinline__ void ld4(const __half* p, float* o) {
+    const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
+    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&r.x));
+    const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&r.y));
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
+}
+__device__ __forceinline__ void ld2(const float* p, float* o) {
+    const float2 f = __ldg(reinterpret_cast<const float2*>(p));
+    o[0] = f.x; o[1] = f.y;
+}
+__device__ __forceinline__ void ld2(const __half* p, float* o) {
+    const float2 f = __half22float2(__ldg(reinterpret_cast<const __half2*>(p)));
+    o[0] = f.x; o[1] = f.y;
+}
+__device__ __forceinline__ float ld1(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld1(const __half* p) { return __half2float(__ldg(p)); }
+
+template <int CG, bool MERGED, typename T>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_t, const Params P) {
+    constexpr bool F16 = sizeof(T) == 2;
     pdl_launch_dependents();            // (the wait on the operand-split kernel comes after the barrier / TMEM prologue)
     extern __shared__ uint8_t smem_raw[];
     // 1024-byte alignment as an OFFSET into the shared array: rounding the pointer through uintptr_t made the compiler
@@ -143,6 +175,8 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
             mbar_init(&bars.acc_empty[a], EPI_WARPS * CG);
             mbar_init(&bars.exp_full[a], BUILD_WARPS);
         }
+        if (F16)
+            for (int s = 0; s < NA_MAX; ++s) *reinterpret_cast<uint64_t*>(aux.lo_nz[s]) = 0ull;
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     for (int d = threadIdx.x; d < D; d += NUM_THREADS) aux.foff[d] = feat_off(P.g, d);
@@ -239,7 +273,12 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
         const bool prof = blockIdx.x == 0;
         long long w_acc = 0, w_b = 0, w_a = 0;
         const long long t_begin = clock64();
+        // F16: bit fb set = block fb of this job's patch tile has a non-zero lo (read once per job, at n == 0)
+        auto lo_flag = [&](int as) -> uint32_t {
+            return *reinterpret_cast<volatile uint64_t*>(aux.lo_nz[as]) != 0ull ? 1u : 0u;
+        };
         for (int q = job0; q < n_jobs; q += job_stride, ++i) {
+            uint32_t lo_mask = 0xFu;
             for (int n = 0; n < P.NT; ++n) {
                 long long c0 = prof ? clock64() : 0;
                 mma_wait(&bars.acc_empty[j & 1u], ((j >> 1) & 1u) ^ 1u);
@@ -254,6 +293,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                             c0 = prof ? clock64() : 0;
                             mma_wait(&bars.a_full[as], (uint32_t)(u / NA) & 1u);
                             if (prof) w_a += clock64() - c0;
+                            if (F16) lo_mask = (lo_mask & ~(1u << fb)) | (lo_flag(as) << fb);
                         }
                         const uint64_t ahi = adesc0 + (uint32_t)as * A_SLOT_UNITS;
                         const uint64_t alo = ahi + A_LO_UNITS;
@@ -270,9 +310,11 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
                                 if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, bhi + 2u * k, 1u);
+                            if (!F16 || ((lo_mask >> fb) & 1u)) {
 #pragma unroll
-                            for (int k = 0; k < 4; ++k)
-                                if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bhi + 2u * k, 1u);
+                                for (int k = 0; k < 4; ++k)
+                                    if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bhi + 2u * k, 1u);
+                            }
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
                                 if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, blo + 2u * k, 1u);
@@ -289,6 +331,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                 if (n == 0) {                   // block 0 of this job (and with it the job's tail rows)
                     const int u = i * DB;
                     mma_wait(&bars.a_full[u % NA], (uint32_t)(u / NA) & 1u);
+                    if (F16) lo_mask = (lo_mask & ~1u) | lo_flag(u % NA);
                 }
                 tc_fence_after();
                 if (leader) {
@@ -300,7 +343,10 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     const int nks = (fb == DB - 1) ? P.nks_last : 4;
                     const int u = i * DB + fb;
                     const int as = u % NA;
-                    if (n == 0 && fb > 0) mma_wait(&bars.a_full[as], (uint32_t)(u / NA) & 1u);
+                    if (n == 0 && fb > 0) {
+                        mma_wait(&bars.a_full[as], (uint32_t)(u / NA) & 1u);
+                        if (F16) lo_mask = (lo_mask & ~(1u << fb)) | (lo_flag(as) << fb);
+                    }
                     const uint64_t ahi = adesc0 + (uint32_t)as * A_SLOT_UNITS;
                     const uint64_t alo = ahi + A_LO_UNITS;
                     mma_wait(&bars.b_full[bs], b_ph);
@@ -310,9 +356,11 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
 #pragma unroll
                         for (int k = 0; k < 4; ++k)
                             if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
+                        if (!F16 || ((lo_mask >> fb) & 1u)) {
 #pragma unroll
-                        for (int k = 0; k < 4; ++k)
-                            if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
+                            for (int k = 0; k < 4; ++k)
+                                if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
+                        }
                         tc_commit_cg<CG>(&bars.b_empty[bs]);
                     }
                     if (++bs == NB) { bs = 0; b_ph ^= 1; }
@@ -344,26 +392,22 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
         const uint32_t sw = (uint32_t)(t & 7);
         float v[64];
         // 64 features [64 fb, 64 fb + 64) of one patch row; zero beyond D and for padding rows
-        auto load_blk = [&](const float* src, bool ok, int fb) {
+        // (vec counts elements: 16- / 8-byte runs of floats, 8- / 4-byte runs of halves)
+        auto load_blk = [&](const T* src, bool ok, int fb) {
 #pragma unroll
             for (int c = 0; c < 16; ++c) {
                 const int d = fb * 64 + c * 4;
                 float tmp[4] = {0.f, 0.f, 0.f, 0.f};
                 if (ok && d < D) {
                     if (vec == 4) {
-                        const float4 f = __ldg(reinterpret_cast<const float4*>(src + aux.foff[d]));
-                        tmp[0] = f.x; tmp[1] = f.y; tmp[2] = f.z; tmp[3] = f.w;
+                        ld4(src + aux.foff[d], tmp);
                     } else if (vec == 2) {
-                        const float2 f0 = __ldg(reinterpret_cast<const float2*>(src + aux.foff[d]));
-                        tmp[0] = f0.x; tmp[1] = f0.y;
-                        if (d + 2 < D) {
-                            const float2 f1 = __ldg(reinterpret_cast<const float2*>(src + aux.foff[d + 2]));
-                            tmp[2] = f1.x; tmp[3] = f1.y;
-                        }
+                        ld2(src + aux.foff[d], tmp);
+                        if (d + 2 < D) ld2(src + aux.foff[d + 2], tmp + 2);
                     } else {
 #pragma unroll
                         for (int e = 0; e < 4; ++e)
-                            if (d + e < D) tmp[e] = __ldg(src + aux.foff[d + e]);
+                            if (d + e < D) tmp[e] = ld1(src + aux.foff[d + e]);
                     }
                 }
 #pragma unroll
@@ -375,7 +419,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
             const int m = CG * q + (int)rank;
             const int64_t p = (int64_t)m * TM + t;
             const bool ok = p < P.rows;
-            const float* src = P.x + (ok ? patch_base(P.g, p) : 0);
+            const T* src = static_cast<const T*>(P.x) + (ok ? patch_base(P.g, p) : 0);
             // pass 1: the row's largest magnitude (a one-block row stays in registers for pass 2)
             float mx = 0.f;
             for (int fb = 0; fb < DB; ++fb) {
@@ -423,6 +467,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                 mbar_wait_warp<true>(&bars.a_empty[as], ((uint32_t)(u / NA) & 1u) ^ 1u, lane);
                 uint8_t* hi_row = a_ring + (size_t)as * A_SLOT_BYTES + (uint32_t)t * 128u;
                 uint8_t* lo_row = hi_row + A_BLK_BYTES;
+                bool lo_nz = false;
 #pragma unroll
                 for (int c = 0; c < 8; ++c) {
                     float h[8], l[8];
@@ -431,6 +476,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                         const float s = v[c * 8 + e] * sp;                   // exact
                         h[e] = __half2float(__float2half_rn(s));
                         l[e] = s - h[e];                                     // exact; rounded to FP16 when packed
+                        if (F16) lo_nz |= l[e] != 0.f;                       // (NaN counts as non-zero)
                     }
                     // 16-byte chunk c of row t lives at t * 128 + ((c ^ (t & 7)) << 4)
                     const uint32_t off = (((uint32_t)c) ^ sw) << 4;
@@ -446,8 +492,24 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     aux.row_exp[i & 1][t] = es;
                 }
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                const bool warp_lo_nz = F16 && __any_sync(0xffffffffu, lo_nz);
                 __syncwarp();
                 if (lane == 0) {
+                    if (F16) {
+                        // this warp's byte of the slot's flag, in the leader CTA; the release arrive below publishes it
+                        uint8_t* fl = &aux.lo_nz[as][rank * BUILD_WARPS + (warp - BUILD_WARP0)];
+                        if (CG == 2) {
+                            asm volatile(
+                                "{\n"
+                                ".reg .b32 ra;\n"
+                                "mapa.shared::cluster.u32 ra, %0, 0;\n"
+                                "st.shared::cluster.u8 [ra], %1;\n"
+                                "}\n" ::"r"(smem_u32(fl)), "r"((uint32_t)warp_lo_nz)
+                                : "memory");
+                        } else {
+                            *reinterpret_cast<volatile uint8_t*>(fl) = (uint8_t)warp_lo_nz;
+                        }
+                    }
                     if (CG == 2) mbar_arrive_remote(&bars.a_full[as], 0);      // the leader's barrier counts both CTAs
                     else mbar_arrive(&bars.a_full[as]);
                     if (fb == 0) mbar_arrive(&bars.exp_full[i & 1]);           // release: row_exp visible
@@ -668,9 +730,9 @@ size_t tc_l16_workspace_bytes(int64_t n_patches, int D, int K, bool force) {
     return tcl16::make_plan(&pl, n_patches, D, K, force) ? pl.total : 0;
 }
 
-int launch_bmu_tc_l16(const float* x, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
-                      int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes, bool force,
-                      cudaStream_t st) {
+int launch_bmu_tc_l16(const void* x, bool x_f16, const Geom& g, const float* W, const float* cn, int K,
+                      int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
+                      bool force, cudaStream_t st) {
     using namespace tcl16;
     const int64_t n = g.n_patches;
     if (n == 0) return SOM_OK;
@@ -713,11 +775,14 @@ int launch_bmu_tc_l16(const float* x, const Geom& g, const float* W, const float
     P.x = x; P.g = g; P.scale = scale; P.stage = stage;
 
     typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const Params);
-    static const KernelFn kernels[4] = {bmu_tc_l16_kernel<1, false>, bmu_tc_l16_kernel<2, false>,
-                                        bmu_tc_l16_kernel<1, true>, bmu_tc_l16_kernel<2, true>};
+    static const KernelFn kernels[8] = {
+        bmu_tc_l16_kernel<1, false, float>, bmu_tc_l16_kernel<2, false, float>,
+        bmu_tc_l16_kernel<1, true, float>, bmu_tc_l16_kernel<2, true, float>,
+        bmu_tc_l16_kernel<1, false, __half>, bmu_tc_l16_kernel<2, false, __half>,
+        bmu_tc_l16_kernel<1, true, __half>, bmu_tc_l16_kernel<2, true, __half>};
     static PerDeviceFlag attr_done;
     if (attr_done.pending()) {
-        for (int c = 0; c < 4; ++c) {
+        for (int c = 0; c < 8; ++c) {
             cudaError_t e = cudaFuncSetAttribute(kernels[c], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
             if (e != cudaSuccess) { set_error("bmu(tc f16): smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
         }
@@ -740,7 +805,7 @@ int launch_bmu_tc_l16(const float* x, const Geom& g, const float* W, const float
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = pdl_enabled() ? 2 : 1;
-    cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[2 * pl.merged + pl.cg - 1], map_b, map_t, P);
+    cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[4 * (x_f16 ? 1 : 0) + 2 * pl.merged + pl.cg - 1], map_b, map_t, P);
     if (le != cudaSuccess) { set_error("bmu_tc_l16_kernel: launch: %s", cudaGetErrorString(le)); return (int)le; }
     return check_launch("bmu_tc_l16_kernel");
 }

@@ -44,7 +44,8 @@ struct Geom {
     int vec;             // widest aligned vector (floats) along a patch row: 4, 2 or 1
 };
 
-int make_geom(Geom* g, const void* x, int64_t n_img, int C, int H, int W, int pH, int pW);
+// elem_bytes: 4 for an fp32 batch, 2 for a binary16 one (vec then counts halves)
+int make_geom(Geom* g, const void* x, int64_t n_img, int C, int H, int W, int pH, int pW, int elem_bytes = 4);
 
 __host__ __device__ __forceinline__ int64_t patch_base(const Geom& g, int64_t p) {
     if (g.seq == 1) return p * g.img_stride;      // one patch per image (e.g. pre-flattened rows): no divisions

@@ -159,7 +159,8 @@ class DataParallelSom(SomTrainer):
             return super()._device_step(feature_map, bmu)
         ops, cb, pm = self.ops, self.cb, self.peer
         w = cb.codebook.weight.data
-        x, geom = cb._input(feature_map)
+        x, geom = cb._input(feature_map, allow_half=True)
+        x = self._half_input(x, geom, staged=bmu is None)
         k, d = cb.num_embeddings, cb.embedding_dim
         rng = cb.neighbourhood_range
         kd = k * d

@@ -6,8 +6,11 @@ DataLoader workers (``dataset_loader/feature_map_dataset.py:22-42``).  At 1e8-1e
 reader, not the GPU, bounds tokenisation and pruning.  This module packs the same data into a few
 large, memory-mappable shards and streams them into pinned batches:
 
-    shard file  = 64-byte header | n * C*H*W float32, C-contiguous (the reference's dtype and layout)
-    header      = b"SOMFMAP1" | u32 version | u32 C | u32 H | u32 W | u64 n | zero padding to 64 bytes
+    shard file  = 64-byte header | n * C*H*W values, C-contiguous (the reference's layout)
+    header v1   = b"SOMFMAP1" | u32 version = 1 | u32 C | u32 H | u32 W | u64 n | zero padding to 64 bytes
+                  (float32 values, the reference's dtype)
+    header v2   = the same with version = 2 and a u32 dtype code at byte 32 (1 = float16): half the bytes to
+                  read and to copy to the device; the searches treat the values as what they are (as ``.float()``)
 
 * ``convert_reference_dataset`` reads the reference layout (TinyDB json -> ``fmap_path`` entries, in
   document order) and writes shards; ``image_path`` is kept in a side ``index.json``.
@@ -23,36 +26,68 @@ import torch
 
 MAGIC = b"SOMFMAP1"
 HEADER_BYTES = 64
-VERSION = 1
+VERSION = 1                       # float32 shards
+VERSION_DTYPE = 2                 # shards of another dtype: u32 code at byte 32
+DTYPE_CODES = {1: np.dtype(np.float16)}
 
 
-def _header(c, h, w, n):
-    head = MAGIC + struct.pack("<IIIIQ", VERSION, c, h, w, n)
+def _header(c, h, w, n, dtype):
+    if dtype == np.float32:
+        head = MAGIC + struct.pack("<IIIIQ", VERSION, c, h, w, n)
+    else:
+        code = next(k for k, v in DTYPE_CODES.items() if v == dtype)
+        head = MAGIC + struct.pack("<IIIIQI", VERSION_DTYPE, c, h, w, n, code)
     return head + b"\0" * (HEADER_BYTES - len(head))
 
 
-def read_header(path):
+def _read_header(path):
     with open(path, "rb") as f:
         head = f.read(HEADER_BYTES)
     if len(head) != HEADER_BYTES or head[:8] != MAGIC:
         raise ValueError(f"{path}: not a feature-map shard")
     version, c, h, w, n = struct.unpack("<IIIIQ", head[8:32])
-    if version != VERSION:
-        raise ValueError(f"{path}: shard version {version}, expected {VERSION}")
-    expect = HEADER_BYTES + n * c * h * w * 4
+    if version == VERSION:
+        dtype = np.dtype(np.float32)
+    elif version == VERSION_DTYPE:
+        (code,) = struct.unpack("<I", head[32:36])
+        if code not in DTYPE_CODES:
+            raise ValueError(f"{path}: unknown dtype code {code}")
+        dtype = DTYPE_CODES[code]
+    else:
+        raise ValueError(f"{path}: shard version {version}, expected {VERSION} or {VERSION_DTYPE}")
+    expect = HEADER_BYTES + n * c * h * w * dtype.itemsize
     if os.path.getsize(path) != expect:
         raise ValueError(f"{path}: size {os.path.getsize(path)} != {expect} implied by the header")
-    return c, h, w, n
+    return c, h, w, n, dtype
 
 
-def write_shard(path, fmaps):
-    """fmaps: (n, C, H, W) float32 array-like.  Returns n."""
-    arr = np.ascontiguousarray(np.asarray(fmaps), dtype=np.float32)
+def read_header(path):
+    """(C, H, W, n) of a shard of either version."""
+    return _read_header(path)[:4]
+
+
+def shard_dtype(path):
+    """numpy dtype of a shard's values (float32 for version 1)."""
+    return _read_header(path)[4]
+
+
+def _check_dtype(dtype):
+    dtype = np.dtype(dtype)
+    if dtype != np.float32 and dtype not in DTYPE_CODES.values():
+        raise ValueError(f"shards hold float32 or float16 values, not {dtype}")
+    return dtype
+
+
+def write_shard(path, fmaps, dtype=np.float32):
+    """fmaps: (n, C, H, W) array-like, stored as ``dtype`` (float32: version 1, float16: version 2; values are
+    rounded to nearest by numpy's conversion).  Returns n."""
+    dtype = _check_dtype(dtype)
+    arr = np.ascontiguousarray(np.asarray(fmaps), dtype=dtype)
     if arr.ndim != 4:
         raise ValueError("write_shard expects (n, C, H, W)")
     n, c, h, w = arr.shape
     with open(path, "wb") as f:
-        f.write(_header(c, h, w, n))
+        f.write(_header(c, h, w, n, dtype))
         f.write(arr.tobytes(order="C"))
     return n
 
@@ -69,9 +104,11 @@ def reference_entries(db_json_path):
     return [table[k] for k in sorted(table, key=lambda s: int(s))]
 
 
-def convert_reference_dataset(db_json_path, out_dir, fmaps_per_shard=65536, path_root=None):
-    """Pack the reference's per-file dataset into shards.  ``path_root`` re-bases relative
-    ``fmap_path`` entries.  Returns the list of shard paths; writes ``index.json`` beside them."""
+def convert_reference_dataset(db_json_path, out_dir, fmaps_per_shard=65536, path_root=None, dtype=np.float32):
+    """Pack the reference's per-file dataset into shards of ``dtype`` (float32 or float16, see ``write_shard``).
+    ``path_root`` re-bases relative ``fmap_path`` entries.  Returns the list of shard paths; writes ``index.json``
+    beside them."""
+    dtype = _check_dtype(dtype)
     entries = reference_entries(db_json_path)
     os.makedirs(out_dir, exist_ok=True)
     shards, index, batch = [], [], []
@@ -80,7 +117,7 @@ def convert_reference_dataset(db_json_path, out_dir, fmaps_per_shard=65536, path
         if not batch:
             return
         path = os.path.join(out_dir, f"fmaps_{len(shards):05d}.shard")
-        write_shard(path, np.stack(batch))
+        write_shard(path, np.stack(batch), dtype=dtype)
         shards.append(path)
         batch.clear()
 
@@ -90,7 +127,7 @@ def convert_reference_dataset(db_json_path, out_dir, fmaps_per_shard=65536, path
             p = os.path.join(path_root, p)
         with open(p, "rb") as f:
             fmap = np.load(f, allow_pickle=False)           # as feature_map_dataset.py:38-39
-        batch.append(np.asarray(fmap, dtype=np.float32))    # .float() of :42
+        batch.append(np.asarray(fmap, dtype=dtype))         # .float() of :42 (float16: one rounding)
         index.append({"i": i, "shard": len(shards), "row": len(batch) - 1,
                       "image_path": doc.get("image_path")})
         if len(batch) == fmaps_per_shard:
@@ -111,14 +148,18 @@ class ShardReader:
             raise Exception("No data found.")
         self.paths = list(shard_paths)
         self.shape = None
+        self.dtype = None             # numpy dtype of every shard (batches come in it)
         self.counts = []
         for p in self.paths:
-            c, h, w, n = read_header(p)
+            c, h, w, n, dt = _read_header(p)
             if self.shape is None:
-                self.shape = (c, h, w)
+                self.shape, self.dtype = (c, h, w), dt
             elif self.shape != (c, h, w):
                 raise ValueError(f"{p}: shape {(c, h, w)} differs from {self.shape}")
+            elif self.dtype != dt:
+                raise ValueError(f"{p}: dtype {dt} differs from {self.dtype}")
             self.counts.append(n)
+        self._torch_dtype = torch.float16 if self.dtype == np.float16 else torch.float32
         self.batch = int(batch_fmaps)
         self.pin = bool(pin) and torch.cuda.is_available()
         self.depth = int(depth)
@@ -139,13 +180,13 @@ class ShardReader:
 
     def _map(self, i):
         c, h, w = self.shape
-        return np.memmap(self.paths[i], dtype=np.float32, mode="r", offset=HEADER_BYTES,
+        return np.memmap(self.paths[i], dtype=self.dtype, mode="r", offset=HEADER_BYTES,
                          shape=(self.counts[i], c, h, w))
 
     def read_all(self):
-        """All feature maps as one (N, C, H, W) float32 tensor (pinned when CUDA is present)."""
+        """All feature maps as one (N, C, H, W) tensor of the shards' dtype (pinned when CUDA is present)."""
         c, h, w = self.shape
-        out = torch.empty(len(self), c, h, w, dtype=torch.float32, pin_memory=self.pin)
+        out = torch.empty(len(self), c, h, w, dtype=self._torch_dtype, pin_memory=self.pin)
         lo = 0
         for i, n in enumerate(self.counts):
             out[lo:lo + n].numpy()[...] = self._map(i)
@@ -153,11 +194,11 @@ class ShardReader:
         return out
 
     def batches(self):
-        """Yields (lo, hi, tensor) with tensor a (hi - lo, C, H, W) float32 view of a staging buffer
+        """Yields (lo, hi, tensor) with tensor a (hi - lo, C, H, W) view (shards' dtype) of a staging buffer
         that stays valid until ``depth`` further batches have been produced."""
         c, h, w = self.shape
         if self._bufs is None:
-            self._bufs = [torch.empty(self.batch, c, h, w, dtype=torch.float32, pin_memory=self.pin)
+            self._bufs = [torch.empty(self.batch, c, h, w, dtype=self._torch_dtype, pin_memory=self.pin)
                           for _ in range(self.depth)]
         k, lo = 0, 0
         for i, n in enumerate(self.counts):

@@ -53,15 +53,15 @@ class HostTokenizer:
         self._bufs = None
         self.done = None
 
-    def _alloc(self, c, h, w, seq):
-        key = (c, h, w, seq)
+    def _alloc(self, c, h, w, seq, dtype):
+        key = (c, h, w, seq, dtype)
         if self._bufs is not None and self._bufs[0] == key:
             return self._bufs[1]
         dev = self.device
         slots = []
         for _ in range(self.depth):
             slots.append({
-                "x": torch.empty(self.chunk, c, h, w, dtype=torch.float32, device=dev),
+                "x": torch.empty(self.chunk, c, h, w, dtype=dtype, device=dev),
                 "idx": torch.empty(self.chunk * seq, dtype=torch.int64, device=dev),
                 "h2d": torch.cuda.Event(), "comp": torch.cuda.Event(), "d2h": torch.cuda.Event(),
             })
@@ -71,7 +71,8 @@ class HostTokenizer:
 
     @torch.no_grad()
     def tokenize(self, fmaps_host, out_host=None, sync=True):
-        """fmaps_host: (N, C, H, W) fp32 host tensor (pinned for async copies).  Returns the
+        """fmaps_host: (N, C, H, W) fp32 or fp16 host tensor (pinned for async copies; an fp16 batch is copied as
+        fp16, half the bytes, and searched as if it were ``fmaps_host.float()``).  Returns the
         (N, Seq) int64 host tensor of BMU indices (``out_host`` if given, pinned otherwise).
 
         With ``sync=True`` (default) the call returns only after the last device-to-host copy has landed and the
@@ -84,7 +85,8 @@ class HostTokenizer:
         seq = _ops.n_patches_of(geom1)
         if out_host is None:
             out_host = torch.empty(n, seq, dtype=torch.int64, pin_memory=True)
-        slots, (s_in, s_out) = self._alloc(c, h, w, seq)
+        dtype = torch.float16 if fmaps_host.dtype == torch.float16 else torch.float32
+        slots, (s_in, s_out) = self._alloc(c, h, w, seq, dtype)
         compute = torch.cuda.current_stream(self.device)
         weight = cb.codebook.weight.detach()
         norms = cb._norms()
@@ -152,20 +154,23 @@ class HostTrainer:
         self._i = 0
         self._copy = torch.cuda.Stream(self.device)
 
-    def _alloc(self, shape):
-        if self._slots is not None and self._slots[0] == tuple(shape):
+    def _alloc(self, shape, dtype):
+        key = (tuple(shape), dtype)
+        if self._slots is not None and self._slots[0] == key:
             return self._slots[1]
-        slots = [{"x": torch.empty(shape, dtype=torch.float32, device=self.device),
+        slots = [{"x": torch.empty(shape, dtype=dtype, device=self.device),
                   "loss": torch.empty((), dtype=torch.float64, pin_memory=True),
                   "h2d": torch.cuda.Event(), "done": None} for _ in range(self.depth)]
-        self._slots = (tuple(shape), slots)
+        self._slots = (key, slots)
         return slots
 
     @torch.no_grad()
     def step(self, fmaps_host):
-        """Enqueue copy + step for one (local) host batch (pinned for asynchronous copies); returns a PendingLoss.
+        """Enqueue copy + step for one (local) host batch (pinned for asynchronous copies; fp16 batches are staged as
+        fp16 and trained on as if they were ``fmaps_host.float()``); returns a PendingLoss.
         ``fmaps_host`` may be refilled once ``h2d_done()`` of this call has completed (or after the loss is read)."""
-        slots = self._alloc(fmaps_host.shape)
+        slots = self._alloc(fmaps_host.shape,
+                            torch.float16 if fmaps_host.dtype == torch.float16 else torch.float32)
         sl = slots[self._i % self.depth]
         self._i += 1
         compute = torch.cuda.current_stream(self.device)

@@ -92,15 +92,45 @@ def bmu_can_stage(geom, num_units, variant=SOM_BMU_AUTO):
     return bool(_lib.load().som_bmu_can_stage(n_patches_of(geom), dim_of(geom), int(num_units), int(variant)))
 
 
+def bmu_f16_native(geom, num_units, variant=SOM_BMU_AUTO):
+    """Whether the BMU kernel for this shape reads an fp16 batch itself (otherwise ``bmu`` upcasts it first)."""
+    return bool(_lib.load().som_bmu_f16_native(n_patches_of(geom), dim_of(geom), int(num_units), int(variant)))
+
+
+def upcast_f16(x, out=None):
+    """Exact fp32 copy of a contiguous fp16 CUDA tensor (som_convert_f16_f32); ``out``: optional fp32 destination of
+    the same number of elements."""
+    lib = _lib.load()
+    x = _req(x, torch.float16, "x")
+    if out is None:
+        out = torch.empty(x.shape, dtype=torch.float32, device=x.device)
+    out = _req(out, torch.float32, "out")
+    if out.numel() != x.numel():
+        raise ValueError("out must hold as many elements as x")
+    with torch.cuda.device(x.device):
+        check("som_convert_f16_f32", lib.som_convert_f16_f32(_ptr(x), x.numel(), _ptr(out), _stream(x)))
+    return out
+
+
 def bmu(x, geom, weight, c_norm2=None, unit_offset=0, want_rd=False, variant=SOM_BMU_AUTO,
         out=None, stage=None):
-    """K1.  x: fp32 contiguous buffer described by ``geom``.  Returns idx (n_patches,) int64
+    """K1.  x: fp32 or fp16 contiguous buffer described by ``geom``.  Returns idx (n_patches,) int64
     [and the reduced distance rd (n_patches,) fp32 when ``want_rd``].  ``stage``: optional (n_patches, D) fp32
-    tensor that receives the patch-major copy of the patch rows (only where ``bmu_can_stage``)."""
+    tensor that receives the patch-major copy of the patch rows (only where ``bmu_can_stage``).
+
+    An fp16 ``x`` gives exactly the results of the same call on ``x.float()``: the FP16-split kernel reads it
+    directly where ``bmu_f16_native`` says so, other shapes search an fp32 copy made by ``upcast_f16``."""
     lib = _lib.load()
-    x = _req(x, torch.float32, "x")
     w = _req(weight, torch.float32, "weight")
     k, d = w.shape
+    if isinstance(x, torch.Tensor) and x.dtype == torch.float16:
+        x = _req(x, torch.float16, "x")
+        if not bmu_f16_native(geom, k, variant):
+            return bmu(upcast_f16(x), geom, w, c_norm2, unit_offset, want_rd, variant, out, stage)
+        entry = "som_bmu_stage_nchw_f16"
+    else:
+        x = _req(x, torch.float32, "x")
+        entry = "som_bmu_stage_nchw_f32"
     if d != dim_of(geom):
         raise ValueError(f"codebook dim {d} != patch dim {dim_of(geom)}")
     npat = n_patches_of(geom)
@@ -118,8 +148,7 @@ def bmu(x, geom, weight, c_norm2=None, unit_offset=0, want_rd=False, variant=SOM
             raise ValueError("stage must hold n_patches x D floats")
     with torch.cuda.device(x.device):
         ws, ws_bytes = _workspace(lib.som_bmu_workspace_bytes(npat, d, k, variant), x.device)
-        check("som_bmu_stage_nchw_f32",
-              lib.som_bmu_stage_nchw_f32(_ptr(x), *geom, _ptr(w), _ptr(c_norm2), k, int(unit_offset),
+        check(entry, getattr(lib, entry)(_ptr(x), *geom, _ptr(w), _ptr(c_norm2), k, int(unit_offset),
                                          _ptr(out), _ptr(rd), _ptr(stage), _ptr(ws), ws_bytes, variant, _stream(x)))
     return (out, rd) if want_rd else out
 

@@ -91,15 +91,17 @@ class SomTrainer:
 
     def _graph_step(self, feature_map):
         cb = self.cb
-        alias = self._graph_alias and feature_map.is_contiguous() and feature_map.dtype == torch.float32
-        key = (tuple(feature_map.shape), float(cb.neighbourhood_range), float(self.lr),
+        # an fp16 batch keeps its dtype in the static buffer (half the bytes to copy); anything else is copied as fp32
+        dtype = torch.float16 if feature_map.dtype == torch.float16 else torch.float32
+        alias = self._graph_alias and feature_map.is_contiguous() and feature_map.dtype == dtype
+        key = (tuple(feature_map.shape), dtype, float(cb.neighbourhood_range), float(self.lr),
                feature_map.data_ptr() if alias else 0)
         entry = self._graphs.get(key)
         if entry is None:
             if len(self._graphs) >= self.MAX_GRAPHS:
                 self._graphs.pop(next(iter(self._graphs)))
             x_static = feature_map if alias else \
-                torch.empty(feature_map.shape, dtype=torch.float32, device=feature_map.device)
+                torch.empty(feature_map.shape, dtype=dtype, device=feature_map.device)
             graph = torch.cuda.CUDAGraph()
             torch.cuda.synchronize(feature_map.device)
             # thread_local: the NCCL watchdog thread may touch the CUDA API while we capture
@@ -137,13 +139,16 @@ class SomTrainer:
         ops = self.ops
         cb = self.cb
         w = cb.codebook.weight.data
-        x, geom = cb._input(feature_map, require_cuda=getattr(ops, 'REQUIRES_CUDA', True))
+        x, geom = cb._input(feature_map, require_cuda=getattr(ops, 'REQUIRES_CUDA', True), allow_half=True)
         k, d = cb.num_embeddings, cb.embedding_dim
         rng = cb.neighbourhood_range
         kd = k * d
 
-        if (bmu is None and self.reduce_fn is None and self.small_step_kernel and cb.bmu_variant == ops.SOM_BMU_AUTO
-                and getattr(ops, "step_small_supported", None) is not None and ops.step_small_supported(geom, k, rng)):
+        small = (bmu is None and self.reduce_fn is None and self.small_step_kernel
+                 and cb.bmu_variant == ops.SOM_BMU_AUTO and getattr(ops, "step_small_supported", None) is not None
+                 and ops.step_small_supported(geom, k, rng))
+        x = self._half_input(x, geom, staged=bmu is None and not small)
+        if small:
             # small problems (BASELINE config 1): the whole step is ONE cooperative kernel, a launch costs more than
             # any of the step's kernels at this size
             loss, self.last_bmu = ops.step_small(x, geom, w, self.m, self.v, rng, self.lr, self.t_dev,
@@ -188,14 +193,26 @@ class SomTrainer:
         if side is not None:
             torch.cuda.current_stream(side.device).wait_stream(side)
 
+    def _can_stage(self, geom):
+        ops, cb = self.ops, self.cb
+        can = getattr(ops, "bmu_can_stage", None)
+        return can is not None and ops.n_patches_of(geom) > 0 and can(geom, cb.num_embeddings, cb.bmu_variant)
+
+    def _half_input(self, x, geom, staged):
+        """An fp16 batch stays fp16 only where the step's search reads it itself and writes the fp32 staging rows that
+        the accumulation reads (``staged``: the step searches with the separate kernels; the staging kernel is the one
+        that reads halves).  Otherwise it is upcast once, exactly, and that copy feeds every kernel of the step."""
+        if x.dtype != torch.float16 or (staged and self._can_stage(geom)):
+            return x
+        return self.ops.upcast_f16(x)
+
     def _search(self, x, geom, w):
         """BMU search of the step.  Where the kernel can emit it, also the patch-major staging copy of the patch rows:
         the segmented gather of the update then reads one contiguous row per patch (returns the buffer and geometry
         the accumulation should read: the staging rows, or x itself)."""
         ops, cb = self.ops, self.cb
         cn = ops.prepare_codebook(w)
-        can = getattr(ops, "bmu_can_stage", None)
-        if can is not None and ops.n_patches_of(geom) > 0 and can(geom, cb.num_embeddings, cb.bmu_variant):
+        if self._can_stage(geom):
             npat, d = ops.n_patches_of(geom), ops.dim_of(geom)
             stage = torch.empty(npat, d, dtype=torch.float32, device=x.device)
             bmu = ops.bmu(x, geom, w, cn, variant=cb.bmu_variant, stage=stage)
