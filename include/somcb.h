@@ -105,21 +105,29 @@ SOM_API int som_bmu_stage_nchw_f32(const float* x, int64_t n_img, int C, int H, 
                            int64_t* out_idx, float* out_rd, float* stage_rows,
                            void* ws, size_t ws_bytes, int variant, void* stream);
 
-/* ---- K1 on binary16 feature maps --------------------------------------------------------------------------
- * An fp16 batch means the data ARE those values: every result equals the fp32 call on x.half().float().
- * som_bmu_stage_nchw_f16 is som_bmu_stage_nchw_f32 on a contiguous NCHW batch of IEEE half bit patterns (2-byte
- * aligned); stage_rows (fp32, may be NULL) is patchify(x.float()).  Only the FP16-split kernel of 16 < D <= 256 reads
- * halves itself -- ask som_bmu_f16_native (host-only) first; SOM_E_UNSUPPORTED where it says 0.  There a tile whose
- * patch rows are exact in FP16 after the row scale skips the A_lo x B_hi product group (9 instead of 13 MMAs per
- * tile at D = 64).  Other shapes: convert with som_convert_f16_f32 and call the fp32 entry points.  Same workspace
- * as som_bmu_workspace_bytes.                                                                                  */
+/* ---- K1 on 16-bit feature maps (binary16 and bfloat16) ---------------------------------------------------
+ * A 16-bit batch means the data ARE those values: every result equals the fp32 call on x.float().
+ * som_bmu_stage_nchw_f16 / _bf16 are som_bmu_stage_nchw_f32 on a contiguous NCHW batch of IEEE half / bfloat16 bit
+ * patterns (2-byte aligned); stage_rows (fp32, may be NULL) is patchify(x.float()).  Only the FP16-split kernel of
+ * 16 < D <= 256 reads 16-bit values itself -- ask som_bmu_f16_native (host-only) first: it answers for BOTH formats,
+ * the kernel being the same; SOM_E_UNSUPPORTED where it says 0.  There a tile whose patch rows are exact in FP16
+ * after the row scale skips the A_lo x B_hi product group (9 instead of 13 MMAs per tile at D = 64).  fp16 rows
+ * always are unless the row scale was clamped; a bf16 element is when it lies within about 2^-23 of its row's
+ * largest magnitude (tanh-range latents: almost every tile), so a bf16 tile may keep the third product where an fp16
+ * tile would not -- the result is exact either way.  Other shapes: convert with som_convert_f16_f32 /
+ * som_convert_bf16_f32 and call the fp32 entry points.  Same workspace as som_bmu_workspace_bytes.              */
 SOM_API int som_bmu_f16_native(int64_t n_patches, int D, int K, int variant);
 SOM_API int som_bmu_stage_nchw_f16(const void* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
                                    const float* W, const float* c_norm2, int K, int64_t unit_offset,
                                    int64_t* out_idx, float* out_rd, float* stage_rows,
                                    void* ws, size_t ws_bytes, int variant, void* stream);
-/* out[i] = (float)in[i] for n binary16 values (exact); in 2-byte, out 4-byte aligned.                        */
+SOM_API int som_bmu_stage_nchw_bf16(const void* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                    const float* W, const float* c_norm2, int K, int64_t unit_offset,
+                                    int64_t* out_idx, float* out_rd, float* stage_rows,
+                                    void* ws, size_t ws_bytes, int variant, void* stream);
+/* out[i] = (float)in[i] for n binary16 / bfloat16 values (exact); in 2-byte, out 4-byte aligned.             */
 SOM_API int som_convert_f16_f32(const void* in, int64_t n, float* out, void* stream);
+SOM_API int som_convert_bf16_f32(const void* in, int64_t n, float* out, void* stream);
 
 /* Same search on pre-flattened patch rows: `patches` is (n, D) row-major fp32 (what patchify +
  * reshape produce in models/Codebook.py:83-84).  Equivalent to som_bmu_nchw_f32 with the rows seen

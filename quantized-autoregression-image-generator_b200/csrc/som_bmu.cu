@@ -16,7 +16,7 @@ int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn
                   int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
                   int arith, cudaStream_t st);
 bool tc_f16_native(int64_t n_patches, int D, int K, int arith);
-int launch_bmu_tc_f16(const void* x, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
+int launch_bmu_tc_16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
                       int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes, int arith,
                       cudaStream_t st);
 }  // namespace som
@@ -99,21 +99,37 @@ extern "C" int som_bmu_f16_native(int64_t n_patches, int D, int K, int variant) 
     return is_tc(variant) && tc_f16_native(n_patches, D, K, arith_of(variant)) ? 1 : 0;
 }
 
-extern "C" int som_bmu_stage_nchw_f16(const void* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
-                                      const float* W, const float* c_norm2, int K, int64_t unit_offset,
-                                      int64_t* out_idx, float* out_rd, float* stage_rows,
-                                      void* ws, size_t ws_bytes, int variant, void* stream) {
-    SOM_REQUIRE(W && c_norm2 && ((x && out_idx) || n_img == 0), SOM_E_BADARG, "bmu(f16): null pointer");
-    SOM_REQUIRE(K > 0, SOM_E_BADARG, "bmu(f16): K=%d", K);
-    SOM_REQUIRE(variant >= SOM_BMU_AUTO && variant <= SOM_BMU_TC_F16, SOM_E_BADARG, "bmu(f16): variant=%d", variant);
+// fp16 / bf16 batches: the same checks and the same kernel, instantiated for the element type
+static int bmu_stage_nchw_16(const char* who, int elem, const void* x, int64_t n_img, int C, int H, int Wd, int pH,
+                             int pW, const float* W, const float* c_norm2, int K, int64_t unit_offset, int64_t* out_idx,
+                             float* out_rd, float* stage_rows, void* ws, size_t ws_bytes, int variant, void* stream) {
+    SOM_REQUIRE(W && c_norm2 && ((x && out_idx) || n_img == 0), SOM_E_BADARG, "%s: null pointer", who);
+    SOM_REQUIRE(K > 0, SOM_E_BADARG, "%s: K=%d", who, K);
+    SOM_REQUIRE(variant >= SOM_BMU_AUTO && variant <= SOM_BMU_TC_F16, SOM_E_BADARG, "%s: variant=%d", who, variant);
     Geom g;
     int rc = make_geom(&g, x, n_img, C, H, Wd, pH, pW, 2);
     if (rc) return rc;
     if (g.n_patches == 0) return SOM_OK;
     if (variant == SOM_BMU_AUTO) variant = som_bmu_pick_variant(g.n_patches, g.D, K);
-    SOM_REQUIRE(is_tc(variant), SOM_E_UNSUPPORTED, "bmu(f16): the FFMA variant does not read fp16 input");
-    return launch_bmu_tc_f16(x, g, W, c_norm2, K, unit_offset, out_idx, out_rd, stage_rows, ws, ws_bytes,
-                             arith_of(variant), (cudaStream_t)stream);
+    SOM_REQUIRE(is_tc(variant), SOM_E_UNSUPPORTED, "%s: the FFMA variant does not read 16-bit input", who);
+    return launch_bmu_tc_16(x, elem, g, W, c_norm2, K, unit_offset, out_idx, out_rd, stage_rows, ws, ws_bytes,
+                            arith_of(variant), (cudaStream_t)stream);
+}
+
+extern "C" int som_bmu_stage_nchw_f16(const void* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                      const float* W, const float* c_norm2, int K, int64_t unit_offset,
+                                      int64_t* out_idx, float* out_rd, float* stage_rows,
+                                      void* ws, size_t ws_bytes, int variant, void* stream) {
+    return bmu_stage_nchw_16("bmu(f16)", ELEM_F16, x, n_img, C, H, Wd, pH, pW, W, c_norm2, K, unit_offset, out_idx,
+                             out_rd, stage_rows, ws, ws_bytes, variant, stream);
+}
+
+extern "C" int som_bmu_stage_nchw_bf16(const void* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                       const float* W, const float* c_norm2, int K, int64_t unit_offset,
+                                       int64_t* out_idx, float* out_rd, float* stage_rows,
+                                       void* ws, size_t ws_bytes, int variant, void* stream) {
+    return bmu_stage_nchw_16("bmu(bf16)", ELEM_BF16, x, n_img, C, H, Wd, pH, pW, W, c_norm2, K, unit_offset, out_idx,
+                             out_rd, stage_rows, ws, ws_bytes, variant, stream);
 }
 
 extern "C" int som_bmu_flat_f32(const float* patches, int64_t n, int D, const float* W, const float* c_norm2, int K,

@@ -25,7 +25,7 @@ int launch_bmu_tc_s(const float* x, const Geom& g, const float* W, const float* 
 // som_bmu_tc_l16.cu
 bool tc_l16_applicable(int64_t n_patches, int D, int K, bool force);
 size_t tc_l16_workspace_bytes(int64_t n_patches, int D, int K, bool force);
-int launch_bmu_tc_l16(const void* x, bool x_f16, const Geom& g, const float* W, const float* cn, int K,
+int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K,
                       int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
                       bool force, cudaStream_t st);
 // som_bmu_tc_l.cu
@@ -71,18 +71,18 @@ bool tc_can_stage(int64_t n_patches, int D, int K, int arith) {
     return tc_supported(n_patches, D, K) && !tc_s_applicable(D) && use_l16(n_patches, D, K, arith);
 }
 
-// the kernels that read a binary16 batch themselves (som_bmu_stage_nchw_f16): the FP16-split kernel of 16 < D <= 256
-// (the same kernel as the one that stages)
+// the kernels that read a 16-bit batch (fp16 or bf16) themselves (som_bmu_stage_nchw_f16 / _bf16): the FP16-split
+// kernel of 16 < D <= 256 (the same kernel as the one that stages)
 bool tc_f16_native(int64_t n_patches, int D, int K, int arith) { return tc_can_stage(n_patches, D, K, arith); }
 
-int launch_bmu_tc_f16(const void* x, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
-                      int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes, int arith,
-                      cudaStream_t st) {
+int launch_bmu_tc_16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K,
+                     int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
+                     int arith, cudaStream_t st) {
     if (g.n_patches == 0) return SOM_OK;
     SOM_REQUIRE(tc_f16_native(g.n_patches, g.D, K, arith), SOM_E_UNSUPPORTED,
-                "bmu(f16): no kernel reads fp16 input at n=%lld D=%d K=%d (ask som_bmu_f16_native first)",
-                (long long)g.n_patches, g.D, K);
-    return launch_bmu_tc_l16(x, true, g, W, cn, K, unit_offset, out_idx, out_rd, stage, ws, ws_bytes, arith == 2, st);
+                "bmu(%s): no kernel reads 16-bit input at n=%lld D=%d K=%d (ask som_bmu_f16_native first)",
+                elem == ELEM_BF16 ? "bf16" : "f16", (long long)g.n_patches, g.D, K);
+    return launch_bmu_tc_l16(x, elem, g, W, cn, K, unit_offset, out_idx, out_rd, stage, ws, ws_bytes, arith == 2, st);
 }
 
 int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn, int K,
@@ -94,7 +94,7 @@ int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn
     if (tc_s_applicable(g.D))
         return launch_bmu_tc_s(x, g, W, cn, K, unit_offset, out_idx, out_rd, ws, ws_bytes, arith, st);
     if (use_l16(g.n_patches, g.D, K, arith))
-        return launch_bmu_tc_l16(x, false, g, W, cn, K, unit_offset, out_idx, out_rd, stage, ws, ws_bytes, arith == 2,
+        return launch_bmu_tc_l16(x, ELEM_F32, g, W, cn, K, unit_offset, out_idx, out_rd, stage, ws, ws_bytes, arith == 2,
                                  st);
     SOM_REQUIRE(arith != 2, SOM_E_UNSUPPORTED, "bmu: no FP16-split kernel for D=%d K=%d (SOM_BMU_TC_F16)", g.D, K);
     return launch_bmu_tc_l(x, g, W, cn, K, unit_offset, out_idx, out_rd, ws, ws_bytes, st);

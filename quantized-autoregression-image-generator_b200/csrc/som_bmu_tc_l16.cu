@@ -31,15 +31,24 @@
 //                             patch row; the N x K distance matrix never leaves TMEM
 // Bound: tensor pipe (FP16 rate / 3).
 //
-// FP16 input (T = __half, som_bmu_stage_nchw_f16): the builders read halves and upcast them exactly, so everything
-// from the row scale on sees the values x.float() would give.  When s_p x is itself exact in FP16 (fp16 data and a
-// row scale of at least 1 that no clamp lowered), lo(s_p x) is zero: every builder warp reports whether any lo of
-// its rows in a 64-feature block is non-zero, and the issuer drops the A_lo x B_hi group of that block when none is
-// (9 instead of 13 MMAs per tile at D = 64).  The dropped products are exact zeros; the fp32 instantiation never reads
-// the flag and keeps its MMA sequence.
+// 16-bit input (T = __half, som_bmu_stage_nchw_f16; T = __nv_bfloat16, som_bmu_stage_nchw_bf16): the builders read
+// the 16-bit values and widen them exactly, so everything from the row scale on sees the values x.float() would
+// give.  Where s_p x is itself exact in FP16, lo(s_p x) is zero: every builder warp reports whether any lo of its rows
+// in a 64-feature block is non-zero, and the issuer drops the A_lo x B_hi group of that block when none is (9 instead
+// of 13 MMAs per tile at D = 64).  The dropped products are exact zeros; the fp32 instantiation never reads the flag
+// and keeps its MMA sequence.
+//   fp16 : s_p x is exact whenever the row scale is at least 1 (row max below 128) and no clamp lowered it: such
+//          fp16 tiles never keep the third product.
+//   bf16 : an 8-bit significand, but fp32's exponent range.  With max |s_p x| in [64, 128) an element is exact in
+//          FP16 when its scaled exponent is at least -17 (its last significand bit then sits on FP16's 2^-24 grid),
+//          i.e. when it lies within about 2^-23 of its row's largest magnitude, and no clamp lowered the row scale.
+//          Tanh-range latents almost always pass.  So a bf16 tile MAY keep the third product where an fp16 tile of
+//          the same row maxima never does (an element further below its row max, a bf16 subnormal); the flag keeps
+//          it then, and the result stays exact.
 #include "som_common.cuh"
 #include "som_tc_ptx.cuh"
 
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 namespace som {
@@ -70,7 +79,7 @@ struct Params {
     int64_t unit_offset;
     int64_t* out_idx;
     float* out_rd;
-    const void* x;          // float or __half, per the kernel's T
+    const void* x;          // float, __half or __nv_bfloat16, per the kernel's T
     Geom g;
     const float* scale;     // [s_c, t_c] written by cb_scale_l_kernel earlier on the stream
     float* stage;           // optional patch-major copy of the patch rows (n_patches x D), written by the builders
@@ -90,7 +99,7 @@ struct Aux {
     float mrg_val[2][TM];
     int mrg_idx[2][TM];
     int row_exp[2][TM];
-    // FP16 input: per A slot one byte per builder warp (CG x 4, all in the leader CTA): "a lo of my rows is non-zero"
+    // 16-bit input: per A slot one byte per builder warp (CG x 4, all in the leader CTA): "a lo of my rows is non-zero"
     alignas(8) uint8_t lo_nz[NA_MAX][8];
 };
 constexpr uint32_t SMEM_BYTES = 1024 + TILES_BYTES + sizeof(Aux);
@@ -114,7 +123,7 @@ __device__ long long g_prof16[8];             // CTA 0's MMA loop: cycles, tiles
 // (block 0) the norm tail -- so the issuing thread pays ONE barrier wait and ONE commit per block instead of three.
 // With 13 MMAs per tile the issuing thread, not the tensor pipe, sets the pace otherwise (~48 cycles per MMA issue,
 // ~100 per barrier check, ~120 per commit).
-// exact fp32 values of 4 / 2 / 1 consecutive input elements (float or __half)
+// exact fp32 values of 4 / 2 / 1 consecutive input elements (float, __half or __nv_bfloat16)
 __device__ __forceinline__ void ld4(const float* p, float* o) {
     const float4 f = __ldg(reinterpret_cast<const float4*>(p));
     o[0] = f.x; o[1] = f.y; o[2] = f.z; o[3] = f.w;
@@ -135,11 +144,22 @@ __device__ __forceinline__ void ld2(const __half* p, float* o) {
 }
 __device__ __forceinline__ float ld1(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float ld1(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ void ld4(const __nv_bfloat16* p, float* o) {
+    const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
+    const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&r.x));
+    const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&r.y));
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
+}
+__device__ __forceinline__ void ld2(const __nv_bfloat16* p, float* o) {
+    const float2 f = __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162*>(p)));
+    o[0] = f.x; o[1] = f.y;
+}
+__device__ __forceinline__ float ld1(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
 
 template <int CG, bool MERGED, typename T>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_t, const Params P) {
-    constexpr bool F16 = sizeof(T) == 2;
+    constexpr bool IN16 = sizeof(T) == 2;          // a 16-bit input type (__half or __nv_bfloat16)
     pdl_launch_dependents();            // (the wait on the operand-split kernel comes after the barrier / TMEM prologue)
     extern __shared__ uint8_t smem_raw[];
     // 1024-byte alignment as an OFFSET into the shared array: rounding the pointer through uintptr_t made the compiler
@@ -175,7 +195,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
             mbar_init(&bars.acc_empty[a], EPI_WARPS * CG);
             mbar_init(&bars.exp_full[a], BUILD_WARPS);
         }
-        if (F16)
+        if (IN16)
             for (int s = 0; s < NA_MAX; ++s) *reinterpret_cast<uint64_t*>(aux.lo_nz[s]) = 0ull;
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -273,7 +293,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
         const bool prof = blockIdx.x == 0;
         long long w_acc = 0, w_b = 0, w_a = 0;
         const long long t_begin = clock64();
-        // F16: bit fb set = block fb of this job's patch tile has a non-zero lo (read once per job, at n == 0)
+        // IN16: bit fb set = block fb of this job's patch tile has a non-zero lo (read once per job, at n == 0)
         auto lo_flag = [&](int as) -> uint32_t {
             return *reinterpret_cast<volatile uint64_t*>(aux.lo_nz[as]) != 0ull ? 1u : 0u;
         };
@@ -293,7 +313,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                             c0 = prof ? clock64() : 0;
                             mma_wait(&bars.a_full[as], (uint32_t)(u / NA) & 1u);
                             if (prof) w_a += clock64() - c0;
-                            if (F16) lo_mask = (lo_mask & ~(1u << fb)) | (lo_flag(as) << fb);
+                            if (IN16) lo_mask = (lo_mask & ~(1u << fb)) | (lo_flag(as) << fb);
                         }
                         const uint64_t ahi = adesc0 + (uint32_t)as * A_SLOT_UNITS;
                         const uint64_t alo = ahi + A_LO_UNITS;
@@ -310,7 +330,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
                                 if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, bhi + 2u * k, 1u);
-                            if (!F16 || ((lo_mask >> fb) & 1u)) {
+                            if (!IN16 || ((lo_mask >> fb) & 1u)) {
 #pragma unroll
                                 for (int k = 0; k < 4; ++k)
                                     if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bhi + 2u * k, 1u);
@@ -331,7 +351,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                 if (n == 0) {                   // block 0 of this job (and with it the job's tail rows)
                     const int u = i * DB;
                     mma_wait(&bars.a_full[u % NA], (uint32_t)(u / NA) & 1u);
-                    if (F16) lo_mask = (lo_mask & ~1u) | lo_flag(u % NA);
+                    if (IN16) lo_mask = (lo_mask & ~1u) | lo_flag(u % NA);
                 }
                 tc_fence_after();
                 if (leader) {
@@ -345,7 +365,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     const int as = u % NA;
                     if (n == 0 && fb > 0) {
                         mma_wait(&bars.a_full[as], (uint32_t)(u / NA) & 1u);
-                        if (F16) lo_mask = (lo_mask & ~(1u << fb)) | (lo_flag(as) << fb);
+                        if (IN16) lo_mask = (lo_mask & ~(1u << fb)) | (lo_flag(as) << fb);
                     }
                     const uint64_t ahi = adesc0 + (uint32_t)as * A_SLOT_UNITS;
                     const uint64_t alo = ahi + A_LO_UNITS;
@@ -356,7 +376,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
 #pragma unroll
                         for (int k = 0; k < 4; ++k)
                             if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
-                        if (!F16 || ((lo_mask >> fb) & 1u)) {
+                        if (!IN16 || ((lo_mask >> fb) & 1u)) {
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
                                 if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
@@ -476,7 +496,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                         const float s = v[c * 8 + e] * sp;                   // exact
                         h[e] = __half2float(__float2half_rn(s));
                         l[e] = s - h[e];                                     // exact; rounded to FP16 when packed
-                        if (F16) lo_nz |= l[e] != 0.f;                       // (NaN counts as non-zero)
+                        if (IN16) lo_nz |= l[e] != 0.f;                       // (NaN counts as non-zero)
                     }
                     // 16-byte chunk c of row t lives at t * 128 + ((c ^ (t & 7)) << 4)
                     const uint32_t off = (((uint32_t)c) ^ sw) << 4;
@@ -492,10 +512,10 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     aux.row_exp[i & 1][t] = es;
                 }
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                const bool warp_lo_nz = F16 && __any_sync(0xffffffffu, lo_nz);
+                const bool warp_lo_nz = IN16 && __any_sync(0xffffffffu, lo_nz);
                 __syncwarp();
                 if (lane == 0) {
-                    if (F16) {
+                    if (IN16) {
                         // this warp's byte of the slot's flag, in the leader CTA; the release arrive below publishes it
                         uint8_t* fl = &aux.lo_nz[as][rank * BUILD_WARPS + (warp - BUILD_WARP0)];
                         if (CG == 2) {
@@ -730,10 +750,12 @@ size_t tc_l16_workspace_bytes(int64_t n_patches, int D, int K, bool force) {
     return tcl16::make_plan(&pl, n_patches, D, K, force) ? pl.total : 0;
 }
 
-int launch_bmu_tc_l16(const void* x, bool x_f16, const Geom& g, const float* W, const float* cn, int K,
+int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K,
                       int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
                       bool force, cudaStream_t st) {
     using namespace tcl16;
+    SOM_REQUIRE(elem == ELEM_F32 || elem == ELEM_F16 || elem == ELEM_BF16, SOM_E_BADARG, "bmu(tc f16): element type %d",
+                elem);
     const int64_t n = g.n_patches;
     if (n == 0) return SOM_OK;
     Plan pl;
@@ -775,14 +797,17 @@ int launch_bmu_tc_l16(const void* x, bool x_f16, const Geom& g, const float* W, 
     P.x = x; P.g = g; P.scale = scale; P.stage = stage;
 
     typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const Params);
-    static const KernelFn kernels[8] = {
+    // [elem][merged][cg - 1], elem = ELEM_F32 / ELEM_F16 / ELEM_BF16
+    static const KernelFn kernels[12] = {
         bmu_tc_l16_kernel<1, false, float>, bmu_tc_l16_kernel<2, false, float>,
         bmu_tc_l16_kernel<1, true, float>, bmu_tc_l16_kernel<2, true, float>,
         bmu_tc_l16_kernel<1, false, __half>, bmu_tc_l16_kernel<2, false, __half>,
-        bmu_tc_l16_kernel<1, true, __half>, bmu_tc_l16_kernel<2, true, __half>};
+        bmu_tc_l16_kernel<1, true, __half>, bmu_tc_l16_kernel<2, true, __half>,
+        bmu_tc_l16_kernel<1, false, __nv_bfloat16>, bmu_tc_l16_kernel<2, false, __nv_bfloat16>,
+        bmu_tc_l16_kernel<1, true, __nv_bfloat16>, bmu_tc_l16_kernel<2, true, __nv_bfloat16>};
     static PerDeviceFlag attr_done;
     if (attr_done.pending()) {
-        for (int c = 0; c < 8; ++c) {
+        for (int c = 0; c < 12; ++c) {
             cudaError_t e = cudaFuncSetAttribute(kernels[c], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
             if (e != cudaSuccess) { set_error("bmu(tc f16): smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
         }
@@ -805,7 +830,7 @@ int launch_bmu_tc_l16(const void* x, bool x_f16, const Geom& g, const float* W, 
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = pdl_enabled() ? 2 : 1;
-    cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[4 * (x_f16 ? 1 : 0) + 2 * pl.merged + pl.cg - 1], map_b, map_t, P);
+    cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[4 * elem + 2 * pl.merged + pl.cg - 1], map_b, map_t, P);
     if (le != cudaSuccess) { set_error("bmu_tc_l16_kernel: launch: %s", cudaGetErrorString(le)); return (int)le; }
     return check_launch("bmu_tc_l16_kernel");
 }

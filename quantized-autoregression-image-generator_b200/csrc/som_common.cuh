@@ -44,7 +44,11 @@ struct Geom {
     int vec;             // widest aligned vector (floats) along a patch row: 4, 2 or 1
 };
 
-// elem_bytes: 4 for an fp32 batch, 2 for a binary16 one (vec then counts halves)
+// element type of a feature-map batch: the BMU entry points and the FP16-split kernel's instantiations
+// (1 and 2 are also the dtype codes of the version-2 feature-map shards)
+enum ElemType : int { ELEM_F32 = 0, ELEM_F16 = 1, ELEM_BF16 = 2 };
+
+// elem_bytes: 4 for an fp32 batch, 2 for a 16-bit one (fp16 or bf16; vec then counts 16-bit elements)
 int make_geom(Geom* g, const void* x, int64_t n_img, int C, int H, int W, int pH, int pW, int elem_bytes = 4);
 
 __host__ __device__ __forceinline__ int64_t patch_base(const Geom& g, int64_t p) {

@@ -2,6 +2,7 @@
 // (codebook norms, candidate merge, hit histogram, quantise/gather, Adam, row compaction).
 #include "som_common.cuh"
 
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include <atomic>
@@ -74,7 +75,7 @@ int make_geom(Geom* g, const void* x, int64_t n_img, int C, int H, int W, int pH
     g->img_stride = (int64_t)C * H * W;
     uintptr_t a = (uintptr_t)x;
     if (elem_bytes == 2) {
-        SOM_REQUIRE((a & 1) == 0, SOM_E_BADARG, "geometry: fp16 buffer is not 2-byte aligned");
+        SOM_REQUIRE((a & 1) == 0, SOM_E_BADARG, "geometry: 16-bit buffer is not 2-byte aligned");
         g->vec = 1;
         if (pW % 4 == 0 && (a & 7) == 0) g->vec = 4;
         else if (pW % 2 == 0 && (a & 3) == 0) g->vec = 2;
@@ -602,10 +603,21 @@ __global__ void __launch_bounds__(256) gather_rows4_kernel(const float4* __restr
     }
 }
 
-// binary16 -> fp32 (exact), eight elements per step with 16-byte loads and stores when both buffers are 16-byte
-// aligned: the fp32 kernels read an fp16 batch through this copy (som_convert_f16_f32)
-__global__ void __launch_bounds__(256) convert_f16_f32_kernel(const __half* __restrict__ in, int64_t n,
-                                                              float* __restrict__ out, int vec8) {
+// exact widening of 16-bit values to fp32: two packed in a 32-bit word, or one
+__device__ __forceinline__ float2 widen2(uint32_t r, const __half*) {
+    return __half22float2(*reinterpret_cast<const __half2*>(&r));
+}
+__device__ __forceinline__ float2 widen2(uint32_t r, const __nv_bfloat16*) {
+    return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&r));
+}
+__device__ __forceinline__ float widen1(__half v) { return __half2float(v); }
+__device__ __forceinline__ float widen1(__nv_bfloat16 v) { return __bfloat162float(v); }
+
+// fp16 / bf16 -> fp32 (exact), eight elements per step with 16-byte loads and stores when both buffers are 16-byte
+// aligned: the fp32 kernels read a 16-bit batch through this copy (som_convert_f16_f32, som_convert_bf16_f32)
+template <typename T>
+__global__ void __launch_bounds__(256) convert_16_f32_kernel(const T* __restrict__ in, int64_t n,
+                                                             float* __restrict__ out, int vec8) {
     pdl_begin();
     const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -614,17 +626,14 @@ __global__ void __launch_bounds__(256) convert_f16_f32_kernel(const __half* __re
         const int64_t n8 = n >> 3;
         for (int64_t i = t; i < n8; i += stride) {
             const uint4 r = __ldcs(reinterpret_cast<const uint4*>(in) + i);
-            const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&r.x));
-            const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&r.y));
-            const float2 c = __half22float2(*reinterpret_cast<const __half2*>(&r.z));
-            const float2 d = __half22float2(*reinterpret_cast<const __half2*>(&r.w));
+            const float2 a = widen2(r.x, in), b = widen2(r.y, in), c = widen2(r.z, in), d = widen2(r.w, in);
             float4* o = reinterpret_cast<float4*>(out) + 2 * i;
             o[0] = make_float4(a.x, a.y, b.x, b.y);
             o[1] = make_float4(c.x, c.y, d.x, d.y);
         }
         done = n8 << 3;
     }
-    for (int64_t i = done + t; i < n; i += stride) out[i] = __half2float(in[i]);
+    for (int64_t i = done + t; i < n; i += stride) out[i] = widen1(in[i]);
 }
 
 static inline int grid_for(int64_t work_items, int threads, int per_sm) {
@@ -632,6 +641,18 @@ static inline int grid_for(int64_t work_items, int threads, int per_sm) {
     int64_t cap = (int64_t)sm_count() * per_sm;
     if (want < 1) want = 1;
     return (int)(want < cap ? want : cap);
+}
+
+template <typename T>
+static int convert_16_f32(const char* who, const void* in, int64_t n, float* out, void* stream) {
+    SOM_REQUIRE(n >= 0, SOM_E_BADARG, "%s: n=%lld", who, (long long)n);
+    if (n == 0) return SOM_OK;
+    SOM_REQUIRE(in && out, SOM_E_BADARG, "%s: null pointer", who);
+    SOM_REQUIRE((((uintptr_t)in) & 1) == 0 && (((uintptr_t)out) & 3) == 0, SOM_E_BADARG, "%s: misaligned buffer", who);
+    const int vec8 = ((((uintptr_t)in) | ((uintptr_t)out)) & 15) == 0 ? 1 : 0;
+    const int blocks = grid_for(vec8 ? ceil_div64(n, 8) : n, 256, 8);
+    launch_pdl(convert_16_f32_kernel<T>, blocks, 256, 0, (cudaStream_t)stream, (const T*)in, n, out, vec8);
+    return check_launch("convert_16_f32_kernel");
 }
 
 }  // namespace som
@@ -853,15 +874,11 @@ int som_adam_dp_f32(float* W, float* m, float* v, const float* g, int64_t n, int
 }
 
 int som_convert_f16_f32(const void* in, int64_t n, float* out, void* stream) {
-    SOM_REQUIRE(n >= 0, SOM_E_BADARG, "convert_f16_f32: n=%lld", (long long)n);
-    if (n == 0) return SOM_OK;
-    SOM_REQUIRE(in && out, SOM_E_BADARG, "convert_f16_f32: null pointer");
-    SOM_REQUIRE((((uintptr_t)in) & 1) == 0 && (((uintptr_t)out) & 3) == 0, SOM_E_BADARG,
-                "convert_f16_f32: misaligned buffer");
-    const int vec8 = ((((uintptr_t)in) | ((uintptr_t)out)) & 15) == 0 ? 1 : 0;
-    const int blocks = grid_for(vec8 ? ceil_div64(n, 8) : n, 256, 8);
-    launch_pdl(convert_f16_f32_kernel, blocks, 256, 0, (cudaStream_t)stream, (const __half*)in, n, out, vec8);
-    return check_launch("convert_f16_f32_kernel");
+    return convert_16_f32<__half>("convert_f16_f32", in, n, out, stream);
+}
+
+int som_convert_bf16_f32(const void* in, int64_t n, float* out, void* stream) {
+    return convert_16_f32<__nv_bfloat16>("convert_bf16_f32", in, n, out, stream);
 }
 
 int som_gather_rows_f32(const float* W, int D, const int64_t* keep, int64_t n_keep,

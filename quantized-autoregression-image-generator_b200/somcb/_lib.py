@@ -33,7 +33,11 @@ SIGNATURES = {
     "som_bmu_stage_nchw_f16": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int,
                                        c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p,
                                        c_void_p, c_size_t, c_int, c_void_p]),
+    "som_bmu_stage_nchw_bf16": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int,
+                                        c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p,
+                                        c_void_p, c_size_t, c_int, c_void_p]),
     "som_convert_f16_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
+    "som_convert_bf16_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "som_bmu_flat_f32": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p,
                                  c_void_p, c_size_t, c_int, c_void_p]),
     "som_backward_nchw_f32": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int,

@@ -6,8 +6,8 @@ Same constructor, attributes (``neighbourhood_range``, ``patch_dim``, ``image_di
 only), so train_codebook.py, prune_codebook.py and the tokenisation calls of
 train_quantized_transformer.py run unchanged.  The arithmetic runs in libsomcb:
 
-  get_patches_bmu        -> som_bmu_nchw_f32                 (models/Codebook.py:77-99; also fp16 feature maps,
-                                                              as if given x.float())
+  get_patches_bmu        -> som_bmu_nchw_f32                 (models/Codebook.py:77-99; also fp16 and bf16
+                                                              feature maps, as if given x.float())
   get_quantized_patches  -> som_filter_f32 + som_quantize    (:102-135, S = onehot(bmu) @ T)
   forward                -> the same with fused unpatchify    (:156-164)
   backward (autograd)    -> som_accumulate_nchw_f32 + som_filter_f32
@@ -147,7 +147,7 @@ class Codebook(nn.Module):
 
     def _input(self, x, require_cuda=True, allow_half=False):
         """(contiguous x, geometry).  fp32 only, except where ``allow_half``: the search and the fast-path trainer
-        also take fp16 feature maps (results as on ``x.float()``); the autograd path does not."""
+        also take fp16 and bf16 feature maps (results as on ``x.float()``); the autograd path does not."""
         if x.dim() != 4:
             raise Exception("Expected a (N, C, H, W) feature map.")
         w = self.codebook.weight
@@ -156,7 +156,7 @@ class Codebook(nn.Module):
                                "and its input to the GPU -- there is no CPU fallback")
         if x.device != w.device:
             raise RuntimeError(f"input on {x.device} but codebook on {w.device}")
-        if x.dtype != torch.float32 and not (allow_half and x.dtype == torch.float16):
+        if x.dtype != torch.float32 and not (allow_half and x.dtype in ops.HALF_DTYPES):
             raise TypeError(f"expected float32 feature maps, got {x.dtype}")
         x = x.detach().contiguous()
         geom = ops.geometry(x.shape, self.patch_dim)

@@ -9,8 +9,10 @@ large, memory-mappable shards and streams them into pinned batches:
     shard file  = 64-byte header | n * C*H*W values, C-contiguous (the reference's layout)
     header v1   = b"SOMFMAP1" | u32 version = 1 | u32 C | u32 H | u32 W | u64 n | zero padding to 64 bytes
                   (float32 values, the reference's dtype)
-    header v2   = the same with version = 2 and a u32 dtype code at byte 32 (1 = float16): half the bytes to
-                  read and to copy to the device; the searches treat the values as what they are (as ``.float()``)
+    header v2   = the same with version = 2 and a u32 dtype code at byte 32 (1 = float16, 2 = bfloat16): half
+                  the bytes to read and to copy to the device; the searches treat the values as what they are (as
+                  ``.float()``).  bfloat16 values are stored as their raw 16-bit patterns (numpy has no bfloat16:
+                  they are read through ``np.uint16`` and handed out as ``torch.bfloat16`` tensors)
 
 * ``convert_reference_dataset`` reads the reference layout (TinyDB json -> ``fmap_path`` entries, in
   document order) and writes shards; ``image_path`` is kept in a side ``index.json``.
@@ -28,11 +30,28 @@ MAGIC = b"SOMFMAP1"
 HEADER_BYTES = 64
 VERSION = 1                       # float32 shards
 VERSION_DTYPE = 2                 # shards of another dtype: u32 code at byte 32
-DTYPE_CODES = {1: np.dtype(np.float16)}
+DTYPE_CODES = {1: torch.float16, 2: torch.bfloat16}
+# how the values of each dtype are stored and memory-mapped
+_STORAGE = {torch.float32: np.dtype(np.float32), torch.float16: np.dtype(np.float16),
+            torch.bfloat16: np.dtype(np.uint16)}
+_FROM_NUMPY = {np.dtype(np.float32): torch.float32, np.dtype(np.float16): torch.float16}
+
+
+def _shard_dtype(dtype):
+    """The torch dtype of a shard dtype given as a torch dtype or as anything ``np.dtype`` takes."""
+    t = dtype if isinstance(dtype, torch.dtype) else None
+    if t is None:
+        try:
+            t = _FROM_NUMPY.get(np.dtype(dtype))
+        except TypeError:
+            pass
+    if t not in _STORAGE:
+        raise ValueError(f"shards hold float32, float16 or bfloat16 values, not {dtype}")
+    return t
 
 
 def _header(c, h, w, n, dtype):
-    if dtype == np.float32:
+    if dtype == torch.float32:
         head = MAGIC + struct.pack("<IIIIQ", VERSION, c, h, w, n)
     else:
         code = next(k for k, v in DTYPE_CODES.items() if v == dtype)
@@ -47,7 +66,7 @@ def _read_header(path):
         raise ValueError(f"{path}: not a feature-map shard")
     version, c, h, w, n = struct.unpack("<IIIIQ", head[8:32])
     if version == VERSION:
-        dtype = np.dtype(np.float32)
+        dtype = torch.float32
     elif version == VERSION_DTYPE:
         (code,) = struct.unpack("<I", head[32:36])
         if code not in DTYPE_CODES:
@@ -55,7 +74,7 @@ def _read_header(path):
         dtype = DTYPE_CODES[code]
     else:
         raise ValueError(f"{path}: shard version {version}, expected {VERSION} or {VERSION_DTYPE}")
-    expect = HEADER_BYTES + n * c * h * w * dtype.itemsize
+    expect = HEADER_BYTES + n * c * h * w * _STORAGE[dtype].itemsize
     if os.path.getsize(path) != expect:
         raise ValueError(f"{path}: size {os.path.getsize(path)} != {expect} implied by the header")
     return c, h, w, n, dtype
@@ -66,23 +85,44 @@ def read_header(path):
     return _read_header(path)[:4]
 
 
-def shard_dtype(path):
-    """numpy dtype of a shard's values (float32 for version 1)."""
+def shard_torch_dtype(path):
+    """torch dtype of a shard's values: float32, float16 or bfloat16."""
     return _read_header(path)[4]
 
 
-def _check_dtype(dtype):
-    dtype = np.dtype(dtype)
-    if dtype != np.float32 and dtype not in DTYPE_CODES.values():
-        raise ValueError(f"shards hold float32 or float16 values, not {dtype}")
-    return dtype
+def shard_dtype(path):
+    """numpy dtype of a shard's values (float32 for version 1, or float16).  numpy has no bfloat16: a bfloat16 shard
+    raises ``ValueError`` (ask ``shard_torch_dtype``)."""
+    dtype = shard_torch_dtype(path)
+    if dtype == torch.bfloat16:
+        raise ValueError(f"{path}: a bfloat16 shard has no numpy dtype; use shard_torch_dtype")
+    return _STORAGE[dtype]
+
+
+def _numpy_view(t):
+    """numpy view of a CPU tensor's storage (the raw 16-bit patterns for bfloat16)."""
+    return t.view(torch.int16).numpy().view(np.uint16) if t.dtype == torch.bfloat16 else t.numpy()
+
+
+def _bf16_bits(fmaps):
+    """bfloat16 bit patterns of ``fmaps``: a bfloat16 tensor as it is, anything else rounded from float32 to nearest
+    even (torch's conversion)."""
+    if isinstance(fmaps, torch.Tensor) and fmaps.dtype == torch.bfloat16:
+        t = fmaps.detach().cpu()
+    else:
+        t = torch.from_numpy(np.ascontiguousarray(np.asarray(fmaps), dtype=np.float32)).to(torch.bfloat16)
+    return _numpy_view(t.contiguous())
 
 
 def write_shard(path, fmaps, dtype=np.float32):
-    """fmaps: (n, C, H, W) array-like, stored as ``dtype`` (float32: version 1, float16: version 2; values are
-    rounded to nearest by numpy's conversion).  Returns n."""
-    dtype = _check_dtype(dtype)
-    arr = np.ascontiguousarray(np.asarray(fmaps), dtype=dtype)
+    """fmaps: (n, C, H, W) array-like, stored as ``dtype`` (float32: version 1; float16 or torch.bfloat16: version 2).
+    float16 values are rounded to nearest by numpy's conversion; bfloat16 values are the float32 values rounded to
+    nearest even by torch's (a bfloat16 tensor is stored as it is).  Returns n."""
+    dtype = _shard_dtype(dtype)
+    if dtype == torch.bfloat16:
+        arr = _bf16_bits(fmaps)
+    else:
+        arr = np.ascontiguousarray(np.asarray(fmaps), dtype=_STORAGE[dtype])
     if arr.ndim != 4:
         raise ValueError("write_shard expects (n, C, H, W)")
     n, c, h, w = arr.shape
@@ -105,10 +145,13 @@ def reference_entries(db_json_path):
 
 
 def convert_reference_dataset(db_json_path, out_dir, fmaps_per_shard=65536, path_root=None, dtype=np.float32):
-    """Pack the reference's per-file dataset into shards of ``dtype`` (float32 or float16, see ``write_shard``).
+    """Pack the reference's per-file dataset into shards of ``dtype`` (float32, float16 or torch.bfloat16, see
+    ``write_shard``).
     ``path_root`` re-bases relative ``fmap_path`` entries.  Returns the list of shard paths; writes ``index.json``
     beside them."""
-    dtype = _check_dtype(dtype)
+    dtype = _shard_dtype(dtype)
+    # bfloat16: the reference's .float() first, then one rounding in write_shard
+    load_as = np.float32 if dtype == torch.bfloat16 else _STORAGE[dtype]
     entries = reference_entries(db_json_path)
     os.makedirs(out_dir, exist_ok=True)
     shards, index, batch = [], [], []
@@ -127,7 +170,7 @@ def convert_reference_dataset(db_json_path, out_dir, fmaps_per_shard=65536, path
             p = os.path.join(path_root, p)
         with open(p, "rb") as f:
             fmap = np.load(f, allow_pickle=False)           # as feature_map_dataset.py:38-39
-        batch.append(np.asarray(fmap, dtype=dtype))         # .float() of :42 (float16: one rounding)
+        batch.append(np.asarray(fmap, dtype=load_as))       # .float() of :42 (float16: one rounding)
         index.append({"i": i, "shard": len(shards), "row": len(batch) - 1,
                       "image_path": doc.get("image_path")})
         if len(batch) == fmaps_per_shard:
@@ -148,18 +191,19 @@ class ShardReader:
             raise Exception("No data found.")
         self.paths = list(shard_paths)
         self.shape = None
-        self.dtype = None             # numpy dtype of every shard (batches come in it)
+        self.torch_dtype = None       # dtype of every shard (batches come in it)
         self.counts = []
         for p in self.paths:
             c, h, w, n, dt = _read_header(p)
             if self.shape is None:
-                self.shape, self.dtype = (c, h, w), dt
+                self.shape, self.torch_dtype = (c, h, w), dt
             elif self.shape != (c, h, w):
                 raise ValueError(f"{p}: shape {(c, h, w)} differs from {self.shape}")
-            elif self.dtype != dt:
-                raise ValueError(f"{p}: dtype {dt} differs from {self.dtype}")
+            elif self.torch_dtype != dt:
+                raise ValueError(f"{p}: dtype {dt} differs from {self.torch_dtype}")
             self.counts.append(n)
-        self._torch_dtype = torch.float16 if self.dtype == np.float16 else torch.float32
+        # numpy dtype of the shards' values (None for bfloat16, which numpy lacks)
+        self.dtype = None if self.torch_dtype == torch.bfloat16 else _STORAGE[self.torch_dtype]
         self.batch = int(batch_fmaps)
         self.pin = bool(pin) and torch.cuda.is_available()
         self.depth = int(depth)
@@ -180,16 +224,16 @@ class ShardReader:
 
     def _map(self, i):
         c, h, w = self.shape
-        return np.memmap(self.paths[i], dtype=self.dtype, mode="r", offset=HEADER_BYTES,
+        return np.memmap(self.paths[i], dtype=_STORAGE[self.torch_dtype], mode="r", offset=HEADER_BYTES,
                          shape=(self.counts[i], c, h, w))
 
     def read_all(self):
         """All feature maps as one (N, C, H, W) tensor of the shards' dtype (pinned when CUDA is present)."""
         c, h, w = self.shape
-        out = torch.empty(len(self), c, h, w, dtype=self._torch_dtype, pin_memory=self.pin)
+        out = torch.empty(len(self), c, h, w, dtype=self.torch_dtype, pin_memory=self.pin)
         lo = 0
         for i, n in enumerate(self.counts):
-            out[lo:lo + n].numpy()[...] = self._map(i)
+            _numpy_view(out[lo:lo + n])[...] = self._map(i)
             lo += n
         return out
 
@@ -198,7 +242,7 @@ class ShardReader:
         that stays valid until ``depth`` further batches have been produced."""
         c, h, w = self.shape
         if self._bufs is None:
-            self._bufs = [torch.empty(self.batch, c, h, w, dtype=self._torch_dtype, pin_memory=self.pin)
+            self._bufs = [torch.empty(self.batch, c, h, w, dtype=self.torch_dtype, pin_memory=self.pin)
                           for _ in range(self.depth)]
         k, lo = 0, 0
         for i, n in enumerate(self.counts):
@@ -210,7 +254,7 @@ class ShardReader:
                 if ev is not None:
                     ev.synchronize()              # an earlier DMA out of this pinned slot is still pending
                 buf = self._bufs[slot]
-                buf[:b - a].numpy()[...] = mm[a:b]
+                _numpy_view(buf[:b - a])[...] = mm[a:b]
                 self._last_slot = slot
                 yield lo + a, lo + b, buf[:b - a]
                 k += 1

@@ -71,9 +71,8 @@ class HostTokenizer:
 
     @torch.no_grad()
     def tokenize(self, fmaps_host, out_host=None, sync=True):
-        """fmaps_host: (N, C, H, W) fp32 or fp16 host tensor (pinned for async copies; an fp16 batch is copied as
-        fp16, half the bytes, and searched as if it were ``fmaps_host.float()``).  Returns the
-        (N, Seq) int64 host tensor of BMU indices (``out_host`` if given, pinned otherwise).
+        """fmaps_host: (N, C, H, W) fp32, fp16 or bf16 host tensor (pinned for async copies; a 16-bit batch is copied
+        as it is, half the bytes, and searched as if it were ``fmaps_host.float()``).  Returns the (N, Seq) int64 host tensor of BMU indices (``out_host`` if given, pinned otherwise).
 
         With ``sync=True`` (default) the call returns only after the last device-to-host copy has landed and the
         last host-to-device copy has been read: the returned indices are valid and ``fmaps_host`` may be refilled.
@@ -85,7 +84,7 @@ class HostTokenizer:
         seq = _ops.n_patches_of(geom1)
         if out_host is None:
             out_host = torch.empty(n, seq, dtype=torch.int64, pin_memory=True)
-        dtype = torch.float16 if fmaps_host.dtype == torch.float16 else torch.float32
+        dtype = fmaps_host.dtype if fmaps_host.dtype in _ops.HALF_DTYPES else torch.float32
         slots, (s_in, s_out) = self._alloc(c, h, w, seq, dtype)
         compute = torch.cuda.current_stream(self.device)
         weight = cb.codebook.weight.detach()
@@ -166,11 +165,11 @@ class HostTrainer:
 
     @torch.no_grad()
     def step(self, fmaps_host):
-        """Enqueue copy + step for one (local) host batch (pinned for asynchronous copies; fp16 batches are staged as
-        fp16 and trained on as if they were ``fmaps_host.float()``); returns a PendingLoss.
+        """Enqueue copy + step for one (local) host batch (pinned for asynchronous copies; fp16 / bf16 batches are
+        staged as they are and trained on as if they were ``fmaps_host.float()``); returns a PendingLoss.
         ``fmaps_host`` may be refilled once ``h2d_done()`` of this call has completed (or after the loss is read)."""
         slots = self._alloc(fmaps_host.shape,
-                            torch.float16 if fmaps_host.dtype == torch.float16 else torch.float32)
+                            fmaps_host.dtype if fmaps_host.dtype in _ops.HALF_DTYPES else torch.float32)
         sl = slots[self._i % self.depth]
         self._i += 1
         compute = torch.cuda.current_stream(self.device)

@@ -93,41 +93,60 @@ def bmu_can_stage(geom, num_units, variant=SOM_BMU_AUTO):
 
 
 def bmu_f16_native(geom, num_units, variant=SOM_BMU_AUTO):
-    """Whether the BMU kernel for this shape reads an fp16 batch itself (otherwise ``bmu`` upcasts it first)."""
+    """Whether the BMU kernel for this shape reads a 16-bit batch (fp16 or bf16: the same kernel) itself (otherwise
+    ``bmu`` upcasts it first)."""
     return bool(_lib.load().som_bmu_f16_native(n_patches_of(geom), dim_of(geom), int(num_units), int(variant)))
 
 
-def upcast_f16(x, out=None):
-    """Exact fp32 copy of a contiguous fp16 CUDA tensor (som_convert_f16_f32); ``out``: optional fp32 destination of
-    the same number of elements."""
+# 16-bit feature-map dtypes: the C entry points of the exact fp32 copy and of the native search
+_HALF_ENTRIES = {torch.float16: ("som_convert_f16_f32", "som_bmu_stage_nchw_f16"),
+                 torch.bfloat16: ("som_convert_bf16_f32", "som_bmu_stage_nchw_bf16")}
+HALF_DTYPES = tuple(_HALF_ENTRIES)          # the feature-map dtypes the search takes besides fp32
+
+
+def _upcast(x, out, dtype):
     lib = _lib.load()
-    x = _req(x, torch.float16, "x")
+    x = _req(x, dtype, "x")
     if out is None:
         out = torch.empty(x.shape, dtype=torch.float32, device=x.device)
     out = _req(out, torch.float32, "out")
     if out.numel() != x.numel():
         raise ValueError("out must hold as many elements as x")
+    entry = _HALF_ENTRIES[dtype][0]
     with torch.cuda.device(x.device):
-        check("som_convert_f16_f32", lib.som_convert_f16_f32(_ptr(x), x.numel(), _ptr(out), _stream(x)))
+        check(entry, getattr(lib, entry)(_ptr(x), x.numel(), _ptr(out), _stream(x)))
     return out
+
+
+def upcast_f16(x, out=None):
+    """Exact fp32 copy of a contiguous fp16 CUDA tensor (som_convert_f16_f32); ``out``: optional fp32 destination of
+    the same number of elements."""
+    return _upcast(x, out, torch.float16)
+
+
+def upcast_bf16(x, out=None):
+    """Exact fp32 copy of a contiguous bf16 CUDA tensor (som_convert_bf16_f32); ``out``: optional fp32 destination of
+    the same number of elements."""
+    return _upcast(x, out, torch.bfloat16)
 
 
 def bmu(x, geom, weight, c_norm2=None, unit_offset=0, want_rd=False, variant=SOM_BMU_AUTO,
         out=None, stage=None):
-    """K1.  x: fp32 or fp16 contiguous buffer described by ``geom``.  Returns idx (n_patches,) int64
+    """K1.  x: fp32, fp16 or bf16 contiguous buffer described by ``geom``.  Returns idx (n_patches,) int64
     [and the reduced distance rd (n_patches,) fp32 when ``want_rd``].  ``stage``: optional (n_patches, D) fp32
     tensor that receives the patch-major copy of the patch rows (only where ``bmu_can_stage``).
 
-    An fp16 ``x`` gives exactly the results of the same call on ``x.float()``: the FP16-split kernel reads it
-    directly where ``bmu_f16_native`` says so, other shapes search an fp32 copy made by ``upcast_f16``."""
+    A 16-bit ``x`` gives exactly the results of the same call on ``x.float()``: the FP16-split kernel reads it
+    directly where ``bmu_f16_native`` says so, other shapes search an fp32 copy made by ``upcast_f16`` /
+    ``upcast_bf16``."""
     lib = _lib.load()
     w = _req(weight, torch.float32, "weight")
     k, d = w.shape
-    if isinstance(x, torch.Tensor) and x.dtype == torch.float16:
-        x = _req(x, torch.float16, "x")
+    if isinstance(x, torch.Tensor) and x.dtype in _HALF_ENTRIES:
+        x = _req(x, x.dtype, "x")
         if not bmu_f16_native(geom, k, variant):
-            return bmu(upcast_f16(x), geom, w, c_norm2, unit_offset, want_rd, variant, out, stage)
-        entry = "som_bmu_stage_nchw_f16"
+            return bmu(_upcast(x, None, x.dtype), geom, w, c_norm2, unit_offset, want_rd, variant, out, stage)
+        entry = _HALF_ENTRIES[x.dtype][1]
     else:
         x = _req(x, torch.float32, "x")
         entry = "som_bmu_stage_nchw_f32"

@@ -91,8 +91,9 @@ class SomTrainer:
 
     def _graph_step(self, feature_map):
         cb = self.cb
-        # an fp16 batch keeps its dtype in the static buffer (half the bytes to copy); anything else is copied as fp32
-        dtype = torch.float16 if feature_map.dtype == torch.float16 else torch.float32
+        # an fp16 / bf16 batch keeps its dtype in the static buffer (half the bytes to copy); anything else is copied as
+        # fp32
+        dtype = feature_map.dtype if feature_map.dtype in _default_ops.HALF_DTYPES else torch.float32
         alias = self._graph_alias and feature_map.is_contiguous() and feature_map.dtype == dtype
         key = (tuple(feature_map.shape), dtype, float(cb.neighbourhood_range), float(self.lr),
                feature_map.data_ptr() if alias else 0)
@@ -199,12 +200,13 @@ class SomTrainer:
         return can is not None and ops.n_patches_of(geom) > 0 and can(geom, cb.num_embeddings, cb.bmu_variant)
 
     def _half_input(self, x, geom, staged):
-        """An fp16 batch stays fp16 only where the step's search reads it itself and writes the fp32 staging rows that
-        the accumulation reads (``staged``: the step searches with the separate kernels; the staging kernel is the one
-        that reads halves).  Otherwise it is upcast once, exactly, and that copy feeds every kernel of the step."""
-        if x.dtype != torch.float16 or (staged and self._can_stage(geom)):
+        """An fp16 / bf16 batch keeps its dtype only where the step's search reads it itself and writes the fp32 staging
+        rows that the accumulation reads (``staged``: the step searches with the separate kernels; the staging kernel is
+        the one that reads 16-bit values).  Otherwise it is upcast once, exactly, and that copy feeds every kernel of
+        the step."""
+        if x.dtype not in _default_ops.HALF_DTYPES or (staged and self._can_stage(geom)):
             return x
-        return self.ops.upcast_f16(x)
+        return self.ops.upcast_bf16(x) if x.dtype == torch.bfloat16 else self.ops.upcast_f16(x)
 
     def _search(self, x, geom, w):
         """BMU search of the step.  Where the kernel can emit it, also the patch-major staging copy of the patch rows:
