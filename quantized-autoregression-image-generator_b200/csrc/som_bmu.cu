@@ -16,6 +16,7 @@ int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn
                   int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
                   int arith, cudaStream_t st);
 bool tc_f16_native(int64_t n_patches, int D, int K, int arith);
+int tc_plan_fields(int64_t n_patches, int D, int K, int arith, int64_t* f);
 int launch_bmu_tc_16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
                       int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes, int arith,
                       cudaStream_t st);
@@ -91,6 +92,28 @@ extern "C" int som_bmu_stage_nchw_f32(const float* x, int64_t n_img, int C, int 
     SOM_REQUIRE(stage_rows == nullptr, SOM_E_UNSUPPORTED, "bmu: the FFMA variant does not emit a staging copy");
     return launch_bmu_ffma(x, g, W, c_norm2, K, unit_offset, out_idx, out_rd, ws, ws_bytes,
                            (cudaStream_t)stream);
+}
+
+// debug: the kernel family and plan that a search of n patches of dimension D against K units runs with `variant`, as
+// PF_COUNT int64 fields (som_common.cuh: PlanField, -1 where a field does not apply); the first n_out are written.  Tests
+// use it to pin which regime a shape reaches.  The answers come from the dispatch and the planners themselves.  The
+// element type of the batch enters no plan: an fp16 / bf16 batch runs the same plan, read natively where
+// som_bmu_f16_native says so.  Not in somcb.h: a test hook, not part of the ABI.
+extern "C" SOM_API int som_debug_bmu_plan(int64_t n_patches, int D, int K, int variant, int64_t* out, int n_out) {
+    SOM_REQUIRE(n_patches > 0 && D > 0 && K > 0, SOM_E_BADARG, "bmu plan: n=%lld D=%d K=%d", (long long)n_patches, D, K);
+    SOM_REQUIRE(variant >= SOM_BMU_AUTO && variant <= SOM_BMU_TC_F16, SOM_E_BADARG, "bmu plan: variant=%d", variant);
+    SOM_REQUIRE(out != nullptr && n_out >= 0, SOM_E_BADARG, "bmu plan: output");
+    int64_t f[PF_COUNT];
+    for (int i = 0; i < PF_COUNT; ++i) f[i] = -1;
+    if (variant == SOM_BMU_AUTO) variant = som_bmu_pick_variant(n_patches, D, K);
+    if (is_tc(variant)) {
+        const int rc = tc_plan_fields(n_patches, D, K, arith_of(variant), f);
+        if (rc) return rc;
+    } else {
+        f[PF_FAMILY] = PLAN_FFMA;
+    }
+    for (int i = 0; i < n_out && i < PF_COUNT; ++i) out[i] = f[i];
+    return SOM_OK;
 }
 
 extern "C" int som_bmu_f16_native(int64_t n_patches, int D, int K, int variant) {

@@ -726,12 +726,30 @@ static void make_plan(Plan* pl, int64_t n, int D, int K) {
     pl->total = o;
 }
 
+// 0 split-K, 1 resident-A, 2 streamed
+static int plan_mode(const Plan& pl) { return pl.S > 1 ? 0 : (pl.DB <= NA ? 1 : 2); }
+
 }  // namespace tcl
 
 size_t tc_l_workspace_bytes(int64_t n_patches, int D, int K) {
     tcl::Plan pl;
     tcl::make_plan(&pl, n_patches, D, K);
     return pl.total;
+}
+
+// the plan of launch_bmu_tc_l for som_debug_bmu_plan (f: PF_COUNT fields, pre-filled with -1)
+void tc_l_plan_fields(int64_t n_patches, int D, int K, int64_t* f) {
+    tcl::Plan pl;
+    tcl::make_plan(&pl, n_patches, D, K);
+    f[PF_CG] = pl.cg;
+    f[PF_MODE] = tcl::plan_mode(pl);
+    f[PF_S] = pl.S;
+    f[PF_FB_PER_SPLIT] = pl.fb_per_split;
+    f[PF_U] = pl.U;
+    f[PF_CHUNK_ROWS] = pl.chunk_rows;
+    f[PF_NT] = pl.NT;
+    f[PF_DB] = pl.DB;
+    f[PF_MTILES] = pl.n_mtiles;
 }
 
 int launch_bmu_tc_l(const float* x, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
@@ -760,7 +778,7 @@ int launch_bmu_tc_l(const float* x, const Geom& g, const float* W, const float* 
     if (rc) return rc;
     rc = make_map2d(&map_t, Tp, (uint64_t)pl.K_pad, 8, 32, 8, box_rows, CU_TENSOR_MAP_SWIZZLE_32B);
     if (rc) return rc;
-    const int mode = pl.S > 1 ? 0 : (pl.DB <= NA ? 1 : 2);          // split-K, resident-A, streamed
+    const int mode = plan_mode(pl);
     float* Ap = (float*)((char*)ws + pl.off_a);
     map_a = map_b;                                                   // unused unless streamed
     if (mode == 2) {

@@ -750,6 +750,19 @@ size_t tc_l16_workspace_bytes(int64_t n_patches, int D, int K, bool force) {
     return tcl16::make_plan(&pl, n_patches, D, K, force) ? pl.total : 0;
 }
 
+// the plan of launch_bmu_tc_l16 for som_debug_bmu_plan (f: PF_COUNT fields, pre-filled with -1); false where no
+// FP16-split kernel covers the shape
+bool tc_l16_plan_fields(int64_t n_patches, int D, int K, bool force, int64_t* f) {
+    tcl16::Plan pl;
+    if (!tcl16::make_plan(&pl, n_patches, D, K, force)) return false;
+    f[PF_CG] = pl.cg;
+    f[PF_MERGED] = pl.merged;
+    f[PF_NT] = pl.NT;
+    f[PF_DB] = pl.DB;
+    f[PF_MTILES] = pl.n_mtiles;
+    return true;
+}
+
 int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K,
                       int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
                       bool force, cudaStream_t st) {

@@ -649,6 +649,26 @@ bool tc_s_f16_mode(int64_t n_patches, int arith) {
     return arith == 0 ? n_patches >= 65536 : arith == 2;
 }
 
+// Resident patch tiles per CTA.  Small batches: fewer resident tiles per CTA so that every SM gets a super-tile (a unit
+// tile then feeds fewer MMAs, but the sweep over the unit tiles is what bounds a small batch).
+static int patch_tiles(int64_t n_patches) { return (int)ceil_div64(n_patches, tc::TM); }
+static int unit_tiles(int K) { return (K + tc::TN - 1) / tc::TN; }
+
+static int tc_s_resident_tiles(int64_t n_patches) {
+    const int n_mtiles = patch_tiles(n_patches);
+    const int rr = (n_mtiles + sm_count() - 1) / sm_count();
+    return rr < 1 ? 1 : (rr > tcs::R ? tcs::R : rr);
+}
+
+// the plan of launch_bmu_tc_s for som_debug_bmu_plan (f: PF_COUNT fields, pre-filled with -1)
+void tc_s_plan_fields(int64_t n_patches, int K, int arith, int64_t* f) {
+    f[PF_ARITH] = tc_s_f16_mode(n_patches, arith) ? 1 : 0;
+    f[PF_CG] = 1;
+    f[PF_RR] = tc_s_resident_tiles(n_patches);
+    f[PF_NT] = unit_tiles(K);
+    f[PF_MTILES] = patch_tiles(n_patches);
+}
+
 int launch_bmu_tc_s(const float* x, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
                     int64_t* out_idx, float* out_rd, void* ws, size_t ws_bytes, int arith, cudaStream_t st) {
     using namespace tcs;
@@ -685,7 +705,7 @@ int launch_bmu_tc_s(const float* x, const Geom& g, const float* W, const float* 
     if (rc) return rc;
 
     Params P;
-    P.nks = Dp / 8; P.NT = K_pad / TN; P.n_mtiles = (int)ceil_div64(n, TM); P.rows = n;
+    P.nks = Dp / 8; P.NT = unit_tiles(K); P.n_mtiles = patch_tiles(n); P.rows = n;
     P.unit_offset = unit_offset; P.out_idx = out_idx; P.out_rd = out_rd;
     P.x = x; P.g = g; P.W = W; P.cn = cn; P.K = K; P.scale = scale;
     P.dbg = 0;
@@ -701,10 +721,7 @@ int launch_bmu_tc_s(const float* x, const Geom& g, const float* W, const float* 
         if (e != cudaSuccess) { set_error("bmu(tc): smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
         attr_done.set();
     }
-    // small batches: fewer resident tiles per CTA so that every SM gets a super-tile (a unit tile then feeds
-    // fewer MMAs, but the sweep over the unit tiles is what bounds a small batch)
-    int rr = (P.n_mtiles + sm_count() - 1) / sm_count();
-    P.Rr = rr < 1 ? 1 : (rr > R ? R : rr);
+    P.Rr = tc_s_resident_tiles(n);
     const int n_super = (P.n_mtiles + P.Rr - 1) / P.Rr;
     const int grid = n_super < sm_count() ? n_super : sm_count();
     if (f16) bmu_tc_s_kernel<true><<<grid, NUM_THREADS, SMEM_BYTES, st>>>(map_b, map_t, P);

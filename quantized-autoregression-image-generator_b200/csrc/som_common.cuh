@@ -48,6 +48,27 @@ struct Geom {
 // (1 and 2 are also the dtype codes of the version-2 feature-map shards)
 enum ElemType : int { ELEM_F32 = 0, ELEM_F16 = 1, ELEM_BF16 = 2 };
 
+// The BMU plan of a shape as som_debug_bmu_plan reports it (som_bmu.cu): one int64 per field, -1 where a field does not
+// apply to the kernel family.  The planners fill it in themselves (tc_plan_fields and below), so a test can assert
+// which regime a shape reaches without restating a rule.
+enum PlanFamily : int { PLAN_FFMA = 0, PLAN_S = 1, PLAN_L16 = 2, PLAN_L = 3 };
+enum PlanField : int {
+    PF_FAMILY,          // PlanFamily
+    PF_ARITH,           // operand split: 0 3xTF32, 1 FP16
+    PF_CG,              // CTAs per cluster (2: CTA pairs)
+    PF_MERGED,          // L16: one ring stage per 64-feature block (D <= 128)
+    PF_MODE,            // L: 0 split-K, 1 resident-A, 2 streamed
+    PF_S,               // L: feature splits
+    PF_FB_PER_SPLIT,    // L: feature blocks per split
+    PF_U,               // L: unit-tile splits
+    PF_CHUNK_ROWS,      // L streamed: patch rows per pre-split chunk
+    PF_NT,              // unit tiles
+    PF_DB,              // feature blocks (32 features in L, 64 in L16)
+    PF_RR,              // S: resident patch tiles per CTA
+    PF_MTILES,          // 128-patch tiles
+    PF_COUNT
+};
+
 // elem_bytes: 4 for an fp32 batch, 2 for a 16-bit one (fp16 or bf16; vec then counts 16-bit elements)
 int make_geom(Geom* g, const void* x, int64_t n_img, int C, int H, int W, int pH, int pW, int elem_bytes = 4);
 
