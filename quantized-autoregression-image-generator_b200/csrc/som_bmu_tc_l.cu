@@ -35,6 +35,7 @@
 // Bound: tensor pipe (TF32 rate / 3): 94.8 % active at C4, 87 % at C5, 58 % at C3 (profiles/).
 #include "som_common.cuh"
 #include "som_tc_ptx.cuh"
+#include "som_tc_split.cuh"
 
 #include <stdlib.h>
 
@@ -92,11 +93,6 @@ struct Aux {
 };
 constexpr uint32_t SMEM_BYTES = 1024 + TILES_BYTES + sizeof(Aux);
 
-__device__ __forceinline__ uint64_t umma_desc_sw32(uint32_t smem_addr) {
-    return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(256 >> 4) << 32) | (1ull << 46) |
-           (6ull << 61);
-}
-
 // SPLITK: partial-distance epilogue (feature axis split over CTAs).  ARES: the patch tile's operand blocks stay
 // resident in the two A slots for all unit tiles (D <= 64: one slot per 32-feature block) instead of streaming.
 // CG = 2: CTA pairs (cluster of two, cta_group::2).  Each CTA builds its own 128-patch A tile and loads HALF of
@@ -107,9 +103,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
 bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_t,
                 const __grid_constant__ CUtensorMap map_a, const Params P) {
     extern __shared__ uint8_t smem_raw[];
-    // 1024-byte alignment as an OFFSET into the shared array: rounding the pointer through uintptr_t made the compiler
-    // forget the address space, and every access below compiled to generic LD.E / ST.E (cuobjdump, round 2)
-    uint8_t* tiles = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+    uint8_t* tiles = aligned_tiles(smem_raw);
     // unit tiles fed by one A-slot fill: split-K jobs use both TMEM accumulators for two unit tiles at once, which
     // halves the builders' work per MMA (they are the bottleneck there); the other modes double-buffer one tile
     constexpr int NI = SPLITK ? 2 : 1;
@@ -140,29 +134,14 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
     if (D <= FOFF_MAX)
         for (int d = threadIdx.x; d < D; d += NUM_THREADS) aux.foff[d] = feat_off(P.g, d);
     if (threadIdx.x < TM) {
-        // constant tail operand: row t = [1 1 1 0 | 0 0 0 0] in the 32-byte swizzle (chunk ^= bit 2 of t)
-        const int t = threadIdx.x;
-        const uint32_t sw = (uint32_t)(t >> 2) & 1u;
-        float4* rowp = reinterpret_cast<float4*>(a_tail + t * 32);
-        rowp[sw] = make_float4(1.f, 1.f, 1.f, 0.f);
-        rowp[sw ^ 1u] = make_float4(0.f, 0.f, 0.f, 0.f);
+        write_tail_ones(a_tail, threadIdx.x);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
     if (CG == 2) {                      // barriers of both CTAs initialised before anything arrives remotely
         __syncthreads();
         cluster_sync_all();
     }
-    if (warp == 1) {
-        if (CG == 1) {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars.tmem_base)),
-                         "r"(512));
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars.tmem_base)),
-                         "r"(512));
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
-        }
-    }
+    if (warp == 1) tmem_alloc<CG>(&bars.tmem_base, 512);
     tc_fence_before();
     __syncthreads();
     if (CG == 2) cluster_sync_all();
@@ -270,8 +249,8 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                             mma_wait(&bars.t_full[ts], t_ph);
                             tc_fence_after();
                             if (leader) {
-                                tc_mma_tf32_cg<CG>(tmem_base + ((j + a) & 1u) * TN, atdesc, btdesc0 + (uint32_t)ts * T_UNITS, 0u);
-                                tc_commit_cg<CG>(&bars.t_empty[ts]);
+                                tc_mma<MmaKind::TF32, CG>(tmem_base + ((j + a) & 1u) * TN, atdesc, btdesc0 + (uint32_t)ts * T_UNITS, 0u);
+                                tc_commit<CG>(&bars.t_empty[ts]);
                             }
                             accum[a] = 1;
                             if (++ts == 2) { ts = 0; t_ph ^= 1; }
@@ -294,11 +273,11 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                             if (leader) {
 #pragma unroll
                                 for (int k = 0; k < 4; ++k)
-                                    if (k < nks) tc_mma_tf32_cg<CG>(d_addr, ahi + 2u * k, bd + 2u * k, accum[a] | (uint32_t)(k > 0));
+                                    if (k < nks) tc_mma<MmaKind::TF32, CG>(d_addr, ahi + 2u * k, bd + 2u * k, accum[a] | (uint32_t)(k > 0));
 #pragma unroll
                                 for (int k = 0; k < 4; ++k)
-                                    if (k < nks) tc_mma_tf32_cg<CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
-                                tc_commit_cg<CG>(&bars.b_empty[bs]);
+                                    if (k < nks) tc_mma<MmaKind::TF32, CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
+                                tc_commit<CG>(&bars.b_empty[bs]);
                             }
                             accum[a] = 1;
                             if (++bs == NB) { bs = 0; b_ph ^= 1; }
@@ -308,19 +287,19 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                             if (leader) {
 #pragma unroll
                                 for (int k = 0; k < 4; ++k)
-                                    if (k < nks) tc_mma_tf32_cg<CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
-                                tc_commit_cg<CG>(&bars.b_empty[bs]);
+                                    if (k < nks) tc_mma<MmaKind::TF32, CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
+                                tc_commit<CG>(&bars.b_empty[bs]);
                             }
                             if (++bs == NB) { bs = 0; b_ph ^= 1; }
                         }
                     }
-                    if (leader && (!ARES || n0 + ni >= nt1)) tc_commit_cg<CG>(&bars.a_empty[as]);
+                    if (leader && (!ARES || n0 + ni >= nt1)) tc_commit<CG>(&bars.a_empty[as]);
                     if (!ARES && ++as == NA) { as = 0; a_ph ^= 1; }
                 }
                 if (leader) {
 #pragma unroll
                     for (int a = 0; a < NI; ++a)
-                        if (a < ni) tc_commit_cg<CG>(&bars.acc_full[(j + a) & 1u]);
+                        if (a < ni) tc_commit<CG>(&bars.acc_full[(j + a) & 1u]);
                 }
                 j += (uint32_t)ni;
             }
@@ -353,33 +332,8 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                 }
                 return;
             }
-#pragma unroll
-            for (int c = 0; c < 8; ++c) {
-                const int d = fb * 32 + c * 4;
-                float tmp[4] = {0.f, 0.f, 0.f, 0.f};
-                if (ok && d < D && !(P.dbg & 1)) {
-                    if (vec == 4) {
-                        const int o = use_tab ? aux.foff[d] : feat_off(P.g, d);
-                        const float4 f = __ldg(reinterpret_cast<const float4*>(src + o));
-                        tmp[0] = f.x; tmp[1] = f.y; tmp[2] = f.z; tmp[3] = f.w;
-                    } else if (vec == 2) {
-                        const int o0 = use_tab ? aux.foff[d] : feat_off(P.g, d);
-                        const float2 f0 = __ldg(reinterpret_cast<const float2*>(src + o0));
-                        tmp[0] = f0.x; tmp[1] = f0.y;
-                        if (d + 2 < D) {
-                            const int o1 = use_tab ? aux.foff[d + 2] : feat_off(P.g, d + 2);
-                            const float2 f1 = __ldg(reinterpret_cast<const float2*>(src + o1));
-                            tmp[2] = f1.x; tmp[3] = f1.y;
-                        }
-                    } else {
-#pragma unroll
-                        for (int e = 0; e < 4; ++e)
-                            if (d + e < D) tmp[e] = __ldg(src + (use_tab ? aux.foff[d + e] : feat_off(P.g, d + e)));
-                    }
-                }
-#pragma unroll
-                for (int e = 0; e < 4; ++e) v[c * 4 + e] = tmp[e];
-            }
+            load_row(v, src, ok && !(P.dbg & 1), fb * 32, D, vec,
+                     [&](int d) { return use_tab ? aux.foff[d] : feat_off(P.g, d); });
         };
         // position in this CTA's (job, unit tile, feature block) stream
         int q = job0, n = 0, fb = 0, fb0 = 0, fb1 = 0;
@@ -437,10 +391,7 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
                 float4 hi, lo;
-                hi.x = tf32_rna(cur[4 * c]);     lo.x = tf32_rna(cur[4 * c] - hi.x);
-                hi.y = tf32_rna(cur[4 * c + 1]); lo.y = tf32_rna(cur[4 * c + 1] - hi.y);
-                hi.z = tf32_rna(cur[4 * c + 2]); lo.z = tf32_rna(cur[4 * c + 2] - hi.z);
-                hi.w = tf32_rna(cur[4 * c + 3]); lo.w = tf32_rna(cur[4 * c + 3] - hi.w);
+                tf32_split4(&cur[4 * c], hi, lo);
                 // 16-byte chunk q of row r lives at r * 128 + ((q ^ (r & 7)) << 4)
                 const uint32_t r = contig ? (uint32_t)(wrow0 + 4 * c + (lane >> 3)) : (uint32_t)t;
                 const uint32_t qk = contig ? (uint32_t)(lane & 7) : (uint32_t)c;
@@ -477,7 +428,6 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ((uint32_t)(lg * 32) << 16) + acc * TN;
                 const int col0 = n * TN;
-                uint32_t va[32], vb[32];
                 auto consume = [&](const uint32_t (&v)[32], int c) {
                     if (SPLITK) {
                         if (p < P.rows) {
@@ -493,26 +443,12 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                         if (mn < best) { best = mn; bidx = col0 + c * 32 + first_eq32(v, mn); }
                     }
                 };
-                tmem_ld32_issue(taddr, va);
-#pragma unroll
-                for (int c = 0; c < 8; c += 2) {
-                    tmem_ld_wait(va);
-                    tmem_ld32_issue(taddr + (c + 1) * 32, vb);
-                    consume(va, c);
-                    tmem_ld_wait(vb);
-                    if (c + 2 < 8) {
-                        tmem_ld32_issue(taddr + (c + 2) * 32, va);
-                    } else {
-                        // accumulator fully read: hand it back before the last reduction
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) {
-                            if (CG == 2) mbar_arrive_remote_relaxed(&bars.acc_empty[acc], 0);
-                            else mbar_arrive(&bars.acc_empty[acc]);
-                        }
+                tmem_drain<8>(taddr, consume, [&] {
+                    if (lane == 0) {
+                        if (CG == 2) mbar_arrive_remote_relaxed(&bars.acc_empty[acc], 0);
+                        else mbar_arrive(&bars.acc_empty[acc]);
                     }
-                    consume(vb, c + 1);
-                }
+                });
                 ++j;
             }
             if (!SPLITK && p < P.rows) {
@@ -532,8 +468,7 @@ bmu_tc_l_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
     if (CG == 2) cluster_sync_all();    // the peer may still multicast into / arrive on this CTA's shared memory
     if (warp == 1) {
         tc_fence_after();
-        if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
-        else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
+        tmem_dealloc<CG>(tmem_base, 512);
     }
 }
 
@@ -567,9 +502,7 @@ __global__ void __launch_bounds__(256) splitk_argmin_kernel(const float* __restr
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
-        const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-        const int oi = __shfl_xor_sync(0xffffffffu, bidx, o);
-        if (ov < best || (ov == best && oi < bidx)) { best = ov; bidx = oi; }
+        argmin_merge(best, bidx, __shfl_xor_sync(0xffffffffu, best, o), __shfl_xor_sync(0xffffffffu, bidx, o));
     }
     if (lane == 0) {
         // a non-finite patch row makes every sum NaN and no '<' fires: unit 0 of the shard, as torch.argmin over an
@@ -592,20 +525,17 @@ __global__ void __launch_bounds__(256) split_w_l_kernel(const float* __restrict_
     const int d = (int)(t - (int64_t)row * cols);
     float hi = 0.f, lo = 0.f;
     if (row < K && d < D) {
-        const float w = W[(int64_t)row * D + d];
-        const float h = tf32_rna(w);
-        hi = -2.0f * h;
-        lo = -2.0f * tf32_rna(w - h);
+        tf32_split(W[(int64_t)row * D + d], hi, lo);
+        hi *= -2.0f;
+        lo *= -2.0f;
     }
     Bp[(int64_t)row * 2 * cols + d] = hi;
     Bp[(int64_t)row * 2 * cols + cols + d] = lo;
     if (d < 8) {
         float out = 0.f;
         if (row < K) {
-            const float nrm = cn[row];
-            const float n1 = tf32_rna(nrm);
-            const float n2 = tf32_rna(nrm - n1);
-            const float n3 = tf32_rna(nrm - n1 - n2);
+            float n1, n2, n3;
+            tf32_norm_split3(cn[row], n1, n2, n3);
             out = (d == 0) ? n1 : (d == 1) ? n2 : (d == 2) ? n3 : 0.f;
         } else if (d == 0) {
             out = PAD_NORM;
@@ -647,10 +577,7 @@ __global__ void __launch_bounds__(256) split_x_l_kernel(const float* __restrict_
             if (d0 + e < g.D) v[e] = __ldg(src + feat_off(g, d0 + e));
     }
     float4 hi, lo;
-    hi.x = tf32_rna(v[0]); lo.x = tf32_rna(v[0] - hi.x);
-    hi.y = tf32_rna(v[1]); lo.y = tf32_rna(v[1] - hi.y);
-    hi.z = tf32_rna(v[2]); lo.z = tf32_rna(v[2] - hi.z);
-    hi.w = tf32_rna(v[3]); lo.w = tf32_rna(v[3] - hi.w);
+    tf32_split4(v, hi, lo);
     float* dst = Ap + pr * (int64_t)DB * 64 + d0;
     *reinterpret_cast<float4*>(dst) = hi;
     *reinterpret_cast<float4*>(dst + (int64_t)DB * 32) = lo;
@@ -759,21 +686,20 @@ int launch_bmu_tc_l(const float* x, const Geom& g, const float* W, const float* 
     if (n == 0) return SOM_OK;
     Plan pl;
     make_plan(&pl, n, g.D, K);
-    SOM_REQUIRE(ws != nullptr && ws_bytes >= pl.total, SOM_E_WORKSPACE, "bmu(tc): workspace %zu < required %zu",
-                ws_bytes, pl.total);
-    SOM_REQUIRE(((uintptr_t)ws & 255) == 0, SOM_E_BADARG, "bmu(tc): workspace must be 256-byte aligned");
+    int rc = check_workspace(ws, ws_bytes, pl.total, "bmu(tc)");
+    if (rc) return rc;
     float* Bp = (float*)((char*)ws + pl.off_b);
     float* Tp = (float*)((char*)ws + pl.off_t);
     float* Pp = (float*)((char*)ws + pl.off_p);
     {
         const int64_t items = (int64_t)pl.K_pad * pl.DB * 32;
         split_w_l_kernel<<<(unsigned)ceil_div64(items, 256), 256, 0, st>>>(W, cn, K, g.D, pl.DB, pl.K_pad, Bp, Tp);
-        int rc = check_launch("split_w_l_kernel");
+        rc = check_launch("split_w_l_kernel");
         if (rc) return rc;
     }
     CUtensorMap map_b, map_t, map_a;
     const uint32_t box_rows = TN / pl.cg;
-    int rc = make_map2d(&map_b, Bp, (uint64_t)pl.K_pad, (uint64_t)pl.DB * 64, (uint64_t)pl.DB * 64 * 4, 32, box_rows,
+    rc = make_map2d(&map_b, Bp, (uint64_t)pl.K_pad, (uint64_t)pl.DB * 64, (uint64_t)pl.DB * 64 * 4, 32, box_rows,
                         CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc) return rc;
     rc = make_map2d(&map_t, Tp, (uint64_t)pl.K_pad, 8, 32, 8, box_rows, CU_TENSOR_MAP_SWIZZLE_32B);
@@ -807,32 +733,15 @@ int launch_bmu_tc_l(const float* x, const Geom& g, const float* W, const float* 
         {bmu_tc_l_kernel<true, false, 2>, bmu_tc_l_kernel<false, true, 2>, bmu_tc_l_kernel<false, false, 2>}};
     static const char* names[3] = {"bmu_tc_l_kernel<splitk>", "bmu_tc_l_kernel<resident>", "bmu_tc_l_kernel<streamed>"};
     static PerDeviceFlag attr_done;
-    if (attr_done.pending()) {
-        for (int c = 0; c < 2; ++c)
-            for (int m = 0; m < 3; ++m) {
-                cudaError_t e = cudaFuncSetAttribute(kernels[c][m], cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                     (int)SMEM_BYTES);
-                if (e != cudaSuccess) { set_error("bmu(tc): smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-            }
-        attr_done.set();
-    }
+    rc = smem_opt_in(attr_done, &kernels[0][0], 6, (int)SMEM_BYTES, "bmu(tc)");
+    if (rc) return rc;
     auto launch = [&](const Params& Pl) -> int {
         const int n_jobs = ((Pl.n_mtiles + pl.cg - 1) / pl.cg) * pl.S * pl.U;
         const int max_groups = sm_count() / pl.cg;
         const int groups = n_jobs < max_groups ? n_jobs : max_groups;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(groups * pl.cg));
-        cfg.blockDim = dim3(NUM_THREADS);
-        cfg.dynamicSmemBytes = SMEM_BYTES;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)pl.cg;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[pl.cg - 1][mode], map_b, map_t, map_a, Pl);
+        // a cluster of cg CTAs, no PDL
+        cudaError_t le = launch_kernel(kernels[pl.cg - 1][mode], (unsigned)(groups * pl.cg), NUM_THREADS, SMEM_BYTES, st,
+                                       (unsigned)pl.cg, false, map_b, map_t, map_a, Pl);
         if (le != cudaSuccess) { set_error("%s: launch: %s", names[mode], cudaGetErrorString(le)); return (int)le; }
         return check_launch(names[mode]);
     };

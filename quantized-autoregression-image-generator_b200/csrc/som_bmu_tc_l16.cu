@@ -47,9 +47,7 @@
 //          it then, and the result stays exact.
 #include "som_common.cuh"
 #include "som_tc_ptx.cuh"
-
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
+#include "som_tc_split.cuh"
 
 namespace som {
 SOM_TRACE_TU(trace_set_l16)
@@ -104,67 +102,19 @@ struct Aux {
 };
 constexpr uint32_t SMEM_BYTES = 1024 + TILES_BYTES + sizeof(Aux);
 
-__device__ __forceinline__ uint64_t umma_desc_sw32(uint32_t smem_addr) {
-    return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(256 >> 4) << 32) | (1ull << 46) |
-           (6ull << 61);
-}
-
-// eight halves (one 16-byte swizzle chunk) from eight floats, round-to-nearest-even
-__device__ __forceinline__ uint4 pack_h8(float v0, float v1, float v2, float v3, float v4, float v5, float v6, float v7) {
-    __half2 a = __floats2half2_rn(v0, v1), b = __floats2half2_rn(v2, v3);
-    __half2 c = __floats2half2_rn(v4, v5), d = __floats2half2_rn(v6, v7);
-    return make_uint4(*reinterpret_cast<uint32_t*>(&a), *reinterpret_cast<uint32_t*>(&b),
-                      *reinterpret_cast<uint32_t*>(&c), *reinterpret_cast<uint32_t*>(&d));
-}
-
 __device__ long long g_prof16[8];             // CTA 0's MMA loop: cycles, tiles, cycles waiting (acc_empty, B, A)
 
 // MERGED (D <= 128): one ring stage carries everything a unit tile needs of one 64-feature block -- B_hi, B_lo and
 // (block 0) the norm tail -- so the issuing thread pays ONE barrier wait and ONE commit per block instead of three.
 // With 13 MMAs per tile the issuing thread, not the tensor pipe, sets the pace otherwise (~48 cycles per MMA issue,
 // ~100 per barrier check, ~120 per commit).
-// exact fp32 values of 4 / 2 / 1 consecutive input elements (float, __half or __nv_bfloat16)
-__device__ __forceinline__ void ld4(const float* p, float* o) {
-    const float4 f = __ldg(reinterpret_cast<const float4*>(p));
-    o[0] = f.x; o[1] = f.y; o[2] = f.z; o[3] = f.w;
-}
-__device__ __forceinline__ void ld4(const __half* p, float* o) {
-    const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
-    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&r.x));
-    const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&r.y));
-    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
-}
-__device__ __forceinline__ void ld2(const float* p, float* o) {
-    const float2 f = __ldg(reinterpret_cast<const float2*>(p));
-    o[0] = f.x; o[1] = f.y;
-}
-__device__ __forceinline__ void ld2(const __half* p, float* o) {
-    const float2 f = __half22float2(__ldg(reinterpret_cast<const __half2*>(p)));
-    o[0] = f.x; o[1] = f.y;
-}
-__device__ __forceinline__ float ld1(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float ld1(const __half* p) { return __half2float(__ldg(p)); }
-__device__ __forceinline__ void ld4(const __nv_bfloat16* p, float* o) {
-    const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
-    const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&r.x));
-    const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&r.y));
-    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
-}
-__device__ __forceinline__ void ld2(const __nv_bfloat16* p, float* o) {
-    const float2 f = __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162*>(p)));
-    o[0] = f.x; o[1] = f.y;
-}
-__device__ __forceinline__ float ld1(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
-
 template <int CG, bool MERGED, typename T>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_t, const Params P) {
     constexpr bool IN16 = sizeof(T) == 2;          // a 16-bit input type (__half or __nv_bfloat16)
     pdl_launch_dependents();            // (the wait on the operand-split kernel comes after the barrier / TMEM prologue)
     extern __shared__ uint8_t smem_raw[];
-    // 1024-byte alignment as an OFFSET into the shared array: rounding the pointer through uintptr_t made the compiler
-    // forget the address space, and every access below compiled to generic LD.E / ST.E (cuobjdump, round 2)
-    uint8_t* tiles = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+    uint8_t* tiles = aligned_tiles(smem_raw);
     constexpr int B_STAGE = B_BLK_BYTES / CG;       // this CTA's share of a 256-unit block
     constexpr int T_STAGE = TAIL_B_BYTES / CG;
     constexpr int M_STAGE = 2 * B_STAGE + T_STAGE;  // merged stage: [hi | lo | tail]
@@ -204,17 +154,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
         __syncthreads();
         cluster_sync_all();
     }
-    if (warp == 1) {
-        if (CG == 1) {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars.tmem_base)),
-                         "r"(512));
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars.tmem_base)),
-                         "r"(512));
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
-        }
-    }
+    if (warp == 1) tmem_alloc<CG>(&bars.tmem_base, 512);
     tc_fence_before();
     __syncthreads();
     if (CG == 2) cluster_sync_all();
@@ -325,25 +265,25 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                         const uint64_t blo = bhi + B_UNITS;
                         if (leader) {
                             if (fb == 0)
-                                tc_mma_f16_cg<CG>(d_addr, atdesc0 + (uint32_t)(i & 1) * TA_UNITS,
+                                tc_mma<MmaKind::F16, CG>(d_addr, atdesc0 + (uint32_t)(i & 1) * TA_UNITS,
                                                   umma_desc_sw32(smem_u32(b_ring + (size_t)bs * M_STAGE + 2 * B_STAGE)), 0u);
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
-                                if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, bhi + 2u * k, 1u);
+                                if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, ahi + 2u * k, bhi + 2u * k, 1u);
                             if (!IN16 || ((lo_mask >> fb) & 1u)) {
 #pragma unroll
                                 for (int k = 0; k < 4; ++k)
-                                    if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bhi + 2u * k, 1u);
+                                    if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, alo + 2u * k, bhi + 2u * k, 1u);
                             }
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
-                                if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, blo + 2u * k, 1u);
-                            tc_commit_cg<CG>(&bars.b_empty[bs]);
-                            if (n == P.NT - 1) tc_commit_cg<CG>(&bars.a_empty[as]);
+                                if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, ahi + 2u * k, blo + 2u * k, 1u);
+                            tc_commit<CG>(&bars.b_empty[bs]);
+                            if (n == P.NT - 1) tc_commit<CG>(&bars.a_empty[as]);
                         }
                         if (++bs == NB) { bs = 0; b_ph ^= 1; }
                     }
-                    if (leader) tc_commit_cg<CG>(&bars.acc_full[j & 1u]);
+                    if (leader) tc_commit<CG>(&bars.acc_full[j & 1u]);
                     ++j;
                     continue;
                 }
@@ -355,8 +295,8 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                 }
                 tc_fence_after();
                 if (leader) {
-                    tc_mma_f16_cg<CG>(d_addr, atdesc0 + (uint32_t)(i & 1) * TA_UNITS, btdesc0 + (uint32_t)ts * T_UNITS, 0u);
-                    tc_commit_cg<CG>(&bars.t_empty[ts]);
+                    tc_mma<MmaKind::F16, CG>(d_addr, atdesc0 + (uint32_t)(i & 1) * TA_UNITS, btdesc0 + (uint32_t)ts * T_UNITS, 0u);
+                    tc_commit<CG>(&bars.t_empty[ts]);
                 }
                 if (++ts == 2) { ts = 0; t_ph ^= 1; }
                 for (int fb = 0; fb < DB; ++fb) {
@@ -375,13 +315,13 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     if (leader) {
 #pragma unroll
                         for (int k = 0; k < 4; ++k)
-                            if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
+                            if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
                         if (!IN16 || ((lo_mask >> fb) & 1u)) {
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
-                                if (k < nks) tc_mma_f16_cg<CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
+                                if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
                         }
-                        tc_commit_cg<CG>(&bars.b_empty[bs]);
+                        tc_commit<CG>(&bars.b_empty[bs]);
                     }
                     if (++bs == NB) { bs = 0; b_ph ^= 1; }
                     mma_wait(&bars.b_full[bs], b_ph);
@@ -390,13 +330,13 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     if (leader) {
 #pragma unroll
                         for (int k = 0; k < 4; ++k)
-                            if (k < nks) tc_mma_f16_cg<CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
-                        tc_commit_cg<CG>(&bars.b_empty[bs]);
-                        if (n == P.NT - 1) tc_commit_cg<CG>(&bars.a_empty[as]);
+                            if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, ahi + 2u * k, bd + 2u * k, 1u);
+                        tc_commit<CG>(&bars.b_empty[bs]);
+                        if (n == P.NT - 1) tc_commit<CG>(&bars.a_empty[as]);
                     }
                     if (++bs == NB) { bs = 0; b_ph ^= 1; }
                 }
-                if (leader) tc_commit_cg<CG>(&bars.acc_full[j & 1u]);
+                if (leader) tc_commit<CG>(&bars.acc_full[j & 1u]);
                 ++j;
             }
         }
@@ -412,27 +352,8 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
         const uint32_t sw = (uint32_t)(t & 7);
         float v[64];
         // 64 features [64 fb, 64 fb + 64) of one patch row; zero beyond D and for padding rows
-        // (vec counts elements: 16- / 8-byte runs of floats, 8- / 4-byte runs of halves)
         auto load_blk = [&](const T* src, bool ok, int fb) {
-#pragma unroll
-            for (int c = 0; c < 16; ++c) {
-                const int d = fb * 64 + c * 4;
-                float tmp[4] = {0.f, 0.f, 0.f, 0.f};
-                if (ok && d < D) {
-                    if (vec == 4) {
-                        ld4(src + aux.foff[d], tmp);
-                    } else if (vec == 2) {
-                        ld2(src + aux.foff[d], tmp);
-                        if (d + 2 < D) ld2(src + aux.foff[d + 2], tmp + 2);
-                    } else {
-#pragma unroll
-                        for (int e = 0; e < 4; ++e)
-                            if (d + e < D) tmp[e] = ld1(src + aux.foff[d + e]);
-                    }
-                }
-#pragma unroll
-                for (int e = 0; e < 4; ++e) v[c * 4 + e] = tmp[e];
-            }
+            load_row(v, src, ok, fb * 64, D, vec, [&](int d) { return aux.foff[d]; });
         };
         int i = 0;
         for (int q = job0; q < n_jobs; q += job_stride, ++i) {
@@ -447,24 +368,9 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
 #pragma unroll
                 for (int e = 0; e < 64; ++e) mx = fmaxf(mx, fabsf(v[e]));
             }
-            // power-of-two row scale: max |s_p x| in [64, 128) as long as a_p = s_p / t_c is an exact FP16 power of
-            // two (2^-24 .. 2^15); an all-zero or non-finite row takes the ideal exponent 0
-            const int eb = (int)((__float_as_uint(mx) >> 23) & 0xffu);
-            int ep = 133 - eb;
-            if (!(mx > 0.f) || eb == 0xff) ep = 0;
-            int ka = ep - tc_exp, es;
-            float ap;
-            if (ka < -24) {
-                // |x| beyond ~2^24 |c|: ||c||^2 is below fp32 resolution of rd; keep the row in range instead
-                es = ep;
-                ap = 0.f;
-            } else {
-                ka = ka > 15 ? 15 : ka;                 // 2^-24 .. 2^15: exact in FP16 (subnormal below 2^-14)
-                es = ka + tc_exp;
-                ap = __uint_as_float((uint32_t)(127 + ka) << 23);
-            }
-            es = es > 120 ? 120 : (es < -120 ? -120 : es);
-            const float sp = __uint_as_float((uint32_t)(127 + es) << 23);
+            float sp, ap;
+            int es;
+            f16_row_scale(mx, tc_exp, sp, ap, es);
             for (int fb = 0; fb < DB; ++fb) {
                 if (DB > 1) load_blk(src, ok, fb);
                 if (P.stage != nullptr && ok) {
@@ -493,21 +399,20 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     float h[8], l[8];
 #pragma unroll
                     for (int e = 0; e < 8; ++e) {
-                        const float s = v[c * 8 + e] * sp;                   // exact
-                        h[e] = __half2float(__float2half_rn(s));
-                        l[e] = s - h[e];                                     // exact; rounded to FP16 when packed
+                        f16_split(v[c * 8 + e] * sp, h[e], l[e]);            // scaling exact
                         if (IN16) lo_nz |= l[e] != 0.f;                       // (NaN counts as non-zero)
                     }
                     // 16-byte chunk c of row t lives at t * 128 + ((c ^ (t & 7)) << 4)
                     const uint32_t off = (((uint32_t)c) ^ sw) << 4;
-                    *reinterpret_cast<uint4*>(hi_row + off) = pack_h8(h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7]);
-                    *reinterpret_cast<uint4*>(lo_row + off) = pack_h8(l[0], l[1], l[2], l[3], l[4], l[5], l[6], l[7]);
+                    *reinterpret_cast<uint4*>(hi_row + off) = pack_h8(h);
+                    *reinterpret_cast<uint4*>(lo_row + off) = pack_h8(l);
                 }
                 if (fb == 0) {
                     // tail row t = [a_p a_p a_p 0.. | 0..] in the 32-byte swizzle (chunk ^= bit 2 of t)
                     const uint32_t sw32 = (uint32_t)(t >> 2) & 1u;
                     uint4* rowp = reinterpret_cast<uint4*>(a_tail + (size_t)(i & 1) * TAIL_A_BYTES + t * 32);
-                    rowp[sw32] = pack_h8(ap, ap, ap, 0.f, 0.f, 0.f, 0.f, 0.f);
+                    const float tl[8] = {ap, ap, ap, 0.f, 0.f, 0.f, 0.f, 0.f};
+                    rowp[sw32] = pack_h8(tl);
                     rowp[sw32 ^ 1u] = make_uint4(0u, 0u, 0u, 0u);
                     aux.row_exp[i & 1][t] = es;
                 }
@@ -558,39 +463,23 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + ((uint32_t)(lg * 32) << 16) + acc * TN + (uint32_t)half * 128u;
                 const int col0 = n * TN + half * 128;
-                uint32_t va[32], vb[32];
                 auto consume = [&](const uint32_t (&vv)[32], int c) {
                     const float mn = min32(vv);
                     if (mn < best) { best = mn; bidx = col0 + c * 32 + first_eq32(vv, mn); }
                 };
-                tmem_ld32_issue(taddr, va);
-                tmem_ld_wait(va);
-                tmem_ld32_issue(taddr + 32, vb);
-                consume(va, 0);
-                tmem_ld_wait(vb);
-                tmem_ld32_issue(taddr + 64, va);
-                consume(vb, 1);
-                tmem_ld_wait(va);
-                tmem_ld32_issue(taddr + 96, vb);
-                consume(va, 2);
-                tmem_ld_wait(vb);
-                // accumulator fully read: hand it back before the last reduction
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) {
-                    if (CG == 2) mbar_arrive_remote_relaxed(&bars.acc_empty[acc], 0);
-                    else mbar_arrive(&bars.acc_empty[acc]);
-                }
-                consume(vb, 3);
+                tmem_drain<4>(taddr, consume, [&] {
+                    if (lane == 0) {
+                        if (CG == 2) mbar_arrive_remote_relaxed(&bars.acc_empty[acc], 0);
+                        else mbar_arrive(&bars.acc_empty[acc]);
+                    }
+                });
                 ++j;
             }
             // merge the two column halves (value asc, index asc); buffers alternate per job
             if (half == 1) { aux.mrg_val[i & 1][row] = best; aux.mrg_idx[i & 1][row] = bidx; }
             asm volatile("bar.sync 1, 256;" ::: "memory");
             if (half == 0 && p < P.rows) {
-                const float ov = aux.mrg_val[i & 1][row];
-                const int oi = aux.mrg_idx[i & 1][row];
-                if (ov < best || (ov == best && oi < bidx)) { best = ov; bidx = oi; }
+                argmin_merge(best, bidx, aux.mrg_val[i & 1][row], aux.mrg_idx[i & 1][row]);
                 P.out_idx[p] = (int64_t)bidx + P.unit_offset;
                 // the accumulator holds s_p s_c rd: undo both powers of two (exact)
                 if (P.out_rd) P.out_rd[p] = ldexpf(best, -(es + sc_exp));
@@ -603,8 +492,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
     if (CG == 2) cluster_sync_all();    // the peer may still multicast into / arrive on this CTA's shared memory
     if (warp == 1) {
         tc_fence_after();
-        if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
-        else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
+        tmem_dealloc<CG>(tmem_base, 512);
     }
 }
 
@@ -684,18 +572,18 @@ __global__ void __launch_bounds__(256) split_w_l16_kernel(const float* __restric
     float v0 = 0.f, v1 = 0.f;
     if (d < D) v0 = -2.0f * sc * W[(int64_t)src * D + d];                   // exact scaling
     if (d + 1 < D) v1 = -2.0f * sc * W[(int64_t)src * D + d + 1];
-    const float h0 = __half2float(__float2half_rn(v0)), h1 = __half2float(__float2half_rn(v1));
+    float h0, l0, h1, l1;
+    f16_split(v0, h0, l0);
+    f16_split(v1, h1, l1);
     const int64_t cols = (int64_t)DB * 64;
     __half* rowp = Bp + (int64_t)row * 2 * cols;
     *reinterpret_cast<__half2*>(rowp + d) = __floats2half2_rn(h0, h1);
-    *reinterpret_cast<__half2*>(rowp + cols + d) = __floats2half2_rn(v0 - h0, v1 - h1);
+    *reinterpret_cast<__half2*>(rowp + cols + d) = __floats2half2_rn(l0, l1);
     if (d < 16) {
         float o0 = 0.f, o1 = 0.f;
         if (d < 4) {
-            const float nrm = cn[src] * sc * tcs;
-            const float n1 = __half2float(__float2half_rn(nrm));
-            const float n2 = __half2float(__float2half_rn(nrm - n1));
-            const float n3 = nrm - n1 - n2;
+            float n1, n2, n3;
+            f16_norm_split3(cn[src] * sc * tcs, n1, n2, n3);
             if (d == 0) { o0 = n1; o1 = n2; } else { o0 = n3; o1 = 0.f; }
         }
         *reinterpret_cast<__half2*>(Tp + (int64_t)row * 16 + d) = __floats2half2_rn(o0, o1);
@@ -774,13 +662,11 @@ int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, co
     Plan pl;
     SOM_REQUIRE(make_plan(&pl, n, g.D, K, force), SOM_E_UNSUPPORTED, "bmu(tc f16): shape n=%lld D=%d K=%d not covered",
                 (long long)n, g.D, K);
-    SOM_REQUIRE(ws != nullptr && ws_bytes >= pl.total, SOM_E_WORKSPACE, "bmu(tc f16): workspace %zu < required %zu",
-                ws_bytes, pl.total);
-    SOM_REQUIRE(((uintptr_t)ws & 255) == 0, SOM_E_BADARG, "bmu(tc f16): workspace must be 256-byte aligned");
+    int rc = check_workspace(ws, ws_bytes, pl.total, "bmu(tc f16)");
+    if (rc) return rc;
     __half* Bp = (__half*)((char*)ws + pl.off_b);
     __half* Tp = (__half*)((char*)ws + pl.off_t);
     float* scale = (float*)((char*)ws + pl.off_s);
-    int rc;
     {
         const int64_t items = (int64_t)pl.K_pad * pl.DB * 32;
         const unsigned blocks = (unsigned)ceil_div64(items, 256);
@@ -819,31 +705,14 @@ int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, co
         bmu_tc_l16_kernel<1, false, __nv_bfloat16>, bmu_tc_l16_kernel<2, false, __nv_bfloat16>,
         bmu_tc_l16_kernel<1, true, __nv_bfloat16>, bmu_tc_l16_kernel<2, true, __nv_bfloat16>};
     static PerDeviceFlag attr_done;
-    if (attr_done.pending()) {
-        for (int c = 0; c < 12; ++c) {
-            cudaError_t e = cudaFuncSetAttribute(kernels[c], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
-            if (e != cudaSuccess) { set_error("bmu(tc f16): smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-        }
-        attr_done.set();
-    }
+    rc = smem_opt_in(attr_done, kernels, 12, (int)SMEM_BYTES, "bmu(tc f16)");
+    if (rc) return rc;
     const int n_jobs = (pl.n_mtiles + pl.cg - 1) / pl.cg;
     const int max_groups = sm_count() / pl.cg;
     const int groups = n_jobs < max_groups ? n_jobs : max_groups;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(groups * pl.cg));
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = SMEM_BYTES;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)pl.cg;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;     // (see som_common.cuh: pdl_begin)
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
-    cudaError_t le = cudaLaunchKernelEx(&cfg, kernels[4 * elem + 2 * pl.merged + pl.cg - 1], map_b, map_t, P);
+    // a cluster of cg CTAs, and PDL (see som_common.cuh: pdl_begin)
+    cudaError_t le = launch_kernel(kernels[4 * elem + 2 * pl.merged + pl.cg - 1], (unsigned)(groups * pl.cg), NUM_THREADS,
+                                   SMEM_BYTES, st, (unsigned)pl.cg, true, map_b, map_t, P);
     if (le != cudaSuccess) { set_error("bmu_tc_l16_kernel: launch: %s", cudaGetErrorString(le)); return (int)le; }
     return check_launch("bmu_tc_l16_kernel");
 }

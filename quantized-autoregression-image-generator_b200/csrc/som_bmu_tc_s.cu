@@ -34,8 +34,8 @@
 // Every streamed unit tile feeds R = 4 patch tiles.  Bound: tensor pipe (TF32 rate / 3).
 #include "som_common.cuh"
 #include "som_tc_ptx.cuh"
+#include "som_tc_split.cuh"
 
-#include <cuda_fp16.h>
 #include <stdlib.h>
 
 namespace som {
@@ -88,21 +88,7 @@ struct Aux {
 };
 constexpr uint32_t SMEM_BYTES = 1024 + TILES_BYTES + sizeof(Aux);
 
-// K-major SWIZZLE_32B operand descriptor: 32-byte rows, 8-row groups 256 B apart
-__device__ __forceinline__ uint64_t umma_desc_sw32(uint32_t smem_addr) {
-    return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(256 >> 4) << 32) | (1ull << 46) |
-           (6ull << 61);
-}
-
 __device__ long long g_prof[4];              // CTA 0: cycles of the MMA loop, tiles issued
-
-// eight halves (one 16-byte swizzle chunk) from eight floats, round-to-nearest-even
-__device__ __forceinline__ uint4 pack_h8(const float (&v)[8]) {
-    __half2 a = __floats2half2_rn(v[0], v[1]), b = __floats2half2_rn(v[2], v[3]);
-    __half2 c = __floats2half2_rn(v[4], v[5]), d = __floats2half2_rn(v[6], v[7]);
-    return make_uint4(*reinterpret_cast<uint32_t*>(&a), *reinterpret_cast<uint32_t*>(&b),
-                      *reinterpret_cast<uint32_t*>(&c), *reinterpret_cast<uint32_t*>(&d));
-}
 
 // F16 = true: the same pipeline with a two-way FP16 split instead of the TF32 one (kind::f16 MMAs have K = 16 at the
 // cycle cost of a K = 8 TF32 MMA: a tile is 4 MMAs instead of 7).  Rows are scaled by exact powers of two so that the
@@ -117,9 +103,7 @@ template <bool F16>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_t, const Params P) {
     extern __shared__ uint8_t smem_raw[];
-    // 1024-byte alignment as an OFFSET into the shared array: rounding the pointer through uintptr_t made the compiler
-    // forget the address space, and every access below compiled to generic LD.E / ST.E (cuobjdump, round 2)
-    uint8_t* tiles = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+    uint8_t* tiles = aligned_tiles(smem_raw);
     uint8_t* a_slots = tiles;
     uint8_t* a_tail = tiles + R * A_BLK_BYTES;
     uint8_t* ring = a_tail + TAIL_A_BYTES;
@@ -144,19 +128,10 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
             reinterpret_cast<uint4*>(a_slots)[i] = make_uint4(0u, 0u, 0u, 0u);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     } else if (threadIdx.x < TM) {
-        // constant tail operand: row t = [1 1 1 0 | 0 0 0 0] in the 32-byte swizzle (chunk ^= bit 2 of t)
-        const int t = threadIdx.x;
-        const uint32_t sw = (uint32_t)(t >> 2) & 1u;
-        float4* rowp = reinterpret_cast<float4*>(a_tail + t * 32);
-        rowp[sw] = make_float4(1.f, 1.f, 1.f, 0.f);
-        rowp[sw ^ 1u] = make_float4(0.f, 0.f, 0.f, 0.f);
+        write_tail_ones(a_tail, threadIdx.x);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars.tmem_base)),
-                     "r"(512));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    if (warp == 1) tmem_alloc(&bars.tmem_base, 512);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -212,25 +187,25 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                     if (F16) {
                         if (leader) {
                             // norm tail (k-step 2 of both rows) first, then hi.hi, lo.hi, hi.lo
-                            tc_mma_f16(d_addr, ad + 4u, bd + 4u, 0u);
-                            tc_mma_f16(d_addr, ad, bd, 1u);
-                            tc_mma_f16(d_addr, ad + 2u, bd, 1u);
-                            tc_mma_f16(d_addr, ad, bd + 2u, 1u);
+                            tc_mma<MmaKind::F16>(d_addr, ad + 4u, bd + 4u, 0u);
+                            tc_mma<MmaKind::F16>(d_addr, ad, bd, 1u);
+                            tc_mma<MmaKind::F16>(d_addr, ad + 2u, bd, 1u);
+                            tc_mma<MmaKind::F16>(d_addr, ad, bd + 2u, 1u);
                             tc_commit(&bars.acc_full[j & 1u]);
                             if (n == P.NT - 1) tc_commit(&bars.a_empty[r]);
                         }
                     } else if (leader) {
                         // norm tail first, then hi.hi, lo.hi, hi.lo
-                        tc_mma_tf32(d_addr, atdesc, btd, 0u);
+                        tc_mma<MmaKind::TF32>(d_addr, atdesc, btd, 0u);
 #pragma unroll
                         for (int ks = 0; ks < DMAX / 8; ++ks)
-                            if (ks < nks) tc_mma_tf32(d_addr, ad + 2u * ks, bd + 2u * ks, 1u);
+                            if (ks < nks) tc_mma<MmaKind::TF32>(d_addr, ad + 2u * ks, bd + 2u * ks, 1u);
 #pragma unroll
                         for (int ks = 0; ks < DMAX / 8; ++ks)
-                            if (ks < nks) tc_mma_tf32(d_addr, ad + 2u * (nks + ks), bd + 2u * ks, 1u);
+                            if (ks < nks) tc_mma<MmaKind::TF32>(d_addr, ad + 2u * (nks + ks), bd + 2u * ks, 1u);
 #pragma unroll
                         for (int ks = 0; ks < DMAX / 8; ++ks)
-                            if (ks < nks) tc_mma_tf32(d_addr, ad + 2u * ks, bd + 2u * (nks + ks), 1u);
+                            if (ks < nks) tc_mma<MmaKind::TF32>(d_addr, ad + 2u * ks, bd + 2u * (nks + ks), 1u);
                         tc_commit(&bars.acc_full[j & 1u]);
                         if (n == P.NT - 1) tc_commit(&bars.a_empty[r]);
                     }
@@ -254,20 +229,21 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
         const bool w4 = v4 && ((reinterpret_cast<uintptr_t>(P.W) & 15) == 0);
         const int tc_exp = F16 ? (int)((__float_as_uint(__ldg(P.scale + 1)) >> 23) & 0xffu) - 127 : 0;
         float xv[R][DMAX];
+        auto foff = [&](int d) { return aux.foff[d]; };
         auto prefetch = [&](int st_next) {
             const int r_nxt = (st_next < n_super) ? min(Rr, P.n_mtiles - st_next * Rr) : 0;
 #pragma unroll
             for (int r = 0; r < R; ++r) {
                 const int64_t p = (int64_t)(st_next * Rr + r) * TM + t;
                 const bool ok = (r < r_nxt) && (p < P.rows);
-                load_row<DMAX>(xv[r], P.x + (ok ? patch_base(P.g, p) : 0), ok, D, vec, aux.foff);
+                load_row(xv[r], P.x + (ok ? patch_base(P.g, p) : 0), ok, 0, D, vec, foff);
             }
         };
         // exact fp32 scores of the CHUNK candidates of one row, four candidates' loads in flight at a time;
         // strict '>' in ascending unit order keeps the lowest index on ties (same arithmetic as the FFMA variant)
         auto refine_row = [&](int64_t p, int u0) {
             float xr[DMAX];
-            load_row<DMAX>(xr, P.x + patch_base(P.g, p), true, D, vec, aux.foff);
+            load_row(xr, P.x + patch_base(P.g, p), true, 0, D, vec, foff);
             if (u0 < 0 || u0 >= P.K) u0 = 0;           // defensive: the epilogue only writes bases in [0, K_pad)
             float best = -INFINITY;
             int bu = u0;
@@ -329,34 +305,15 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                     mbar_wait_warp<true>(&bars.a_empty[r], a_epar, lane);
                     uint8_t* slot = a_slots + (size_t)r * A_BLK_BYTES + row_off;
                     if (F16) {
-                        // power-of-two row scale: max |s_p x| in [64, 128) as long as a_p = s_p / t_c is an exact FP16
-                        // power of two (2^-24 .. 2^15); an all-zero or non-finite row takes the ideal exponent 0
                         float m = 0.f;
 #pragma unroll
                         for (int d = 0; d < DMAX; ++d) m = fmaxf(m, fabsf(xv[r][d]));
-                        const int eb = (int)((__float_as_uint(m) >> 23) & 0xffu);
-                        int ep = 133 - eb;
-                        if (!(m > 0.f) || eb == 0xff) ep = 0;
-                        int ka = ep - tc_exp, es;
-                        float ap;
-                        if (ka < -24) {
-                            // |x| beyond ~2^24 |c|: ||c||^2 is below fp32 resolution of rd; keep the row in range instead
-                            es = ep;
-                            ap = 0.f;
-                        } else {
-                            ka = ka > 15 ? 15 : ka;                 // 2^-24 .. 2^15: exact in FP16 (subnormal below 2^-14)
-                            es = ka + tc_exp;
-                            ap = __uint_as_float((uint32_t)(127 + ka) << 23);
-                        }
-                        es = es > 120 ? 120 : (es < -120 ? -120 : es);
-                        const float sp = __uint_as_float((uint32_t)(127 + es) << 23);
+                        float sp, ap;
+                        int es;
+                        f16_row_scale(m, tc_exp, sp, ap, es);
                         float hi[DMAX], lo[DMAX];
 #pragma unroll
-                        for (int d = 0; d < DMAX; ++d) {
-                            const float v = xv[r][d] * sp;              // exact
-                            hi[d] = __half2float(__float2half_rn(v));
-                            lo[d] = v - hi[d];                          // exact; rounded to FP16 when packed
-                        }
+                        for (int d = 0; d < DMAX; ++d) f16_split(xv[r][d] * sp, hi[d], lo[d]);     // scaling exact
                         const float h0[8] = {hi[0], hi[1], hi[2], hi[3], hi[4], hi[5], hi[6], hi[7]};
                         const float h1[8] = {hi[8], hi[9], hi[10], hi[11], hi[12], hi[13], hi[14], hi[15]};
                         const float l0[8] = {lo[0], lo[1], lo[2], lo[3], lo[4], lo[5], lo[6], lo[7]};
@@ -375,10 +332,7 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                         for (int d4 = 0; d4 < DMAX / 4; ++d4) {
                             if (d4 < dq) {
                                 float4 hi, lo;
-                                hi.x = tf32_rna(xv[r][4 * d4]);     lo.x = tf32_rna(xv[r][4 * d4] - hi.x);
-                                hi.y = tf32_rna(xv[r][4 * d4 + 1]); lo.y = tf32_rna(xv[r][4 * d4 + 1] - hi.y);
-                                hi.z = tf32_rna(xv[r][4 * d4 + 2]); lo.z = tf32_rna(xv[r][4 * d4 + 2] - hi.z);
-                                hi.w = tf32_rna(xv[r][4 * d4 + 3]); lo.w = tf32_rna(xv[r][4 * d4 + 3] - hi.w);
+                                tf32_split4(&xv[r][4 * d4], hi, lo);
                                 *reinterpret_cast<float4*>(slot + ((((uint32_t)d4) ^ sw) << 4)) = hi;
                                 *reinterpret_cast<float4*>(slot + ((((uint32_t)(dq + d4)) ^ sw) << 4)) = lo;
                             }
@@ -387,9 +341,8 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
 #pragma unroll
                         for (int d = 0; d < DMAX; ++d) {
                             if (d < Dp) {
-                                const float v = xv[r][d];           // zero beyond D (load_row)
-                                const float hi = tf32_rna(v);
-                                const float lo = tf32_rna(v - hi);
+                                float hi, lo;
+                                tf32_split(xv[r][d], hi, lo);       // zero beyond D (load_row)
                                 const uint32_t kh = (uint32_t)d, kl = (uint32_t)(Dp + d);
                                 *reinterpret_cast<float*>(slot + ((((kh >> 2) ^ sw) << 4) | ((kh & 3u) << 2))) = hi;
                                 *reinterpret_cast<float*>(slot + ((((kl >> 2) ^ sw) << 4) | ((kl & 3u) << 2))) = lo;
@@ -430,7 +383,6 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                         tc_fence_after();
                         const uint32_t taddr = tmem_base + ((uint32_t)(lg * 32) << 16) + acc * TN + (uint32_t)half * 128u;
                         const int col0 = n * TN + half * 128;
-                        uint32_t va[32], vb[32];
                         // minimum per CHUNK(8)-column group; only (min, chunk) is tracked
                         auto consume = [&](const uint32_t (&v)[32], int c) {
                             float q[4];
@@ -455,6 +407,7 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                         if (P.dbg & 6) {
                             // timing elimination (experiment builds): 2 = loads without the reduction, 4 = no loads
                             if (P.dbg & 2) {
+                                uint32_t va[32], vb[32];
                                 tmem_ld32_issue(taddr, va); tmem_ld_wait(va);
                                 tmem_ld32_issue(taddr + 32, vb); tmem_ld_wait(vb);
                                 tmem_ld32_issue(taddr + 64, va); tmem_ld_wait(va);
@@ -467,22 +420,7 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                             ++j;
                             continue;
                         }
-                        tmem_ld32_issue(taddr, va);
-                        tmem_ld_wait(va);
-                        tmem_ld32_issue(taddr + 32, vb);
-                        consume(va, 0);
-                        tmem_ld_wait(vb);
-                        tmem_ld32_issue(taddr + 64, va);
-                        consume(vb, 1);
-                        tmem_ld_wait(va);
-                        tmem_ld32_issue(taddr + 96, vb);
-                        consume(va, 2);
-                        tmem_ld_wait(vb);
-                        // accumulator fully read: hand it back before the last reduction
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(&bars.acc_empty[acc]);
-                        consume(vb, 3);
+                        tmem_drain<4>(taddr, consume, [&] { if (lane == 0) mbar_arrive(&bars.acc_empty[acc]); });
                         ++j;
                     }
                 }
@@ -497,11 +435,8 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
 #pragma unroll
                 for (int r = 0; r < R; ++r) {
                     if (r < r_eff) {
-                        const float ov = aux.mrg_val[r][row];
-                        const int oi = aux.mrg_idx[r][row];
-                        int bi = bidx[r];
-                        if (ov < best[r] || (ov == best[r] && oi < bi)) bi = oi;
-                        aux.cbase[it & 1][r][row] = bi;
+                        argmin_merge(best[r], bidx[r], aux.mrg_val[r][row], aux.mrg_idx[r][row]);
+                        aux.cbase[it & 1][r][row] = bidx[r];
                     }
                 }
                 __syncwarp();
@@ -514,7 +449,7 @@ bmu_tc_s_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
     __syncthreads();
     if (warp == 1) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
+        tmem_dealloc(tmem_base, 512);
     }
 }
 
@@ -532,9 +467,9 @@ __global__ void __launch_bounds__(256) split_w_s_kernel(const float* __restrict_
         if (row < K && c < 2 * Dp) {
             const int d = (c < Dp) ? c : c - Dp;
             if (d < D) {
-                const float w = W[(int64_t)row * D + d];
-                const float hi = tf32_rna(w);
-                out = -2.0f * (c < Dp ? hi : tf32_rna(w - hi));
+                float hi, lo;
+                tf32_split(W[(int64_t)row * D + d], hi, lo);
+                out = -2.0f * (c < Dp ? hi : lo);
             }
         }
         Bp[(int64_t)row * 32 + c] = out;
@@ -542,10 +477,8 @@ __global__ void __launch_bounds__(256) split_w_s_kernel(const float* __restrict_
         const int k = c - 32;
         float out = 0.f;
         if (row < K) {
-            const float nrm = cn[row];
-            const float n1 = tf32_rna(nrm);
-            const float n2 = tf32_rna(nrm - n1);
-            const float n3 = tf32_rna(nrm - n1 - n2);
+            float n1, n2, n3;
+            tf32_norm_split3(cn[row], n1, n2, n3);
             out = (k == 0) ? n1 : (k == 1) ? n2 : (k == 2) ? n3 : 0.f;
         } else if (k == 0) {
             out = PAD_NORM;
@@ -619,15 +552,14 @@ __global__ void __launch_bounds__(256) split_w_s16_kernel(const float* __restric
     if (c < 32) {
         const int d = c & 15;
         if (d < D) {
-            const float v = -2.0f * sc * W[(int64_t)src * D + d];          // exact scaling
-            const float hi = __half2float(__float2half_rn(v));
-            out = (c < 16) ? hi : v - hi;
+            float hi, lo;
+            f16_split(-2.0f * sc * W[(int64_t)src * D + d], hi, lo);          // exact scaling
+            out = (c < 16) ? hi : lo;
         }
     } else if (c < 35) {
-        const float nrm = cn[src] * sc * tcs;
-        const float n1 = __half2float(__float2half_rn(nrm));
-        const float n2 = __half2float(__float2half_rn(nrm - n1));
-        out = (c == 32) ? n1 : (c == 33) ? n2 : (nrm - n1 - n2);
+        float n1, n2, n3;
+        f16_norm_split3(cn[src] * sc * tcs, n1, n2, n3);
+        out = (c == 32) ? n1 : (c == 33) ? n2 : n3;
     }
     Bp[(int64_t)row * 64 + c] = __float2half_rn(out);
 }
@@ -677,16 +609,15 @@ int launch_bmu_tc_s(const float* x, const Geom& g, const float* W, const float* 
     const int D = g.D;
     const int Dp = (D + 7) / 8 * 8;
     const int K_pad = (K + TN - 1) / TN * TN;
-    const size_t need = tc_s_workspace_bytes(n, D, K);
-    SOM_REQUIRE(ws != nullptr && ws_bytes >= need, SOM_E_WORKSPACE, "bmu(tc): workspace %zu < required %zu", ws_bytes, need);
-    SOM_REQUIRE(((uintptr_t)ws & 255) == 0, SOM_E_BADARG, "bmu(tc): workspace must be 256-byte aligned");
+    int rc = check_workspace(ws, ws_bytes, tc_s_workspace_bytes(n, D, K), "bmu(tc)");
+    if (rc) return rc;
     float* Bp = (float*)ws;
     float* Tp = (float*)((char*)ws + align_up((size_t)K_pad * 32 * 4, 1024));
     float* scale = (float*)((char*)Tp + align_up((size_t)K_pad * 8 * 4, 1024));
     const bool f16 = tc_s_f16_mode(n, arith);
     if (f16) {
         cb_scale_kernel<<<1, 1024, 0, st>>>(W, cn, K, D, scale);
-        int rc = check_launch("cb_scale_kernel");
+        rc = check_launch("cb_scale_kernel");
         if (rc) return rc;
         const int64_t items = (int64_t)K_pad * 64;
         split_w_s16_kernel<<<(unsigned)ceil_div64(items, 256), 256, 0, st>>>(W, cn, K, D, K_pad, scale, (__half*)Bp);
@@ -695,11 +626,11 @@ int launch_bmu_tc_s(const float* x, const Geom& g, const float* W, const float* 
     } else {
         const int64_t items = (int64_t)K_pad * 40;
         split_w_s_kernel<<<(unsigned)ceil_div64(items, 256), 256, 0, st>>>(W, cn, K, D, Dp, K_pad, Bp, Tp);
-        int rc = check_launch("split_w_s_kernel");
+        rc = check_launch("split_w_s_kernel");
         if (rc) return rc;
     }
     CUtensorMap map_b, map_t;
-    int rc = make_map2d(&map_b, Bp, (uint64_t)K_pad, 32, 128, 32, TN, CU_TENSOR_MAP_SWIZZLE_128B);
+    rc = make_map2d(&map_b, Bp, (uint64_t)K_pad, 32, 128, 32, TN, CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc) return rc;
     rc = make_map2d(&map_t, Tp, (uint64_t)K_pad, 8, 32, 8, TN, CU_TENSOR_MAP_SWIZZLE_32B);
     if (rc) return rc;
@@ -714,18 +645,14 @@ int launch_bmu_tc_s(const float* x, const Geom& g, const float* W, const float* 
     { static int dbg = -1; if (dbg < 0) { const char* e = getenv("SOM_TC_DEBUG"); dbg = e ? atoi(e) : 0; } P.dbg = dbg; }
 #endif
     static PerDeviceFlag attr_done;
-    if (attr_done.pending()) {
-        cudaError_t e = cudaFuncSetAttribute(bmu_tc_s_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(bmu_tc_s_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
-        if (e != cudaSuccess) { set_error("bmu(tc): smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-        attr_done.set();
-    }
+    typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const Params);
+    static const KernelFn kernels[2] = {bmu_tc_s_kernel<false>, bmu_tc_s_kernel<true>};
+    rc = smem_opt_in(attr_done, kernels, 2, (int)SMEM_BYTES, "bmu(tc)");
+    if (rc) return rc;
     P.Rr = tc_s_resident_tiles(n);
     const int n_super = (P.n_mtiles + P.Rr - 1) / P.Rr;
     const int grid = n_super < sm_count() ? n_super : sm_count();
-    if (f16) bmu_tc_s_kernel<true><<<grid, NUM_THREADS, SMEM_BYTES, st>>>(map_b, map_t, P);
-    else bmu_tc_s_kernel<false><<<grid, NUM_THREADS, SMEM_BYTES, st>>>(map_b, map_t, P);
+    kernels[f16]<<<grid, NUM_THREADS, SMEM_BYTES, st>>>(map_b, map_t, P);
     return check_launch("bmu_tc_s_kernel");
 }
 

@@ -91,6 +91,13 @@ __host__ __device__ __forceinline__ int feat_off(const Geom& g, int d) {
     return (c * g.H + i) * g.W + j;
 }
 
+// the argmin tie rule of every BMU merge: the smaller value wins, on equal values the lower index (torch.argmin's
+// first minimum)
+template <typename I>
+__device__ __forceinline__ void argmin_merge(float& best, I& bidx, float v, I i) {
+    if (v < best || (v == best && i < bidx)) { best = v; bidx = i; }
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -129,20 +136,58 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 __device__ __forceinline__ void pdl_begin() { pdl_launch_dependents(); pdl_wait(); }
 
 bool pdl_enabled();                                   // som_core.cu; som_debug_set_pdl(0) turns the attribute off (A/B timing)
+// cudaLaunchKernelEx with the programmatic-stream-serialization attribute (pdl, while pdl_enabled()) and, for
+// cluster > 0, a cluster of `cluster` CTAs along x
 template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                     Args&&... args) {
+static inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                        unsigned cluster, bool pdl, Args&&... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchAttribute attr[2];
+    unsigned n = 0;
+    if (cluster > 0) {
+        attr[n].id = cudaLaunchAttributeClusterDimension;
+        attr[n].val.clusterDim.x = cluster;
+        attr[n].val.clusterDim.y = 1;
+        attr[n].val.clusterDim.z = 1;
+        ++n;
+    }
+    if (pdl && pdl_enabled()) {
+        attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[n].val.programmaticStreamSerializationAllowed = 1;
+        ++n;
+    }
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = n;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+template <typename... KArgs, typename... Args>
+static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                     Args&&... args) {
+    return launch_kernel(kernel, grid, block, smem, st, 0u, true, static_cast<Args&&>(args)...);
+}
+
+// raise the dynamic shared-memory limit of every kernel of a launcher's table to `bytes`, once per device
+template <typename Fn>
+static inline int smem_opt_in(PerDeviceFlag& done, const Fn* kernels, int n, int bytes, const char* who) {
+    if (!done.pending()) return SOM_OK;
+    for (int i = 0; i < n; ++i) {
+        const cudaError_t e = cudaFuncSetAttribute(kernels[i], cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        if (e != cudaSuccess) { set_error("%s: smem opt-in: %s", who, cudaGetErrorString(e)); return (int)e; }
+    }
+    done.set();
+    return SOM_OK;
+}
+
+// a caller's workspace: at least `need` bytes, 256-byte aligned
+static inline int check_workspace(const void* ws, size_t ws_bytes, size_t need, const char* who) {
+    SOM_REQUIRE(ws != nullptr && ws_bytes >= need, SOM_E_WORKSPACE, "%s: workspace %zu < required %zu", who, ws_bytes,
+                need);
+    SOM_REQUIRE(((uintptr_t)ws & 255) == 0, SOM_E_BADARG, "%s: workspace must be 256-byte aligned", who);
+    return SOM_OK;
 }
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

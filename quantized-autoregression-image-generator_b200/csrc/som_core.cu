@@ -172,9 +172,9 @@ __global__ void __launch_bounds__(256) merge_kernel(const float* __restrict__ rd
     float best = rd[p];
     int64_t bi = idx[p];
     for (int r = 1; r < R; ++r) {
-        float v = rd[(int64_t)r * n + p];
-        int64_t i = idx[(int64_t)r * n + p];
-        if (v < best || (v == best && i < bi)) { best = v; bi = i; }
+        const float v = rd[(int64_t)r * n + p];
+        const int64_t i = idx[(int64_t)r * n + p];
+        argmin_merge(best, bi, v, i);
     }
     out_idx[p] = bi;
     if (out_rd) out_rd[p] = best;

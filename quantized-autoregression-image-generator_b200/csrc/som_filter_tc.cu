@@ -25,6 +25,7 @@
 #include "som_common.cuh"
 #include "som_peer.cuh"
 #include "som_tc_ptx.cuh"
+#include "som_tc_split.cuh"
 
 namespace som {
 SOM_TRACE_TU(trace_set_filter_tc)
@@ -70,23 +71,6 @@ __device__ __forceinline__ void sts_v4(uint32_t addr, const float4& v) {
     asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
 
-__device__ __forceinline__ void tc_commit_addr(uint32_t bar_addr) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_addr) : "memory");
-}
-
-template <int TNF>
-__device__ __forceinline__ void mma_tf32_n(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accum) {
-    constexpr uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(TNF >> 3) << 17) |
-                               ((uint32_t)(TMU >> 4) << 24);
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
-        : "memory");
-}
-
 // Bt_hi / Bt_lo [D][Kp]: column h + j holds in[j][d] (hi / lo part), zero elsewhere.  32 x 32 tiles through shared
 // memory: reads coalesced along d, writes coalesced along j.
 // MC: `in` is the NVSwitch multicast address of the ranks' accumulator rows (som_peer.cu) and the load is the in-switch
@@ -127,10 +111,10 @@ __global__ void __launch_bounds__(256) split_in_t_kernel(const float* __restrict
     for (int i = 0; i < 4; ++i) {
         const int d = d0 + ty + 8 * i, jp = jp0 + tx;
         if (d < D && jp < Kp) {
-            const float v = tile[tx][ty + 8 * i];
-            const float hi = tf32_rna(v);
+            float hi, lo;
+            tf32_split(tile[tx][ty + 8 * i], hi, lo);
             Bhi[(int64_t)d * Kp + jp] = hi;
-            Blo[(int64_t)d * Kp + jp] = tf32_rna(v - hi);
+            Blo[(int64_t)d * Kp + jp] = lo;
         }
     }
 }
@@ -151,9 +135,7 @@ filter_tc_kernel(const __grid_constant__ CUtensorMap map_bhi, const __grid_const
     constexpr int B_BYTES = TNF * KBLK * 4;
     constexpr int B_STAGE = 2 * B_BYTES;
     extern __shared__ uint8_t smem_raw[];
-    // 1024-byte alignment as an OFFSET into the shared array: rounding the pointer through uintptr_t made the compiler
-    // forget the address space, and every access below compiled to generic LD.E / ST.E (cuobjdump, round 2)
-    uint8_t* strips = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+    uint8_t* strips = aligned_tiles(smem_raw);
     uint8_t* b_ring = strips + 4 * STRIP_BYTES;          // [strip 0: hi | lo][strip 1: hi | lo][B stages]
     Barriers& bars = *reinterpret_cast<Barriers*>(b_ring + NSB * B_STAGE);
     float* tab_hi = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(&bars) + sizeof(Barriers));
@@ -187,15 +169,9 @@ filter_tc_kernel(const __grid_constant__ CUtensorMap map_bhi, const __grid_const
             const float sq = (float)((long long)at * (long long)at);
             w = expf(-(__fdiv_rn(sq, P.two_var)));
         }
-        const float hi = tf32_rna(w);
-        tab_hi[i] = hi;
-        tab_lo[i] = tf32_rna(w - hi);
+        tf32_split(w, tab_hi[i], tab_lo[i]);
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars.tmem_base)),
-                     "r"(NACC * ACC_COLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    if (warp == 1) tmem_alloc(&bars.tmem_base, NACC * ACC_COLS);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -253,17 +229,17 @@ filter_tc_kernel(const __grid_constant__ CUtensorMap map_bhi, const __grid_const
                     for (int ks = 0; ks < KBLK / 8; ++ks) {
                         const uint32_t acc0 = (!first || ks != 0) ? 1u : 0u;
                         if (CAT) {
-                            mma_tf32_n<ACC_COLS>(d_addr, ahi + 2u * ks, bhi + 2u * ks, acc0);
-                            mma_tf32_n<ACC_COLS>(d_addr, alo + 2u * ks, bhi + 2u * ks, 1u);
+                            tc_mma<MmaKind::TF32, 1, ACC_COLS>(d_addr, ahi + 2u * ks, bhi + 2u * ks, acc0);
+                            tc_mma<MmaKind::TF32, 1, ACC_COLS>(d_addr, alo + 2u * ks, bhi + 2u * ks, 1u);
                         } else {
-                            mma_tf32_n<TNF>(d_addr, ahi + 2u * ks, bhi + 2u * ks, acc0);
-                            mma_tf32_n<TNF>(d_addr, alo + 2u * ks, bhi + 2u * ks, 1u);
-                            mma_tf32_n<TNF>(d_addr, ahi + 2u * ks, blo + 2u * ks, 1u);
+                            tc_mma<MmaKind::TF32, 1, TNF>(d_addr, ahi + 2u * ks, bhi + 2u * ks, acc0);
+                            tc_mma<MmaKind::TF32, 1, TNF>(d_addr, alo + 2u * ks, bhi + 2u * ks, 1u);
+                            tc_mma<MmaKind::TF32, 1, TNF>(d_addr, ahi + 2u * ks, blo + 2u * ks, 1u);
                         }
                     }
-                    tc_commit_addr(bempty0 + 8u * (uint32_t)stage);
-                    if (kb + 1 == c1) tc_commit_addr(sempty0 + 8u * (uint32_t)sbuf);
-                    if (kb + 1 == kb_hi) tc_commit_addr(accfull);
+                    tc_commit(bempty0 + 8u * (uint32_t)stage);
+                    if (kb + 1 == c1) tc_commit(sempty0 + 8u * (uint32_t)sbuf);
+                    if (kb + 1 == kb_hi) tc_commit(accfull);
                 }
                 first = false;
                 if (KS == 1 && ++in_chain == P.q) { in_chain = 0; d_addr += ACC_COLS; first = true; }
@@ -370,7 +346,7 @@ done:
     __syncthreads();
     if (warp == 1) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(NACC * ACC_COLS));
+        tmem_dealloc(tmem_base, NACC * ACC_COLS);
     }
 }
 
@@ -446,20 +422,19 @@ int launch_filter_tc_in(const float* in, float* out, int K, int D, float two_var
     using namespace ftc;
     Plan pl;
     make_plan(&pl, K, D, h);
-    SOM_REQUIRE(ws != nullptr && ws_bytes >= pl.total, SOM_E_WORKSPACE, "filter(tc): workspace %zu < required %zu",
-                ws_bytes, pl.total);
-    SOM_REQUIRE(((uintptr_t)ws & 255) == 0, SOM_E_BADARG, "filter(tc): workspace must be 256-byte aligned");
+    int rc = check_workspace(ws, ws_bytes, pl.total, "filter(tc)");
+    if (rc) return rc;
     float* Bhi = (float*)((char*)ws + pl.off_hi);
     float* Blo = (float*)((char*)ws + pl.off_lo);
     {
         dim3 grid((unsigned)(pl.Kp / 32), (unsigned)ceil_div64(D, 32));
         if (pin != nullptr) launch_pdl(split_in_t_kernel<true>, grid, 256, 0, st, in, K, D, h, pl.Kp, Bhi, Blo, *pin);
         else launch_pdl(split_in_t_kernel<false>, grid, 256, 0, st, in, K, D, h, pl.Kp, Bhi, Blo, PeerIn{});
-        int rc = check_launch("split_in_t_kernel");
+        rc = check_launch("split_in_t_kernel");
         if (rc) return rc;
     }
     CUtensorMap map_bhi, map_blo;
-    int rc = make_map2d(&map_bhi, Bhi, (uint64_t)D, (uint64_t)pl.Kp, (uint64_t)pl.Kp * 4, KBLK, (uint32_t)pl.tnf,
+    rc = make_map2d(&map_bhi, Bhi, (uint64_t)D, (uint64_t)pl.Kp, (uint64_t)pl.Kp * 4, KBLK, (uint32_t)pl.tnf,
                         CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc) return rc;
     rc = make_map2d(&map_blo, Blo, (uint64_t)D, (uint64_t)pl.Kp, (uint64_t)pl.Kp * 4, KBLK, (uint32_t)pl.tnf,
@@ -470,17 +445,13 @@ int launch_filter_tc_in(const float* in, float* out, int K, int D, float two_var
     P.q = pl.q; P.na = pl.na;
     P.ks = pl.ks; P.partial = (float*)((char*)ws + pl.off_part);
     const size_t smem = smem_bytes(pl.tnf, h);
+    typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const Params);
+    static const KernelFn kernels[2] = {filter_tc_kernel<64>, filter_tc_kernel<128>};
     static PerDeviceFlag attr_done;
-    if (attr_done.pending()) {
-        cudaError_t e = cudaFuncSetAttribute(filter_tc_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(filter_tc_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e != cudaSuccess) { set_error("filter(tc): smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-        attr_done.set();
-    }
+    rc = smem_opt_in(attr_done, kernels, 2, 227 * 1024, "filter(tc)");
+    if (rc) return rc;
     dim3 grid((unsigned)ceil_div64(K, TMU), (unsigned)ceil_div64(D, pl.tnf), (unsigned)pl.ks);
-    if (pl.tnf == 128) launch_pdl(filter_tc_kernel<128>, grid, NUM_THREADS, smem, st, map_bhi, map_blo, P);
-    else launch_pdl(filter_tc_kernel<64>, grid, NUM_THREADS, smem, st, map_bhi, map_blo, P);
+    launch_pdl(kernels[pl.tnf == 128], grid, NUM_THREADS, smem, st, map_bhi, map_blo, P);
     rc = check_launch("filter_tc_kernel");
     if (rc || pl.ks == 1) return rc;
     const int64_t n = (int64_t)K * D;

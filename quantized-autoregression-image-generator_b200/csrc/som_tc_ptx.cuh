@@ -1,6 +1,9 @@
-// PTX helpers shared by the tcgen05 BMU kernels (sm_100a): mbarrier, TMA, tcgen05 MMA / TMEM loads.
+// PTX helpers shared by the tcgen05 kernels (sm_100a): mbarrier, TMA, tcgen05 MMA / commit / TMEM, the builders' row
+// loader and the epilogue drain.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 
 #include "som_common.cuh"
@@ -13,8 +16,6 @@ constexpr int TN = 256;              // units per MMA tile (UMMA N)
 constexpr int KBLK = 32;             // floats per k-block: one 128-byte swizzle row
 constexpr int A_BLK_BYTES = TM * KBLK * 4;     // 16 KB
 constexpr int B_BLK_BYTES = TN * KBLK * 4;     // 32 KB
-constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(TN >> 3) << 17) |
-                           ((uint32_t)(TM >> 4) << 24);
 constexpr float PAD_NORM = 1.0e30f;            // ||c||^2 of padding units: never the minimum
 
 // ---- PTX helpers ---------------------------------------------------------------------------------
@@ -150,46 +151,6 @@ __device__ __forceinline__ void tma_load_2d_pair(const CUtensorMap* map, uint64_
         ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1)
         : "memory");
 }
-// M = 128 * CG rows (one 128-row half per CTA), N = 256, K = 8, kind::tf32, K-major operands, fp32 accumulate
-template <int CG>
-__device__ __forceinline__ void tc_mma_tf32_cg(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accum) {
-    constexpr uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(TN >> 3) << 17) |
-                               ((uint32_t)((TM * CG) >> 4) << 24);
-    if (CG == 1) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
-            : "memory");
-    } else {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
-            : "memory");
-    }
-}
-// commit: arrive (once the issued MMAs completed) on the barrier at this offset in every CTA of the pair
-template <int CG>
-__device__ __forceinline__ void tc_commit_cg(uint64_t* bar) {
-    if (CG == 1) {
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-                     : "memory");
-    } else {
-        asm volatile(
-            "{\n"
-            ".reg .b16 m;\n"
-            "mov.b16 m, 3;\n"
-            "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], m;\n"
-            "}\n" ::"r"(smem_u32(bar))
-            : "memory");
-    }
-}
-
 // one lane of a converged warp (elect.sync): the MMA warp keeps warp-uniform control flow, so descriptors
 // live in uniform registers, and only the tcgen05 instructions themselves are predicated on the elected lane
 __device__ __forceinline__ bool elect_one() {
@@ -207,58 +168,92 @@ __device__ __forceinline__ bool elect_one() {
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-                 : "memory");
+
+// ---- tcgen05.mma / tcgen05.commit --------------------------------------------------------------------
+// kind::tf32: TF32 operands, M x N x K8.  kind::f16 with FP16 operands: M x N x K16 at the cycle cost of the K8 TF32 MMA.
+enum class MmaKind { TF32, F16 };
+// instruction descriptor: fp32 accumulate, a/b format (TF32 2, FP16 0), K-major operands, N >> 3, M >> 4
+constexpr uint32_t make_idesc(MmaKind kind, int M, int N) {
+    return (1u << 4) | ((kind == MmaKind::TF32 ? 2u : 0u) << 7) | ((kind == MmaKind::TF32 ? 2u : 0u) << 10) |
+           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
-__device__ __forceinline__ void tc_mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accum) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(IDESC), "r"(accum)
-        : "memory");
+#define SOM_TC_MMA_ASM(cg, kind)                                                                 \
+    asm volatile(                                                                                \
+        "{\n"                                                                                    \
+        ".reg .pred p;\n"                                                                        \
+        "setp.ne.b32 p, %4, 0;\n"                                                                \
+        "tcgen05.mma.cta_group::" #cg ".kind::" #kind " [%0], %1, %2, %3, p;\n"                  \
+        "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)                      \
+        : "memory")
+// M = 128 * CG rows (one 128-row half per CTA), N columns; accum = 0 overwrites the accumulator
+template <MmaKind KIND, int CG = 1, int N = TN>
+__device__ __forceinline__ void tc_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accum) {
+    constexpr uint32_t idesc = make_idesc(KIND, TM * CG, N);
+    if constexpr (KIND == MmaKind::TF32) {
+        if constexpr (CG == 1) SOM_TC_MMA_ASM(1, tf32); else SOM_TC_MMA_ASM(2, tf32);
+    } else {
+        if constexpr (CG == 1) SOM_TC_MMA_ASM(1, f16); else SOM_TC_MMA_ASM(2, f16);
+    }
 }
-// kind::f16 with FP16 operands (a/b format 0), fp32 accumulate: M128 x N256 x K16 at the cycle cost of the K8 TF32 MMA
-constexpr uint32_t IDESC_F16 = (1u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)(TN >> 3) << 17) |
-                               ((uint32_t)(TM >> 4) << 24);
-__device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accum) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(IDESC_F16), "r"(accum)
-        : "memory");
-}
-// kind::f16 (FP16 operands, fp32 accumulate), M = 128 * CG rows (one 128-row half per CTA), N = 256, K = 16
-template <int CG>
-__device__ __forceinline__ void tc_mma_f16_cg(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accum) {
-    constexpr uint32_t idesc = (1u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)(TN >> 3) << 17) |
-                               ((uint32_t)((TM * CG) >> 4) << 24);
-    if (CG == 1) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
-            : "memory");
+#undef SOM_TC_MMA_ASM
+// arrive (once the issued MMAs completed) on the barrier at shared address `bar` in every CTA of the pair (CG = 2:
+// multicast to both)
+template <int CG = 1>
+__device__ __forceinline__ void tc_commit(uint32_t bar) {
+    if constexpr (CG == 1) {
+        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
     } else {
         asm volatile(
             "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
+            ".reg .b16 m;\n"
+            "mov.b16 m, 3;\n"
+            "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], m;\n"
+            "}\n" ::"r"(bar)
             : "memory");
     }
+}
+template <int CG = 1>
+__device__ __forceinline__ void tc_commit(uint64_t* bar) { tc_commit<CG>(smem_u32(bar)); }
+
+// ---- TMEM allocation (warp-wide: one warp allocates, the same warp frees) ----------------------------------
+template <int CG = 1>
+__device__ __forceinline__ void tmem_alloc(uint32_t* dst, uint32_t cols) {
+    if constexpr (CG == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst)), "r"(cols));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    } else {
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst)), "r"(cols));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
+    }
+}
+template <int CG = 1>
+__device__ __forceinline__ void tmem_dealloc(uint32_t base, uint32_t cols) {
+    if constexpr (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols));
+    else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols));
+}
+
+// the 1024-byte aligned start of the dynamic shared memory (SWIZZLE_128B tiles).  The alignment is an OFFSET into the
+// shared array: rounding the pointer through uintptr_t made the compiler forget the address space, and every access
+// compiled to generic LD.E / ST.E (cuobjdump, round 2)
+__device__ __forceinline__ uint8_t* aligned_tiles(uint8_t* smem_raw) {
+    return smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
 }
 // K-major, SWIZZLE_128B operand descriptor (cute::UMMA::SmemDescriptor): start>>4 | LBO=1 | SBO=1024>>4
 // | version=1 | layout_type=2.  Advancing one K=8 step inside the 128-byte row adds 32 B (2 units).
 __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) {
     return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
+}
+// K-major SWIZZLE_32B operand descriptor (the norm tail k-step): 32-byte rows, 8-row groups 256 B apart
+__device__ __forceinline__ uint64_t umma_desc_sw32(uint32_t smem_addr) {
+    return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(256 >> 4) << 32) | (1ull << 46) |
+           (6ull << 61);
+}
+// TF32 norm tail operand A: row t = [1 1 1 0 | 0 0 0 0] in the 32-byte swizzle (chunk ^= bit 2 of t)
+__device__ __forceinline__ void write_tail_ones(uint8_t* a_tail, int t) {
+    const uint32_t sw = (uint32_t)(t >> 2) & 1u;
+    float4* rowp = reinterpret_cast<float4*>(a_tail + t * 32);
+    rowp[sw] = make_float4(1.f, 1.f, 1.f, 0.f);
+    rowp[sw ^ 1u] = make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
 #define SOM_R32(a) "=r"(a[0]), "=r"(a[1]), "=r"(a[2]), "=r"(a[3]), "=r"(a[4]), "=r"(a[5]), "=r"(a[6]), "=r"(a[7]), \
@@ -284,6 +279,29 @@ __device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32
 __device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[32]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;\n" : SOM_RW32(r)::"memory");
 }
+// epilogue drain of one TMEM accumulator: NCH chunks of 32 columns from taddr, the next chunk's load in flight while
+// consume(v, c) reduces chunk c.  Once the last load has landed the accumulator is handed back (fence, warp sync, then
+// release(), which arrives on the accumulator's empty barrier) BEFORE the last chunk is consumed.
+template <int NCH, typename Consume, typename Release>
+__device__ __forceinline__ void tmem_drain(uint32_t taddr, Consume&& consume, Release&& release) {
+    uint32_t va[32], vb[32];
+    tmem_ld32_issue(taddr, va);
+#pragma unroll
+    for (int c = 0; c < NCH; c += 2) {
+        tmem_ld_wait(va);
+        tmem_ld32_issue(taddr + (c + 1) * 32, vb);
+        consume(va, c);
+        tmem_ld_wait(vb);
+        if (c + 2 < NCH) {
+            tmem_ld32_issue(taddr + (c + 2) * 32, va);
+        } else {
+            tc_fence_before();
+            __syncwarp();
+            release();
+        }
+        consume(vb, c + 1);
+    }
+}
 __device__ __forceinline__ float min32(const uint32_t (&r)[32]) {
     float m = __uint_as_float(r[0]);
 #pragma unroll
@@ -303,35 +321,64 @@ __device__ __forceinline__ float tf32_rna(float v) {
 }
 
 
-// builder-side loader: D features of patch row `src` into registers (static indexing, DCAP >= D)
-template <int DCAP>
-__device__ __forceinline__ void load_row(float (&xr)[DCAP], const float* src, bool ok, int D, int vec,
-                                         const int* foff) {
+// exact fp32 values of 4 / 2 / 1 consecutive input elements (float, __half or __nv_bfloat16)
+__device__ __forceinline__ void ld4(const float* p, float* o) {
+    const float4 f = __ldg(reinterpret_cast<const float4*>(p));
+    o[0] = f.x; o[1] = f.y; o[2] = f.z; o[3] = f.w;
+}
+__device__ __forceinline__ void ld4(const __half* p, float* o) {
+    const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
+    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&r.x));
+    const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&r.y));
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
+}
+__device__ __forceinline__ void ld4(const __nv_bfloat16* p, float* o) {
+    const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
+    const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&r.x));
+    const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&r.y));
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
+}
+__device__ __forceinline__ void ld2(const float* p, float* o) {
+    const float2 f = __ldg(reinterpret_cast<const float2*>(p));
+    o[0] = f.x; o[1] = f.y;
+}
+__device__ __forceinline__ void ld2(const __half* p, float* o) {
+    const float2 f = __half22float2(__ldg(reinterpret_cast<const __half2*>(p)));
+    o[0] = f.x; o[1] = f.y;
+}
+__device__ __forceinline__ void ld2(const __nv_bfloat16* p, float* o) {
+    const float2 f = __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162*>(p)));
+    o[0] = f.x; o[1] = f.y;
+}
+__device__ __forceinline__ float ld1(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld1(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ float ld1(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+
+// builder-side loader: features [d0, d0 + N) of the NCHW patch row `src` into registers (static indexing), zero beyond
+// D and where !ok.  vec is the run width of the row in elements (4, 2 or 1: Geom::vec); foff(d) is the element offset
+// of feature d from the row's base.
+template <int N, typename T, typename FeatOff>
+__device__ __forceinline__ void load_row(float (&v)[N], const T* src, bool ok, int d0, int D, int vec, FeatOff&& foff) {
 #pragma unroll
-    for (int d = 0; d < DCAP; d += 4) {
+    for (int c = 0; c < N; c += 4) {
+        const int d = d0 + c;
         float tmp[4] = {0.f, 0.f, 0.f, 0.f};
         if (ok && d < D) {
             if (vec == 4) {
-                float4 v = __ldg(reinterpret_cast<const float4*>(src + foff[d]));
-                tmp[0] = v.x; tmp[1] = v.y; tmp[2] = v.z; tmp[3] = v.w;
+                ld4(src + foff(d), tmp);
             } else if (vec == 2) {
-                float2 v0 = __ldg(reinterpret_cast<const float2*>(src + foff[d]));
-                tmp[0] = v0.x; tmp[1] = v0.y;
-                if (d + 2 < D) {
-                    float2 v1 = __ldg(reinterpret_cast<const float2*>(src + foff[d + 2]));
-                    tmp[2] = v1.x; tmp[3] = v1.y;
-                }
+                ld2(src + foff(d), tmp);
+                if (d + 2 < D) ld2(src + foff(d + 2), tmp + 2);
             } else {
 #pragma unroll
                 for (int e = 0; e < 4; ++e)
-                    if (d + e < D) tmp[e] = __ldg(src + foff[d + e]);
+                    if (d + e < D) tmp[e] = ld1(src + foff(d + e));
             }
         }
 #pragma unroll
-        for (int e = 0; e < 4; ++e) xr[d + e] = tmp[e];
+        for (int e = 0; e < 4; ++e) v[c + e] = tmp[e];
     }
 }
-
 
 // ---- host side: tensor maps ------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
