@@ -20,6 +20,7 @@
 //      order, zero-fills empty units, and writes counts; a single CTA reduces the sse partials.
 // Bound: HBM -- algorithmic bytes 4*D per patch (x read once) + 8 (index) + 4*K*D (Rbar).
 #include "som_common.cuh"
+#include "som_step_rules.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -655,8 +656,7 @@ acc_scan_kernel(const float* __restrict__ x, Geom g, const int64_t* __restrict__
 }
 
 // fixed-order double reduction of the per-(chunk, slice) squared-error partials.  `tail` (data-parallel form, may be
-// NULL) receives [sse_hi, sse_lo, n / 4096, n % 4096] as floats: the fp64 sum as a float pair and the local patch
-// count as two exactly representable floats, so that ONE fp32 all-reduce(sum) of [Rbar | tail] carries them too.
+// NULL) receives the packed tail of the sum and the local patch count (pack_tail; 4-byte aligned, stored as floats).
 __global__ void __launch_bounds__(1024) sse_reduce_kernel(const double* __restrict__ part, int64_t m,
                                                           double* __restrict__ out, float* __restrict__ tail,
                                                           int64_t n_patches) {
@@ -674,11 +674,8 @@ __global__ void __launch_bounds__(1024) sse_reduce_kernel(const double* __restri
     if (threadIdx.x == 0) {
         if (out != nullptr) *out = sh[0];
         if (tail != nullptr) {
-            const float hi = (float)sh[0];
-            tail[0] = hi;
-            tail[1] = (float)(sh[0] - (double)hi);
-            tail[2] = (float)(n_patches >> 12);
-            tail[3] = (float)(n_patches & 4095);
+            const float4 t = pack_tail(sh[0], n_patches);
+            tail[0] = t.x; tail[1] = t.y; tail[2] = t.z; tail[3] = t.w;
         }
     }
 }
@@ -695,16 +692,13 @@ static int launch_levels(const float* x, const Geom& g, const AccumPlan& pl, con
         constexpr size_t ring_bytes = (size_t)ACC_WARPS * 2 * 2 * L1_GROUP<VEC>::value * 32 * VEC * sizeof(float) +
                                       (size_t)ACC_WARPS * 2 * L1_GROUP<VEC>::value * sizeof(int4);
         static PerDeviceFlag attr_done;
-        if (attr_done.pending()) {
-            cudaError_t e = cudaFuncSetAttribute(seg_level1_kernel<VEC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 (int)ring_bytes);
-            if (e != cudaSuccess) { set_error("accumulate: smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-            attr_done.set();
-        }
+        const auto kernel = seg_level1_kernel<VEC>;
+        int rc = smem_opt_in(attr_done, &kernel, 1, (int)ring_bytes, "accumulate");
+        if (rc) return rc;
         launch_pdl(seg_level1_kernel<VEC>, blocks, ACC_WARPS * 32, ring_bytes, st, 
             x, g, skey, sid, offsets, Wt, Rbar, partial, ((sse || tail) && Wt) ? sse_part : nullptr,
             pl.S, pl.n_chunks, n_slices);
-        int rc = check_launch("seg_level1_kernel");
+        rc = check_launch("seg_level1_kernel");
         if (rc) return rc;
     }
     {
@@ -790,13 +784,9 @@ static int accumulate_impl(const float* x, int64_t n_img, int C, int H, int Wd, 
         int* total = hist + (size_t)pl.cs_blocks * K;
         const size_t bins = (size_t)K * sizeof(int);
         static PerDeviceFlag attr_done;
-        if (attr_done.pending()) {
-            cudaError_t e = cudaFuncSetAttribute(csort_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, CS_KMAX * 4);
-            if (e == cudaSuccess)
-                e = cudaFuncSetAttribute(csort_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, CS_KMAX * 4);
-            if (e != cudaSuccess) { set_error("accumulate: smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-            attr_done.set();
-        }
+        static const void* const kernels[2] = {(const void*)csort_hist_kernel, (const void*)csort_scatter_kernel};
+        rc = smem_opt_in(attr_done, kernels, 2, CS_KMAX * 4, "accumulate");
+        if (rc) return rc;
         launch_pdl(csort_hist_kernel, pl.cs_blocks, CS_THREADS, bins, st, bmu, n, K, pl.cs_per, hist);
         rc = check_launch("csort_hist_kernel");
         if (rc) return rc;

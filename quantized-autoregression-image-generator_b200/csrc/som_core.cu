@@ -1,6 +1,7 @@
 // libsomcb core: error plumbing, geometry, and the small HBM-bound kernels of the SOM path
 // (codebook norms, candidate merge, hit histogram, quantise/gather, Adam, row compaction).
 #include "som_common.cuh"
+#include "som_step_rules.cuh"
 
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -443,23 +444,14 @@ __global__ void __launch_bounds__(256, 4) quantize_out_kernel(const int64_t* __r
 }
 
 // ---------------------------------------------------------------------------------------------
-// K4: Adam, torch.optim.Adam single-tensor rule (lerp form of the first moment)
+// K4: Adam (som_step_rules.cuh)
 // ---------------------------------------------------------------------------------------------
-struct AdamScalars { float w1, b2, one_m_b2, step_size, bc2_sqrt, eps; };
-
-__device__ __forceinline__ void adam_update(const AdamScalars& a, float gi, float& mi, float& vi, float& wi) {
-    float diff = gi - mi;
-    // torch lerp: weight < 0.5 ? start + w*diff : end - diff*(1-w)
-    mi = (a.w1 < 0.5f) ? __fmaf_rn(a.w1, diff, mi) : __fmaf_rn(-diff, 1.0f - a.w1, gi);
-    vi = __fmaf_rn(a.one_m_b2 * gi, gi, vi * a.b2);
-    float denom = __fdiv_rn(__fsqrt_rn(vi), a.bc2_sqrt) + a.eps;
-    wi = __fmaf_rn(-a.step_size, __fdiv_rn(mi, denom), wi);
-}
-
 // Four streams in, three out, 28 bytes per weight: 16-byte accesses, four weights per thread per iteration
 // (the scalar one-weight loop reached 73 % of the HBM copy rate; the element-wise arithmetic is unchanged).
+// SCALED: the gradient arrives unscaled (adam_update4).
+template <bool SCALED>
 __device__ __forceinline__ void adam_body(float* __restrict__ W, float* __restrict__ m, float* __restrict__ v,
-                                          const float* __restrict__ g, int64_t n, const AdamScalars& a) {
+                                          const float* __restrict__ g, int64_t n, const AdamScalars& a, float gscale) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     const bool al = ((reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(m) |
@@ -471,15 +463,12 @@ __device__ __forceinline__ void adam_body(float* __restrict__ W, float* __restri
     const float4* g4 = reinterpret_cast<const float4*>(g);
     for (int64_t q = tid; q < n4; q += stride) {
         float4 gq = __ldcs(g4 + q), mq = m4[q], vq = v4[q], wq = W4[q];
-        adam_update(a, gq.x, mq.x, vq.x, wq.x);
-        adam_update(a, gq.y, mq.y, vq.y, wq.y);
-        adam_update(a, gq.z, mq.z, vq.z, wq.z);
-        adam_update(a, gq.w, mq.w, vq.w, wq.w);
+        adam_update4<SCALED>(a, gq, gscale, mq, vq, wq);
         W4[q] = wq; m4[q] = mq; v4[q] = vq;
     }
     for (int64_t i = n4 * 4 + tid; i < n; i += stride) {
         float mi = m[i], vi = v[i], wi = W[i];
-        adam_update(a, g[i], mi, vi, wi);
+        adam_update(a, SCALED ? g[i] * gscale : g[i], mi, vi, wi);
         W[i] = wi; m[i] = mi; v[i] = vi;
     }
 }
@@ -489,31 +478,25 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ W, float*
                                                    int64_t n, AdamScalars a) {
     pdl_begin();
     trace_stamp(s_trace_buf, 19);
-    adam_body(W, m, v, g, n, a);
+    adam_body<false>(W, m, v, g, n, a, 0.f);
 }
 
 // Same rule with the step count read from device memory, so a captured CUDA graph of the training step can be
-// replayed: t = *steps_done + 1; bias corrections in double as on the host path.  step_bump_kernel advances it.
+// replayed: t = *steps_done + 1.  step_bump_kernel advances it.
 __global__ void __launch_bounds__(256) adam_dev_kernel(float* __restrict__ W, float* __restrict__ m,
                                                        float* __restrict__ v, const float* __restrict__ g,
                                                        int64_t n, double lr, double b1, double b2, float eps,
                                                        const int64_t* __restrict__ steps_done) {
     pdl_begin();
     trace_stamp(s_trace_buf, 19);
-    const double t = (double)(*steps_done + 1);
-    AdamScalars a;
-    a.w1 = (float)(1.0 - b1); a.b2 = (float)b2; a.one_m_b2 = (float)(1.0 - b2);
-    a.step_size = (float)(lr / (1.0 - pow(b1, t)));
-    a.bc2_sqrt = (float)sqrt(1.0 - pow(b2, t));
-    a.eps = eps;
-    adam_body(W, m, v, g, n, a);
+    const AdamScalars a = adam_scalars(lr, b1, b2, eps, (double)(*steps_done + 1));
+    adam_body<false>(W, m, v, g, n, a, 0.f);
 }
 __global__ void step_bump_kernel(int64_t* steps_done) { *steps_done += 1; }
 
 // Data-parallel tail: the gradient arrives UNSCALED (g = T @ Rbar_global) and the global batch size is only known on
-// the device, from the all-reduced tail [sse_hi, sse_lo, n / 4096, n % 4096] (som_accumulate_packed_nchw_f32):
-// g_eff = g * (float)(2 / numel), numel = D * n_global -- the same single rounding as the filter's own `scale * acc`
-// epilogue, so the result is bit-identical to the host-scaled path; thread 0 also writes the mean squared error.
+// the device, from the all-reduced packed tail (som_accumulate_packed_nchw_f32); thread 0 also writes the mean squared
+// error.
 __global__ void __launch_bounds__(256) adam_dp_kernel(float* __restrict__ W, float* __restrict__ m,
                                                       float* __restrict__ v, const float* __restrict__ g,
                                                       int64_t n, int D, double lr, double b1, double b2, float eps,
@@ -522,37 +505,10 @@ __global__ void __launch_bounds__(256) adam_dp_kernel(float* __restrict__ W, flo
     pdl_begin();
     trace_stamp(s_trace_buf, 18);
     const double t = (double)(steps_done[0] + 1);
-    const double numel = ((double)tail[2] * 4096.0 + (double)tail[3]) * (double)D;
-    const float gscale = (float)(2.0 / numel);
-    AdamScalars a;
-    a.w1 = (float)(1.0 - b1); a.b2 = (float)b2; a.one_m_b2 = (float)(1.0 - b2);
-    a.step_size = (float)(lr / (1.0 - pow(b1, t)));
-    a.bc2_sqrt = (float)sqrt(1.0 - pow(b2, t));
-    a.eps = eps;
-    if (loss_out != nullptr && blockIdx.x == 0 && threadIdx.x == 0)
-        *loss_out = ((double)tail[0] + (double)tail[1]) / numel;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    const bool al = ((reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(m) |
-                      reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(g)) & 15) == 0;
-    const int64_t n4 = al ? n / 4 : 0;
-    float4* W4 = reinterpret_cast<float4*>(W);
-    float4* m4 = reinterpret_cast<float4*>(m);
-    float4* v4 = reinterpret_cast<float4*>(v);
-    const float4* g4 = reinterpret_cast<const float4*>(g);
-    for (int64_t q = tid; q < n4; q += stride) {
-        float4 gq = __ldcs(g4 + q), mq = m4[q], vq = v4[q], wq = W4[q];
-        adam_update(a, gq.x * gscale, mq.x, vq.x, wq.x);
-        adam_update(a, gq.y * gscale, mq.y, vq.y, wq.y);
-        adam_update(a, gq.z * gscale, mq.z, vq.z, wq.z);
-        adam_update(a, gq.w * gscale, mq.w, vq.w, wq.w);
-        W4[q] = wq; m4[q] = mq; v4[q] = vq;
-    }
-    for (int64_t i = n4 * 4 + tid; i < n; i += stride) {
-        float mi = m[i], vi = v[i], wi = W[i];
-        adam_update(a, g[i] * gscale, mi, vi, wi);
-        W[i] = wi; m[i] = mi; v[i] = vi;
-    }
+    const TailTotals tt = tail_totals(tail, D);
+    const AdamScalars a = adam_scalars(lr, b1, b2, eps, t);
+    if (loss_out != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *loss_out = tail_loss(tail, tt.numel);
+    adam_body<true>(W, m, v, g, n, a, tt.gscale);
     // the last block to finish advances the step count (every block read it when it started): steps_done[1] is the
     // arrival counter, left at zero again
     __syncthreads();
@@ -748,13 +704,10 @@ int som_histogram_i64(const int64_t* idx, int64_t n, int K, int64_t* counts, voi
     // also for few indices per unit (C5 shard, 2^20 indices against 32768 units: 12.7-14.3 us, the same as direct
     // global atomics on uniform hits) -- skewed hits would serialise on one L2 address there
     if (P <= sms) {
-        static std::once_flag once[64];
-        int dev = 0;
-        cudaGetDevice(&dev);
-        std::call_once(once[dev & 63], [] {
-            cudaFuncSetAttribute(hist_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 HIST_RANGE_MAX * (int)sizeof(unsigned int));
-        });
+        static PerDeviceFlag attr_done;
+        const auto kernel = hist_range_kernel;
+        int rc = smem_opt_in(attr_done, &kernel, 1, HIST_RANGE_MAX * (int)sizeof(unsigned int), "histogram");
+        if (rc) return rc;
         const int Kr = (int)(ceil_div64(ceil_div64(K, P), 32) * 32);
         int S = sms / P;                                     // index slices; every CTA is resident (one per SM)
         const int64_t per_cta = (int64_t)1024 * 8;
@@ -765,7 +718,7 @@ int som_histogram_i64(const int64_t* idx, int64_t n, int K, int64_t* counts, voi
             const int64_t m = (n - at < chunk) ? n - at : chunk;
             hist_range_kernel<<<P * S, 1024, (size_t)Kr * sizeof(unsigned int), (cudaStream_t)stream>>>(
                 idx + at, m, K, Kr, P, c);
-            int rc = check_launch("hist_range_kernel");
+            rc = check_launch("hist_range_kernel");
             if (rc) return rc;
         }
         return SOM_OK;
@@ -833,13 +786,8 @@ int som_adam_f32(float* W, float* m, float* v, const float* g, int64_t n,
     SOM_REQUIRE(W && m && v && g, SOM_E_BADARG, "adam: null pointer");
     SOM_REQUIRE(n >= 0 && step >= 1, SOM_E_BADARG, "adam: n=%lld step=%lld", (long long)n, (long long)step);
     if (n == 0) return SOM_OK;
-    // scalars in double on the host exactly as torch/optim/adam.py does, then narrowed
-    double bc1 = 1.0 - pow(b1, (double)step);
-    double bc2 = 1.0 - pow(b2, (double)step);
-    double step_size = lr / bc1;
-    double bc2_sqrt = sqrt(bc2);
     int blocks = grid_for(n, 256 * 4, 8);
-    AdamScalars a{(float)(1.0 - b1), (float)b2, (float)(1.0 - b2), (float)step_size, (float)bc2_sqrt, (float)eps};
+    const AdamScalars a = adam_scalars(lr, b1, b2, (float)eps, (double)step);      // on the host
     launch_pdl(adam_kernel, blocks, 256, 0, (cudaStream_t)stream, W, m, v, g, n, a);
     return check_launch("adam_kernel");
 }

@@ -5,14 +5,15 @@
 // This is T @ in with T the K x K banded symmetric Toeplitz matrix that the reference builds
 // densely, one row per patch, in models/Codebook.py:112-125 and multiplies in :128-130
 // (forward, in = W) and in the matmul backward (in = Rbar).  Weights are generated exactly as
-// the reference does: (j-b)^2 exact in integers, converted to fp32, divided by fp32(two_var),
-// negated, expf.  The band half-width h is where expf underflows to exactly 0 (SURVEY 0.7).
+// the reference does (band_weight, som_step_rules.cuh).  The band half-width h is where expf
+// underflows to exactly 0 (SURVEY 0.7).
 //
 // Mapping: lane <-> feature d (coalesced 128-byte rows), each warp owns TA consecutive units
 // and slides a TA-wide window of weights held in registers over the rows j it needs, so each
 // loaded value feeds TA FFMAs and each step needs one weight from the shared table.
 // Bound: FFMA (2*K*D*band flop) -- in[] is K*D*4 bytes and stays L1/L2 resident.
 #include "som_common.cuh"
+#include "som_step_rules.cuh"
 
 namespace som {
 SOM_TRACE_TU(trace_set_filter)
@@ -31,14 +32,8 @@ filter_kernel(const float* __restrict__ in, float* __restrict__ out, int K, int 
     const int off = h + FILT_PAD;
     const int tab_n = 2 * off + 1;
     for (int i = threadIdx.x; i < tab_n; i += blockDim.x) {
-        int t = i - off;
-        int at = t < 0 ? -t : t;
-        float w = 0.f;
-        if (at <= h) {
-            float sq = (float)((long long)at * (long long)at);
-            w = expf(-(__fdiv_rn(sq, two_var)));
-        }
-        tab[i] = w;
+        const int t = i - off;
+        tab[i] = band_weight(t < 0 ? -t : t, h, two_var);
     }
     __syncthreads();
 
@@ -119,14 +114,8 @@ filter_tile_kernel(const float* __restrict__ in, float* __restrict__ out, int K,
     float* tab = fsm;
     float4* chunk = reinterpret_cast<float4*>(fsm + ((tab_n + 3) & ~3));         // [2][FT_JC][FG]
     for (int i = threadIdx.x; i < tab_n; i += FT_THREADS) {
-        int t = i - off;
-        int at = t < 0 ? -t : t;
-        float w = 0.f;
-        if (at <= h) {
-            float sq = (float)((long long)at * (long long)at);
-            w = expf(-(__fdiv_rn(sq, two_var)));
-        }
-        tab[i] = w;
+        const int t = i - off;
+        tab[i] = band_weight(t < 0 ? -t : t, h, two_var);
     }
     const int a_tile = blockIdx.x * FT_TK;
     const int d_tile = blockIdx.y * TD;
@@ -214,36 +203,11 @@ filter_tile_kernel(const float* __restrict__ in, float* __restrict__ out, int K,
     }
 }
 
-// largest t with expf(-(float(t*t)/two_var)) > 0, found on the host with the same fp32 steps
-static int host_band_half_width(float two_var, int K) {
-    // expf underflows to 0 below about -103.98; search a small window around that root
-    double guess = sqrt(104.5 * (double)two_var);
-    long long t = (long long)guess + 2;
-    if (t > K) t = K;                      // rows further than K-1 apart never meet
-    while (t > 0) {
-        float sq = (float)(t * t);
-        float w = expf(-(sq / two_var));
-        if (w > 0.f) break;
-        --t;
-    }
-    return (int)t;
-}
-
-int filter_band_half_width(float two_var, int K) { return host_band_half_width(two_var, K); }
-
 // som_filter_tc.cu
 bool filter_tc_applicable(int K, int D, int h);
 size_t filter_tc_workspace_bytes(int K, int D, int h);
 int launch_filter_tc(const float* in, float* out, int K, int D, float two_var, int h, float scale, void* ws,
                      size_t ws_bytes, cudaStream_t st);
-
-// models/Codebook.py:118 -- Python double arithmetic, then one rounding to fp32 at the divide
-static inline float two_var_of(double neighbourhood_range) {
-    const double variance = -(neighbourhood_range / (2.0 * log(0.1)));
-    return (float)(2.0 * variance);
-}
-
-float filter_two_var(double neighbourhood_range) { return two_var_of(neighbourhood_range); }
 
 }  // namespace som
 
@@ -251,13 +215,13 @@ using namespace som;
 
 extern "C" int som_filter_half_width(int K, double neighbourhood_range) {
     if (K <= 0 || !(neighbourhood_range > 0.0)) return 0;
-    return host_band_half_width(two_var_of(neighbourhood_range), K);
+    return filter_band_half_width(filter_two_var(neighbourhood_range), K);
 }
 
 extern "C" size_t som_filter_workspace_bytes(int K, int D, double neighbourhood_range) {
     if (K <= 0 || D <= 0 || !(neighbourhood_range > 0.0)) return 0;
-    const float two_var = two_var_of(neighbourhood_range);
-    const int h = host_band_half_width(two_var, K);
+    const float two_var = filter_two_var(neighbourhood_range);
+    const int h = filter_band_half_width(two_var, K);
     return filter_tc_applicable(K, D, h) ? filter_tc_workspace_bytes(K, D, h) : 0;
 }
 
@@ -267,8 +231,8 @@ extern "C" int som_filter_ws_f32(const float* in, float* out, int K, int D, doub
     SOM_REQUIRE(in != out, SOM_E_BADARG, "filter: in-place operation is not supported");
     SOM_REQUIRE(K > 0 && D > 0, SOM_E_BADARG, "filter: K=%d D=%d", K, D);
     SOM_REQUIRE(neighbourhood_range > 0.0, SOM_E_BADARG, "filter: neighbourhood_range=%g", neighbourhood_range);
-    const float two_var = two_var_of(neighbourhood_range);
-    const int h = host_band_half_width(two_var, K);
+    const float two_var = filter_two_var(neighbourhood_range);
+    const int h = filter_band_half_width(two_var, K);
     // static rule on the shape: tensor cores for K >= 256 units and rows of >= 48 features (som_filter_tc.cu)
     if (filter_tc_applicable(K, D, h) && ws != nullptr)
         return launch_filter_tc(in, out, K, D, two_var, h, scale, ws, ws_bytes, (cudaStream_t)stream);
@@ -282,36 +246,28 @@ extern "C" int som_filter_f32(const float* in, float* out, int K, int D,
     SOM_REQUIRE(K > 0 && D > 0, SOM_E_BADARG, "filter: K=%d D=%d", K, D);
     SOM_REQUIRE(neighbourhood_range > 0.0, SOM_E_BADARG, "filter: neighbourhood_range=%g",
                 neighbourhood_range);
-    // models/Codebook.py:118 -- Python double arithmetic, then one rounding to fp32 at the divide
-    double variance = -(neighbourhood_range / (2.0 * log(0.1)));
-    float two_var = (float)(2.0 * variance);
-    int h = host_band_half_width(two_var, K);
+    const float two_var = filter_two_var(neighbourhood_range);
+    const int h = filter_band_half_width(two_var, K);
     size_t smem = (size_t)(2 * (h + FILT_PAD) + 1) * sizeof(float);
     SOM_REQUIRE(smem <= 200 * 1024, SOM_E_SHAPE, "filter: band half-width %d too large", h);
-    static PerDeviceFlag attr_set;   // idempotent; worst case it is set twice
-    if (smem > 48 * 1024 && attr_set.pending()) {
-        cudaError_t e = cudaFuncSetAttribute(filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             200 * 1024);
-        if (e != cudaSuccess) { set_error("filter: smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-        attr_set.set();
+    typedef void (*FilterFn)(const float*, float*, int, int, float, int, float);
+    if (smem > 48 * 1024) {
+        static PerDeviceFlag attr_done;
+        const FilterFn kernel = filter_kernel;
+        const int rc = smem_opt_in(attr_done, &kernel, 1, 200 * 1024, "filter");
+        if (rc) return rc;
     }
     if ((D & 3) == 0 && D >= 48 && (((uintptr_t)in | (uintptr_t)out) & 15) == 0) {
         const int td = D >= 128 ? 128 : 64;
         const size_t tab_n = (size_t)(2 * (h + FT_PAD) + 1);
         const size_t smem_t = ((tab_n + 3) & ~(size_t)3) * sizeof(float) + 2 * (size_t)FT_JC * td * sizeof(float);
         SOM_REQUIRE(smem_t <= 200 * 1024, SOM_E_SHAPE, "filter: band half-width %d too large", h);
-        static PerDeviceFlag attr_t;
-        if (attr_t.pending()) {
-            cudaError_t e = cudaFuncSetAttribute(filter_tile_kernel<128, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 200 * 1024);
-            if (e == cudaSuccess)
-                e = cudaFuncSetAttribute(filter_tile_kernel<64, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-            if (e != cudaSuccess) { set_error("filter: smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-            attr_t.set();
-        }
+        static const FilterFn tile_kernels[2] = {filter_tile_kernel<128, 2>, filter_tile_kernel<64, 4>};
+        static PerDeviceFlag attr_done;
+        const int rc = smem_opt_in(attr_done, tile_kernels, 2, 200 * 1024, "filter");
+        if (rc) return rc;
         dim3 gt((unsigned)ceil_div64(K, 32), (unsigned)ceil_div64(D, td));      // 32 units per CTA in both shapes
-        if (td == 128) launch_pdl(filter_tile_kernel<128, 2>, gt, FT_THREADS, smem_t, (cudaStream_t)stream, in, out, K, D, two_var, h, scale);
-        else launch_pdl(filter_tile_kernel<64, 4>, gt, FT_THREADS, smem_t, (cudaStream_t)stream, in, out, K, D, two_var, h, scale);
+        launch_pdl(tile_kernels[td == 64], gt, FT_THREADS, smem_t, (cudaStream_t)stream, in, out, K, D, two_var, h, scale);
         return check_launch("filter_tile_kernel");
     }
     dim3 grid((unsigned)ceil_div64(K, FILT_WARPS * FILT_TA), (unsigned)ceil_div64(D, 32));

@@ -24,6 +24,7 @@
 // Algorithmic work: 2*K*D*(2h+1) flop; executed: 3 * 2*128*TNF*L per tile with L = 32*ceil((128+2h)/32).
 #include "som_common.cuh"
 #include "som_peer.cuh"
+#include "som_step_rules.cuh"
 #include "som_tc_ptx.cuh"
 #include "som_tc_split.cuh"
 
@@ -160,16 +161,9 @@ filter_tc_kernel(const __grid_constant__ CUtensorMap map_bhi, const __grid_const
         mbar_init(&bars.acc_full, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    // weight table, generated exactly as the FFMA kernel / the reference do: (j-b)^2 exact, fp32 divide, expf
     for (int i = threadIdx.x; i < tab_n; i += NUM_THREADS) {
         const int t = i - off;
-        const int at = t < 0 ? -t : t;
-        float w = 0.f;
-        if (at <= P.h) {
-            const float sq = (float)((long long)at * (long long)at);
-            w = expf(-(__fdiv_rn(sq, P.two_var)));
-        }
-        tf32_split(w, tab_hi[i], tab_lo[i]);
+        tf32_split(band_weight(t < 0 ? -t : t, P.h, P.two_var), tab_hi[i], tab_lo[i]);
     }
     if (warp == 1) tmem_alloc(&bars.tmem_base, NACC * ACC_COLS);
     tc_fence_before();
@@ -388,9 +382,6 @@ static void make_plan(Plan* pl, int K, int D, int h) {
 }
 
 }  // namespace ftc
-
-// largest t with expf(-(float(t*t)/two_var)) > 0 (som_filter.cu)
-int filter_band_half_width(float two_var, int K);
 
 // Static rule on the shape: the tensor-core filter pays a transposing pre-pass and 128-unit tiles.
 bool filter_tc_applicable(int K, int D, int h) {

@@ -157,19 +157,9 @@ __global__ void __launch_bounds__(THREADS) bcast_rows_kernel(const float4* __res
     grid_sync_ranks<true, true>(pads, counter, channel, rank, world);
 }
 
-struct AdamScalars { float w1, b2, one_m_b2, step_size, bc2_sqrt, eps; };
-__device__ __forceinline__ void adam_update(const AdamScalars& a, float gi, float& mi, float& vi, float& wi) {
-    // torch.optim.Adam single-tensor rule, same arithmetic as som_core.cu's adam_update
-    float diff = gi - mi;
-    mi = (a.w1 < 0.5f) ? __fmaf_rn(a.w1, diff, mi) : __fmaf_rn(-diff, 1.0f - a.w1, gi);
-    vi = __fmaf_rn(a.one_m_b2 * gi, gi, vi * a.b2);
-    float denom = __fdiv_rn(__fsqrt_rn(vi), a.bc2_sqrt) + a.eps;
-    wi = __fmaf_rn(-a.step_size, __fdiv_rn(mi, denom), wi);
-}
-
 // Adam on the n4 float4 of this rank's rows (W, m, v, g all local pointers to the slice), new rows stored to every
-// rank's codebook through the multicast address, then the barrier.  g is unscaled: g * (float)(2 / numel), numel from
-// the reduced tail, as som_adam_dp_f32.
+// rank's codebook through the multicast address, then the barrier.  g is unscaled: scaled by the reduced tail's
+// gradient scale, as som_adam_dp_f32.
 __global__ void __launch_bounds__(THREADS) adam_slice_bcast_kernel(const float4* __restrict__ W, float* mc_W,
                                                                    float4* __restrict__ m, float4* __restrict__ v,
                                                                    const float4* __restrict__ g, int64_t n4, int D,
@@ -181,22 +171,13 @@ __global__ void __launch_bounds__(THREADS) adam_slice_bcast_kernel(const float4*
     pdl_begin();
     trace_stamp(s_trace_buf, 15);
     const double t = (double)(steps_done[0] + 1);
-    const double numel = ((double)tail[2] * 4096.0 + (double)tail[3]) * (double)D;
-    const float gs = (float)(2.0 / numel);
-    AdamScalars a;
-    a.w1 = (float)(1.0 - b1); a.b2 = (float)b2; a.one_m_b2 = (float)(1.0 - b2);
-    a.step_size = (float)(lr / (1.0 - pow(b1, t)));
-    a.bc2_sqrt = (float)sqrt(1.0 - pow(b2, t));
-    a.eps = eps;
-    if (loss_out != nullptr && blockIdx.x == 0 && threadIdx.x == 0)
-        *loss_out = ((double)tail[0] + (double)tail[1]) / numel;
+    const TailTotals tt = tail_totals(tail, D);
+    const AdamScalars a = adam_scalars(lr, b1, b2, eps, t);
+    if (loss_out != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *loss_out = tail_loss(tail, tt.numel);
     const int64_t stride = (int64_t)gridDim.x * THREADS;
     for (int64_t q = blockIdx.x * (int64_t)THREADS + threadIdx.x; q < n4; q += stride) {
         float4 gq = g[q], mq = m[q], vq = v[q], wq = W[q];
-        adam_update(a, gq.x * gs, mq.x, vq.x, wq.x);
-        adam_update(a, gq.y * gs, mq.y, vq.y, wq.y);
-        adam_update(a, gq.z * gs, mq.z, vq.z, wq.z);
-        adam_update(a, gq.w * gs, mq.w, vq.w, wq.w);
+        adam_update4<true>(a, gq, tt.gscale, mq, vq, wq);
         m[q] = mq; v[q] = vq;
         mm_st(mc_W + 4 * q, wq);
     }
@@ -229,9 +210,7 @@ static int grid_for(int64_t n4) {
 
 }  // namespace peer
 
-// som_filter.cu / som_filter_tc.cu
-float filter_two_var(double neighbourhood_range);
-int filter_band_half_width(float two_var, int K);
+// som_filter_tc.cu
 bool filter_tc_applicable(int K, int D, int h);
 int launch_filter_tc_peer(const float* mc_in, float* out, int K, int D, float two_var, int h, float scale, void* ws,
                           size_t ws_bytes, cudaStream_t st, const peer::Pads& bufs, int64_t q_tail, int world,

@@ -2,6 +2,7 @@
 // reducing load and the exact reduction of the packed buffer's 4-float tail.
 #pragma once
 #include "som_common.cuh"
+#include "som_step_rules.cuh"
 
 namespace som {
 namespace peer {
@@ -16,7 +17,7 @@ __device__ __forceinline__ float4 mm_ld_reduce(const float* mc) {
     return v;
 }
 
-// The 4-float tail [sse_hi, sse_lo, n / 4096, n % 4096] of the packed accumulator buffer is NOT reduced in the
+// The 4-float tail (pack_tail, som_step_rules.cuh) of the packed accumulator buffer is NOT reduced in the
 // switch: the in-switch fp32 adder is not exact enough for the loss (measured 1.2e-6 relative over 8 ranks), and the
 // patch count must be exact.  Every rank reads the R tails through the peer addresses and adds them in rank order,
 // the squared error in fp64 -- the same bits on every rank.
@@ -44,10 +45,8 @@ __device__ __forceinline__ float4 exact_tail(const Pads& bufs, int64_t q_tail, i
             }
         }
     }
-    const double cnt = cnt_hi * 4096.0 + cnt_lo;
-    const float hi = (float)sse;
-    const double c_hi = floor(cnt / 4096.0);
-    return make_float4(hi, (float)(sse - (double)hi), (float)c_hi, (float)(cnt - c_hi * 4096.0));
+    // the summed count is an exact integer in fp64
+    return pack_tail(sse, (int64_t)tail_count(cnt_hi, cnt_lo));
 }
 
 

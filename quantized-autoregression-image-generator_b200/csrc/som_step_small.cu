@@ -16,16 +16,16 @@
 //   phase 3  G rows = (2 / numel) sum_t w(t) Rbar[a+t], Adam on the own rows of W; CTA 0 adds the squared-error
 //            partials in CTA order (fp64), writes the loss and advances the step count
 //
-// Deterministic (fixed summation orders, no atomics).  Filter weights are generated exactly as the reference does
-// (integer t^2 -> fp32, divided by fp32(2 var), expf).  Everything stays in L2: the working set is K*D*4*5 bytes.
+// Deterministic (fixed summation orders, no atomics).  Filter weights and Adam follow som_step_rules.cuh.  Everything
+// stays in L2: the working set is K*D*4*5 bytes.
 #include "som_common.cuh"
+#include "som_step_rules.cuh"
 
 #include <cooperative_groups.h>
 
 namespace cg = cooperative_groups;
 
 namespace som {
-int filter_band_half_width(float two_var, int K);       // som_filter.cu
 namespace sstep {
 
 constexpr int THREADS = 256;
@@ -60,16 +60,6 @@ __device__ __forceinline__ void stamp(int i) {
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(v)::"memory");
         g_prof_small[i] = v;
     }
-}
-
-struct AdamScalars { float w1, b2, one_m_b2, step_size, bc2_sqrt, eps; };
-__device__ __forceinline__ void adam_update(const AdamScalars& a, float gi, float& mi, float& vi, float& wi) {
-    // torch.optim.Adam single-tensor rule, same arithmetic as som_core.cu's adam_update
-    float diff = gi - mi;
-    mi = (a.w1 < 0.5f) ? __fmaf_rn(a.w1, diff, mi) : __fmaf_rn(-diff, 1.0f - a.w1, gi);
-    vi = __fmaf_rn(a.one_m_b2 * gi, gi, vi * a.b2);
-    float denom = __fdiv_rn(__fsqrt_rn(vi), a.bc2_sqrt) + a.eps;
-    wi = __fmaf_rn(-a.step_size, __fdiv_rn(mi, denom), wi);
 }
 
 // Rows [a0, a1) of T @ in for the features of this thread.  The CTA first stages the input rows it needs,
@@ -141,18 +131,13 @@ __global__ void __launch_bounds__(THREADS, 1) step_small_kernel(const Params P) 
     const int d = threadIdx.x % D, g = threadIdx.x / D;
     const int64_t n = P.g.n_patches;
     const double t_step = (double)(P.steps_done[0] + 1);           // read before any barrier: CTA 0 bumps it at the end
-    for (int t = threadIdx.x; t <= h; t += THREADS) wtab[t] = expf(-(__fdiv_rn((float)t * (float)t, P.two_var)));
+    for (int t = threadIdx.x; t <= h; t += THREADS) wtab[t] = band_weight(t, h, P.two_var);
     for (int t = threadIdx.x; t < D; t += THREADS) foff[t] = feat_off(P.g, t);
     const int a0 = min(K, (int)blockIdx.x * P.R), a1 = min(K, a0 + P.R);
     const int R = a1 - a0;
     const int RB = (P.R + NQ - 1) / NQ;
     __shared__ AdamScalars adam_s;
-    if (threadIdx.x == 0) {                              // bias corrections in double as torch/optim/adam.py, once per CTA
-        adam_s.w1 = (float)(1.0 - P.b1); adam_s.b2 = (float)P.b2; adam_s.one_m_b2 = (float)(1.0 - P.b2);
-        adam_s.step_size = (float)(P.lr / (1.0 - pow(P.b1, t_step)));
-        adam_s.bc2_sqrt = (float)sqrt(1.0 - pow(P.b2, t_step));
-        adam_s.eps = P.eps;
-    }
+    if (threadIdx.x == 0) adam_s = adam_scalars(P.lr, P.b1, P.b2, P.eps, t_step);     // once per CTA
     stamp(0);
 
     // ---- phase 0: W~ rows of the own units --------------------------------------------------------------------------
@@ -414,9 +399,8 @@ static bool make_plan(Plan* pl, int64_t n, int D, int K, double range) {
     pl->R = (K + sms - 1) / sms;
     if (pl->R > RMAX) return false;
     pl->RB = (pl->R + THREADS / D - 1) / (THREADS / D);
-    const double variance = -(range / (2.0 * log(0.1)));
-    pl->two_var = (float)(2.0 * variance);
-    pl->h = som::filter_band_half_width(pl->two_var, K);
+    pl->two_var = filter_two_var(range);
+    pl->h = filter_band_half_width(pl->two_var, K);
     if (pl->h > HMAX) return false;
     if ((int64_t)(pl->R + 2 * pl->h) * D > UNION_FLOATS) return false;         // staged filter rows
     if (PB * D + PB * (CU + 1) > UNION_FLOATS) return false;                   // BMU phase: patches + scores
@@ -489,12 +473,8 @@ extern "C" int som_step_small_f32(const float* x, int64_t n_img, int C, int H, i
     KernelFn fn = fns[dslot][rslot];
     const size_t smem = smem_bytes();
     static PerDeviceFlag attr_done[15];
-    const int slot = 3 * dslot + rslot;
-    if (attr_done[slot].pending()) {
-        cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) { set_error("step_small: smem opt-in: %s", cudaGetErrorString(e)); return (int)e; }
-        attr_done[slot].set();
-    }
+    rc = smem_opt_in(attr_done[3 * dslot + rslot], &fn, 1, (int)smem, "step_small");
+    if (rc) return rc;
     void* args[] = {(void*)&P};
     cudaError_t le = cudaLaunchCooperativeKernel((const void*)fn, dim3((unsigned)pl.grid), dim3(THREADS), args, smem,
                                                  (cudaStream_t)stream);

@@ -388,7 +388,8 @@ def test_trainer_nan_guard():
 
 def test_packed_accumulate_and_device_scaled_adam_match_the_host_scaled_path():
     """som_accumulate_packed_nchw_f32 + som_adam_dp_f32 (batch size and loss on the device) against
-    som_accumulate_nchw_f32 + host-scaled filter + som_adam_f32: bit-identical weights, loss to fp64 rounding."""
+    som_accumulate_nchw_f32 + host-scaled filter + som_adam_f32: bit-identical weights, loss to fp64 rounding.
+    som_adam_devstep_f32 (step count on the device) on the host-scaled gradient: bit-identical weights and moments."""
     from oracle.step_oracle import synthetic_fmaps, trained_like_codebook
     pd, k, d = (4, 4), 2048, 64
     x = synthetic_fmaps(96, 5).to(DEV)
@@ -405,14 +406,19 @@ def test_packed_accumulate_and_device_scaled_adam_match_the_host_scaled_path():
     numel = x.numel()
     w_a, m_a, v_a = w.clone(), torch.zeros_like(w), torch.zeros_like(w)
     w_b, m_b, v_b = w.clone(), torch.zeros_like(w), torch.zeros_like(w)
+    w_c, m_c, v_c = w.clone(), torch.zeros_like(w), torch.zeros_like(w)
     t_dev = torch.zeros(2, dtype=torch.int64, device=DEV)
+    t_devstep = torch.zeros(1, dtype=torch.int64, device=DEV)
     for t in (1, 2, 3):
         g_a = ops.neighbourhood_filter(rbar, 300, scale=2.0 / numel)
         ops.adam_step(w_a, m_a, v_a, g_a, 1e-4, t)
         g_b = ops.neighbourhood_filter(rbar, 300, scale=1.0)
         loss = ops.adam_step_dp(w_b, m_b, v_b, g_b, d, 1e-4, t_dev, packed[k * d:])
-        assert torch.equal(w_a, w_b) and torch.equal(v_a, v_b)
+        assert torch.equal(w_a, w_b) and torch.equal(m_a, m_b) and torch.equal(v_a, v_b)
+        ops.adam_step_dev(w_c, m_c, v_c, g_a, 1e-4, t_devstep)
+        assert torch.equal(w_a, w_c) and torch.equal(m_a, m_c) and torch.equal(v_a, v_c)
     assert int(t_dev[0]) == 3 and int(t_dev[1]) == 0
+    assert int(t_devstep[0]) == 3
     assert abs(float(loss) - float(sse) / numel) <= 1e-12 * float(loss)
 
 
