@@ -137,6 +137,30 @@ SOM_API int som_bmu_flat_f32(const float* patches, int64_t n, int D,
                      int64_t* out_idx, float* out_rd,
                      void* ws, size_t ws_bytes, int variant, void* stream);
 
+/* ---- K0 / K1 with 16-bit codebooks (binary16 and bfloat16 weights; inference only) ---------------------------
+ * A 16-bit codebook means the weights ARE those values: every result equals the fp32 call on W.float() -- indices,
+ * reduced distances, unit_offset, NaN rows and ties included, for every variant.  w_dtype: 1 = binary16, 2 = bfloat16
+ * (the dtype codes of the feature-map shards); x_dtype: 0 = fp32, 1 = binary16, 2 = bfloat16.  W is K x D row-major,
+ * 2-byte aligned.
+ * som_prepare_codebook_w16: c_norm2 bit-identical to som_prepare_codebook_f32 on W.float() (same summation order). */
+SOM_API int    som_prepare_codebook_w16(const void* W, int w_dtype, int K, int D, float* c_norm2, void* stream);
+/* som_bmu_w16_nchw is som_bmu_nchw_f32 (x fp32) or som_bmu_stage_nchw_f16 / _bf16 without stage_rows (x 16-bit; like
+ * them SOM_E_UNSUPPORTED where som_bmu_f16_native says 0 -- pass the batch's fp32 copy then).  The workspace
+ * (som_bmu_w16_workspace_bytes) holds the fp32 search's workspace, an exact fp32 copy of W made on every call (the
+ * weights may have changed since the last one, as for c_norm2) and one flag bit per (256-unit tile, 64-feature block).
+ * The FP16-split kernel (16 < D <= 256) splits -2 s_c c into FP16 hi + lo; where every lo of a tile's block is zero it
+ * skips that block's B_lo load and its A_hi x B_lo product group (17 instead of 33 MMAs per tile at D = 256 when the
+ * batch is 16-bit too).  The dropped products are exact zeros, so the result does not depend on the skip:
+ *   binary16 : every finite lo is zero whenever s_c >= 1, i.e. whenever the largest unit norm is below 256 (a
+ *              tanh-range codebook has ||c|| <= sqrt(D) <= 16);
+ *   bfloat16 : lo is zero for an element within about 2^-23 of the largest |s_c c| of the codebook (the rule of bf16
+ *              patch rows); units far below the largest, subnormals, inf and NaN keep the product.
+ * The other kernels search the fp32 copy unchanged.                                                              */
+SOM_API size_t som_bmu_w16_workspace_bytes(int64_t n_patches, int D, int K, int variant);
+SOM_API int    som_bmu_w16_nchw(const void* x, int x_dtype, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                const void* W, int w_dtype, const float* c_norm2, int K, int64_t unit_offset,
+                                int64_t* out_idx, float* out_rd, void* ws, size_t ws_bytes, int variant, void* stream);
+
 /* ---- K1b: merge per-shard candidates (new; multi-GPU unit-sharded search) ---------------
  * rd, idx are (R, n) row-major; picks the smaller rd, ties -> the smaller global index,
  * which reproduces the single-device first-minimum rule when shards are index-ordered.   */
@@ -205,6 +229,11 @@ SOM_API int som_backward_nchw_f32(const float* grad_out, int64_t n_img, int C, i
 SOM_API int som_quantize_nchw_f32(const int64_t* idx, const float* table, int K,
                           int64_t n_img, int C, int H, int Wd, int pH, int pW,
                           float* out, void* stream);
+/* The same gather of 16-bit values (binary16, bfloat16 or any other 2-byte format: the bit patterns are copied
+ * exactly); table and out 2-byte aligned.  Decodes a 16-bit codebook in its own dtype.                          */
+SOM_API int som_quantize_nchw_b16(const int64_t* idx, const void* table, int K,
+                                  int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                  void* out, void* stream);
 
 /* ---- K4: Adam on the codebook (fast-path trainer; the drop-in leaves it to torch) -------
  * torch.optim.Adam(betas=(b1,b2), eps) single-tensor rule, no weight decay / amsgrad
@@ -300,6 +329,9 @@ SOM_API int som_peer_adam_slice_f32(const float* W_rows, void* mc_W_rows, float*
  * out[r] = W[keep[r]] for r < n_keep (prune_codebook.py:161-162).                        */
 SOM_API int som_gather_rows_f32(const float* W, int D, const int64_t* keep, int64_t n_keep,
                         float* out, void* stream);
+/* The same for 16-bit rows (bit patterns copied exactly, 2-byte aligned): pruning a 16-bit codebook.            */
+SOM_API int som_gather_rows_b16(const void* W, int D, const int64_t* keep, int64_t n_keep,
+                                void* out, void* stream);
 
 /* ---- dual-codebook token assembly (tokenisation call site of the Transformer trainer) ----
  * Replaces the index arithmetic of train_quantized_transformer.py:411-455 after the two

@@ -14,12 +14,12 @@ int tc_split_mode(int64_t n_patches, int D, int K, int arith);
 bool tc_can_stage(int64_t n_patches, int D, int K, int arith);
 int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn, int K,
                   int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
-                  int arith, cudaStream_t st);
+                  int arith, uint32_t* wflags, cudaStream_t st);
 bool tc_f16_native(int64_t n_patches, int D, int K, int arith);
 int tc_plan_fields(int64_t n_patches, int D, int K, int arith, int64_t* f);
 int launch_bmu_tc_16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K, int64_t unit_offset,
                       int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes, int arith,
-                      cudaStream_t st);
+                      uint32_t* wflags, cudaStream_t st);
 }  // namespace som
 
 using namespace som;
@@ -87,7 +87,7 @@ extern "C" int som_bmu_stage_nchw_f32(const float* x, int64_t n_img, int C, int 
         SOM_REQUIRE(tc_supported(g.n_patches, g.D, K), SOM_E_UNSUPPORTED,
                     "bmu: tensor-core variant does not support D=%d K=%d", g.D, K);
         return launch_bmu_tc(x, g, W, c_norm2, K, unit_offset, out_idx, out_rd, stage_rows, ws, ws_bytes,
-                             arith_of(variant), (cudaStream_t)stream);
+                             arith_of(variant), nullptr, (cudaStream_t)stream);
     }
     SOM_REQUIRE(stage_rows == nullptr, SOM_E_UNSUPPORTED, "bmu: the FFMA variant does not emit a staging copy");
     return launch_bmu_ffma(x, g, W, c_norm2, K, unit_offset, out_idx, out_rd, ws, ws_bytes,
@@ -136,7 +136,7 @@ static int bmu_stage_nchw_16(const char* who, int elem, const void* x, int64_t n
     if (variant == SOM_BMU_AUTO) variant = som_bmu_pick_variant(g.n_patches, g.D, K);
     SOM_REQUIRE(is_tc(variant), SOM_E_UNSUPPORTED, "%s: the FFMA variant does not read 16-bit input", who);
     return launch_bmu_tc_16(x, elem, g, W, c_norm2, K, unit_offset, out_idx, out_rd, stage_rows, ws, ws_bytes,
-                            arith_of(variant), (cudaStream_t)stream);
+                            arith_of(variant), nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int som_bmu_stage_nchw_f16(const void* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
@@ -161,4 +161,60 @@ extern "C" int som_bmu_flat_f32(const float* patches, int64_t n, int D, const fl
     SOM_REQUIRE(D > 0, SOM_E_BADARG, "bmu(flat): D=%d", D);
     return som_bmu_nchw_f32(patches, n, 1, 1, D, 1, D, W, c_norm2, K, unit_offset, out_idx, out_rd, ws, ws_bytes,
                             variant, stream);
+}
+
+// ---- 16-bit codebooks -----------------------------------------------------------------------------------------------
+// Workspace: [ the fp32 search's workspace | exact fp32 copy of W (K x D) | B-side flag words of the FP16-split kernel ]
+struct W16Layout { size_t w32, flags, total; };
+static W16Layout w16_layout(int64_t n_patches, int D, int K, int variant) {
+    W16Layout l;
+    l.w32 = align_up(som_bmu_workspace_bytes(n_patches, D, K, variant), 256);
+    l.flags = align_up(l.w32 + (size_t)K * D * sizeof(float), 256);
+    const int64_t bits = ceil_div64(K, 256) * ceil_div64(D, 64);           // (256-unit tile, 64-feature block) pairs
+    l.total = l.flags + align_up((size_t)ceil_div64(bits, 32) * 4, 256);
+    return l;
+}
+
+extern "C" size_t som_bmu_w16_workspace_bytes(int64_t n_patches, int D, int K, int variant) {
+    if (n_patches <= 0 || D <= 0 || K <= 0) return 0;
+    if (variant == SOM_BMU_AUTO) variant = som_bmu_pick_variant(n_patches, D, K);
+    return w16_layout(n_patches, D, K, variant).total;
+}
+
+extern "C" int som_bmu_w16_nchw(const void* x, int x_dtype, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                const void* W, int w_dtype, const float* c_norm2, int K, int64_t unit_offset,
+                                int64_t* out_idx, float* out_rd, void* ws, size_t ws_bytes, int variant, void* stream) {
+    SOM_REQUIRE(x_dtype >= ELEM_F32 && x_dtype <= ELEM_BF16, SOM_E_BADARG, "bmu(w16): x_dtype=%d", x_dtype);
+    SOM_REQUIRE(w_dtype == ELEM_F16 || w_dtype == ELEM_BF16, SOM_E_BADARG, "bmu(w16): w_dtype=%d", w_dtype);
+    SOM_REQUIRE(W && c_norm2 && ((x && out_idx) || n_img == 0), SOM_E_BADARG, "bmu(w16): null pointer");
+    SOM_REQUIRE(K > 0, SOM_E_BADARG, "bmu(w16): K=%d", K);
+    SOM_REQUIRE(variant >= SOM_BMU_AUTO && variant <= SOM_BMU_TC_F16, SOM_E_BADARG, "bmu(w16): variant=%d", variant);
+    SOM_REQUIRE(((uintptr_t)W & 1) == 0, SOM_E_BADARG, "bmu(w16): W is not 2-byte aligned");
+    Geom g;
+    int rc = make_geom(&g, x, n_img, C, H, Wd, pH, pW, x_dtype == ELEM_F32 ? 4 : 2);
+    if (rc) return rc;
+    if (g.n_patches == 0) return SOM_OK;
+    if (variant == SOM_BMU_AUTO) variant = som_bmu_pick_variant(g.n_patches, g.D, K);
+    SOM_REQUIRE(x_dtype == ELEM_F32 || som_bmu_f16_native(g.n_patches, g.D, K, variant), SOM_E_UNSUPPORTED,
+                "bmu(w16): no kernel reads a 16-bit batch at n=%lld D=%d K=%d (pass its fp32 copy)",
+                (long long)g.n_patches, g.D, K);
+    SOM_REQUIRE(!is_tc(variant) || tc_supported(g.n_patches, g.D, K), SOM_E_UNSUPPORTED,
+                "bmu(w16): tensor-core variant does not support D=%d K=%d", g.D, K);
+    const W16Layout l = w16_layout(g.n_patches, g.D, K, variant);
+    rc = check_workspace(ws, ws_bytes, l.total, "bmu(w16)");
+    if (rc) return rc;
+    float* w32 = (float*)((char*)ws + l.w32);
+    uint32_t* wflags = (uint32_t*)((char*)ws + l.flags);
+    cudaStream_t st = (cudaStream_t)stream;
+    // the exact fp32 copy, made per call for the same reason c_norm2 is: the weights may have changed since the last one
+    const int64_t nw = (int64_t)K * g.D;
+    rc = w_dtype == ELEM_F16 ? som_convert_f16_f32(W, nw, w32, stream) : som_convert_bf16_f32(W, nw, w32, stream);
+    if (rc) return rc;
+    if (x_dtype != ELEM_F32)
+        return launch_bmu_tc_16(x, x_dtype, g, w32, c_norm2, K, unit_offset, out_idx, out_rd, nullptr, ws, l.w32,
+                                arith_of(variant), wflags, st);
+    if (is_tc(variant))
+        return launch_bmu_tc((const float*)x, g, w32, c_norm2, K, unit_offset, out_idx, out_rd, nullptr, ws, l.w32,
+                             arith_of(variant), wflags, st);
+    return launch_bmu_ffma((const float*)x, g, w32, c_norm2, K, unit_offset, out_idx, out_rd, ws, l.w32, st);
 }

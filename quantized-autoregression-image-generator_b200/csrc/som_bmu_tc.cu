@@ -29,7 +29,7 @@ size_t tc_l16_workspace_bytes(int64_t n_patches, int D, int K, bool force);
 bool tc_l16_plan_fields(int64_t n_patches, int D, int K, bool force, int64_t* f);
 int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K,
                       int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
-                      bool force, cudaStream_t st);
+                      bool force, uint32_t* wflags, cudaStream_t st);
 // som_bmu_tc_l.cu
 size_t tc_l_workspace_bytes(int64_t n_patches, int D, int K);
 void tc_l_plan_fields(int64_t n_patches, int D, int K, int64_t* f);
@@ -108,19 +108,22 @@ int tc_plan_fields(int64_t n_patches, int D, int K, int arith, int64_t* f) {
 // kernel of 16 < D <= 256 (the same kernel as the one that stages)
 bool tc_f16_native(int64_t n_patches, int D, int K, int arith) { return tc_can_stage(n_patches, D, K, arith); }
 
+// wflags (launch_bmu_tc too): NULL, or the B-side flag words of a 16-bit codebook whose exact fp32 copy is W
+// (som_bmu_w16_nchw); only the FP16-split kernel reads them
 int launch_bmu_tc_16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K,
                      int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
-                     int arith, cudaStream_t st) {
+                     int arith, uint32_t* wflags, cudaStream_t st) {
     if (g.n_patches == 0) return SOM_OK;
     SOM_REQUIRE(tc_f16_native(g.n_patches, g.D, K, arith), SOM_E_UNSUPPORTED,
                 "bmu(%s): no kernel reads 16-bit input at n=%lld D=%d K=%d (ask som_bmu_f16_native first)",
                 elem == ELEM_BF16 ? "bf16" : "f16", (long long)g.n_patches, g.D, K);
-    return launch_bmu_tc_l16(x, elem, g, W, cn, K, unit_offset, out_idx, out_rd, stage, ws, ws_bytes, arith == 2, st);
+    return launch_bmu_tc_l16(x, elem, g, W, cn, K, unit_offset, out_idx, out_rd, stage, ws, ws_bytes, arith == 2, wflags,
+                             st);
 }
 
 int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn, int K,
                   int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
-                  int arith, cudaStream_t st) {
+                  int arith, uint32_t* wflags, cudaStream_t st) {
     if (g.n_patches == 0) return SOM_OK;
     SOM_REQUIRE(stage == nullptr || tc_can_stage(g.n_patches, g.D, K, arith), SOM_E_UNSUPPORTED,
                 "bmu: the kernel for this shape does not emit a staging copy (ask som_bmu_can_stage first)");
@@ -129,7 +132,7 @@ int launch_bmu_tc(const float* x, const Geom& g, const float* W, const float* cn
         return launch_bmu_tc_s(x, g, W, cn, K, unit_offset, out_idx, out_rd, ws, ws_bytes, arith, st);
     if (k == PLAN_L16)
         return launch_bmu_tc_l16(x, ELEM_F32, g, W, cn, K, unit_offset, out_idx, out_rd, stage, ws, ws_bytes, arith == 2,
-                                 st);
+                                 wflags, st);
     SOM_REQUIRE(k == PLAN_L, SOM_E_UNSUPPORTED, "bmu: no FP16-split kernel for D=%d K=%d (SOM_BMU_TC_F16)", g.D, K);
     return launch_bmu_tc_l(x, g, W, cn, K, unit_offset, out_idx, out_rd, ws, ws_bytes, st);
 }

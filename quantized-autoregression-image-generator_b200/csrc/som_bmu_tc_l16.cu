@@ -81,6 +81,7 @@ struct Params {
     Geom g;
     const float* scale;     // [s_c, t_c] written by cb_scale_l_kernel earlier on the stream
     float* stage;           // optional patch-major copy of the patch rows (n_patches x D), written by the builders
+    const uint32_t* wflags; // W16: bit n * DB + fb set = some lo(-2 s_c c) of unit tile n, block fb is non-zero
 };
 
 struct __align__(8) Barriers {
@@ -101,6 +102,11 @@ struct Aux {
     alignas(8) uint8_t lo_nz[NA_MAX][8];
 };
 constexpr uint32_t SMEM_BYTES = 1024 + TILES_BYTES + sizeof(Aux);
+// 16-bit codebooks: the B-side flags follow Aux, one bit per (unit tile, 64-feature block); 32 768 bits cover 2^21
+// units at D = 256.  A codebook with more (tile, block) pairs runs the kernel without the skip.
+constexpr int WFLAG_WORDS_MAX = 1024;
+constexpr uint32_t SMEM_BYTES_W16 = SMEM_BYTES + WFLAG_WORDS_MAX * 4;
+static_assert(SMEM_BYTES_W16 <= 227 * 1024, "FP16-split kernel: shared memory over the 227 KB limit");
 
 __device__ long long g_prof16[8];             // CTA 0's MMA loop: cycles, tiles, cycles waiting (acc_empty, B, A)
 
@@ -108,7 +114,10 @@ __device__ long long g_prof16[8];             // CTA 0's MMA loop: cycles, tiles
 // (block 0) the norm tail -- so the issuing thread pays ONE barrier wait and ONE commit per block instead of three.
 // With 13 MMAs per tile the issuing thread, not the tensor pipe, sets the pace otherwise (~48 cycles per MMA issue,
 // ~100 per barrier check, ~120 per commit).
-template <int CG, bool MERGED, typename T>
+//
+// W16 (a 16-bit codebook): where every lo(-2 s_c c) of a (unit tile, 64-feature block) is zero, the producers skip that
+// block's B_lo load and the issuer its A_hi x B_lo group.  Both CTAs of a pair read the same per-tile flag.
+template <int CG, bool MERGED, typename T, bool W16 = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_t, const Params P) {
     constexpr bool IN16 = sizeof(T) == 2;          // a 16-bit input type (__half or __nv_bfloat16)
@@ -162,6 +171,17 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
     const uint32_t tmem_base = bars.tmem_base;
     pdl_wait();
     trace_stamp(s_trace_buf, 7);
+    uint32_t* wbits = reinterpret_cast<uint32_t*>(tiles + TILES_BYTES + sizeof(Aux));
+    if (W16) {                          // the flags of split_w_l16_kernel, once per CTA
+        for (int w = threadIdx.x; w < (P.NT * DB + 31) >> 5; w += NUM_THREADS) wbits[w] = P.wflags[w];
+        __syncthreads();
+    }
+    // whether unit tile n, block fb needs its B_lo block
+    auto b_lo = [&](int n, int fb) -> bool {
+        if (!W16) return true;
+        const int b = n * DB + fb;
+        return (wbits[b >> 5] >> (b & 31)) & 1u;
+    };
 
     if (warp == 0) {
         // ================================ TMA producer ================================
@@ -174,11 +194,14 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                 for (int n = 0; n < P.NT; ++n) {
                     if (MERGED) {
                         for (int fb = 0; fb < DB; ++fb) {
+                            const bool blo = b_lo(n, fb);
                             mbar_wait(&bars.b_empty[bs], b_ph ^ 1);
-                            if (rank == 0) mbar_expect_tx(&bars.b_full[bs], 2 * B_BLK_BYTES + (fb == 0 ? TAIL_B_BYTES : 0));
+                            if (rank == 0)
+                                mbar_expect_tx(&bars.b_full[bs], (blo ? 2 : 1) * B_BLK_BYTES + (fb == 0 ? TAIL_B_BYTES : 0));
                             uint8_t* dst = b_ring + (size_t)bs * M_STAGE;
 #pragma unroll
                             for (int part = 0; part < 2; ++part) {
+                                if (part == 1 && !blo) break;           // the lo slot stays untouched
                                 if (CG == 1) tma_load_2d(&map_b, &bars.b_full[bs], dst + part * B_STAGE, (part * DB + fb) * KBLK, n * TN);
                                 else tma_load_2d_pair(&map_b, &bars.b_full[bs], dst + part * B_STAGE, (part * DB + fb) * KBLK, n * TN + row_off);
                             }
@@ -196,8 +219,10 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     else tma_load_2d_pair(&map_t, &bars.t_full[ts], t_ring + ts * T_STAGE, 0, n * TN + row_off);
                     if (++ts == 2) { ts = 0; t_ph ^= 1; }
                     for (int fb = 0; fb < DB; ++fb) {
+                        const bool blo = b_lo(n, fb);
 #pragma unroll
-                        for (int part = 0; part < 2; ++part) {      // hi block, then lo block
+                        for (int part = 0; part < 2; ++part) {      // hi block, then lo block (no ring stage without it)
+                            if (part == 1 && !blo) break;
                             mbar_wait(&bars.b_empty[bs], b_ph ^ 1);
                             if (rank == 0) mbar_expect_tx(&bars.b_full[bs], B_BLK_BYTES);
                             uint8_t* dst = b_ring + (size_t)bs * B_STAGE;
@@ -275,9 +300,11 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                                 for (int k = 0; k < 4; ++k)
                                     if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, alo + 2u * k, bhi + 2u * k, 1u);
                             }
+                            if (b_lo(n, fb)) {
 #pragma unroll
-                            for (int k = 0; k < 4; ++k)
-                                if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, ahi + 2u * k, blo + 2u * k, 1u);
+                                for (int k = 0; k < 4; ++k)
+                                    if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, ahi + 2u * k, blo + 2u * k, 1u);
+                            }
                             tc_commit<CG>(&bars.b_empty[bs]);
                             if (n == P.NT - 1) tc_commit<CG>(&bars.a_empty[as]);
                         }
@@ -309,6 +336,7 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                     }
                     const uint64_t ahi = adesc0 + (uint32_t)as * A_SLOT_UNITS;
                     const uint64_t alo = ahi + A_LO_UNITS;
+                    const bool blo = b_lo(n, fb);
                     mma_wait(&bars.b_full[bs], b_ph);
                     tc_fence_after();
                     uint64_t bd = bdesc0 + (uint32_t)bs * B_UNITS;
@@ -322,8 +350,10 @@ bmu_tc_l16_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_consta
                                 if (k < nks) tc_mma<MmaKind::F16, CG>(d_addr, alo + 2u * k, bd + 2u * k, 1u);
                         }
                         tc_commit<CG>(&bars.b_empty[bs]);
+                        if (!blo && n == P.NT - 1) tc_commit<CG>(&bars.a_empty[as]);
                     }
                     if (++bs == NB) { bs = 0; b_ph ^= 1; }
+                    if (!blo) continue;                         // the producer loaded no lo stage
                     mma_wait(&bars.b_full[bs], b_ph);
                     tc_fence_after();
                     bd = bdesc0 + (uint32_t)bs * B_UNITS;
@@ -523,6 +553,9 @@ __global__ void __launch_bounds__(1024) cb_scale_l_kernel(const float* __restric
 // One thread per (row, pair of features).  OWN_SCALE (codebooks of up to 32 768 units): every CTA derives the two
 // scales itself from the K norms (L2-resident) instead of waiting for cb_scale_l_kernel -- one launch fewer on the
 // per-step critical path; CTA 0 publishes them for the search kernel.
+// W16 (16-bit codebooks; W is their exact fp32 copy): a warp covers one (row, 64-feature block), and ORs the bit of its
+// (unit tile, block) into wflags (zeroed on the stream before) when some lo of it is non-zero -- NaN counts, as for the
+// patch rows.  The flag is a property of the values only, so it is the same in every launch and graph replay.
 __device__ __forceinline__ void scales_from_max_norm(float mn, float* out2) {
     // a NaN norm is dropped by fmaxf; an infinite one shows up as exponent 0xff
     const int en = (int)((__float_as_uint(mn) >> 23) & 0xffu);
@@ -539,11 +572,11 @@ __device__ __forceinline__ void scales_from_max_norm(float mn, float* out2) {
     out2[1] = __uint_as_float((uint32_t)(127 + g) << 23);
 }
 
-template <bool OWN_SCALE>
+template <bool OWN_SCALE, bool W16 = false>
 __global__ void __launch_bounds__(256) split_w_l16_kernel(const float* __restrict__ W, const float* __restrict__ cn,
                                                           int K, int D, int DB, int K_pad,
                                                           float* __restrict__ scale, __half* __restrict__ Bp,
-                                                          __half* __restrict__ Tp) {
+                                                          __half* __restrict__ Tp, uint32_t* __restrict__ wflags) {
     pdl_begin();
     trace_stamp(s_trace_buf, 6);
     __shared__ float sh_max[8];
@@ -575,6 +608,13 @@ __global__ void __launch_bounds__(256) split_w_l16_kernel(const float* __restric
     float h0, l0, h1, l1;
     f16_split(v0, h0, l0);
     f16_split(v1, h1, l1);
+    if (W16) {                  // K_pad * pairs is a multiple of 32: whole warps return above
+        const unsigned nz = __ballot_sync(0xffffffffu, l0 != 0.f || l1 != 0.f);
+        if (nz != 0u && (threadIdx.x & 31) == 0) {
+            const int b = (row / TN) * DB + d / 64;
+            atomicOr(wflags + (b >> 5), 1u << (b & 31));
+        }
+    }
     const int64_t cols = (int64_t)DB * 64;
     __half* rowp = Bp + (int64_t)row * 2 * cols;
     *reinterpret_cast<__half2*>(rowp + d) = __floats2half2_rn(h0, h1);
@@ -653,7 +693,7 @@ bool tc_l16_plan_fields(int64_t n_patches, int D, int K, bool force, int64_t* f)
 
 int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, const float* cn, int K,
                       int64_t unit_offset, int64_t* out_idx, float* out_rd, float* stage, void* ws, size_t ws_bytes,
-                      bool force, cudaStream_t st) {
+                      bool force, uint32_t* wflags, cudaStream_t st) {
     using namespace tcl16;
     SOM_REQUIRE(elem == ELEM_F32 || elem == ELEM_F16 || elem == ELEM_BF16, SOM_E_BADARG, "bmu(tc f16): element type %d",
                 elem);
@@ -667,16 +707,25 @@ int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, co
     __half* Bp = (__half*)((char*)ws + pl.off_b);
     __half* Tp = (__half*)((char*)ws + pl.off_t);
     float* scale = (float*)((char*)ws + pl.off_s);
+    // wflags: a 16-bit codebook (W its exact fp32 copy) whose (tile, block) pairs fit the kernel's flag words
+    const int wwords = (pl.NT * pl.DB + 31) / 32;
+    const bool w16 = wflags != nullptr && wwords <= WFLAG_WORDS_MAX;
+    if (w16) {
+        const cudaError_t me = cudaMemsetAsync(wflags, 0, (size_t)wwords * 4, st);
+        if (me != cudaSuccess) { set_error("bmu(tc f16): flag reset: %s", cudaGetErrorString(me)); return (int)me; }
+    }
     {
         const int64_t items = (int64_t)pl.K_pad * pl.DB * 32;
         const unsigned blocks = (unsigned)ceil_div64(items, 256);
         if (K <= 32768) {
-            launch_pdl(split_w_l16_kernel<true>, blocks, 256, 0, st, W, cn, K, g.D, pl.DB, pl.K_pad, scale, Bp, Tp);
+            launch_pdl(w16 ? split_w_l16_kernel<true, true> : split_w_l16_kernel<true>, blocks, 256, 0, st, W, cn, K,
+                       g.D, pl.DB, pl.K_pad, scale, Bp, Tp, wflags);
         } else {
             launch_pdl(cb_scale_l_kernel, 1, 1024, 0, st, cn, K, scale);
             rc = check_launch("cb_scale_l_kernel");
             if (rc) return rc;
-            launch_pdl(split_w_l16_kernel<false>, blocks, 256, 0, st, W, cn, K, g.D, pl.DB, pl.K_pad, scale, Bp, Tp);
+            launch_pdl(w16 ? split_w_l16_kernel<false, true> : split_w_l16_kernel<false>, blocks, 256, 0, st, W, cn, K,
+                       g.D, pl.DB, pl.K_pad, scale, Bp, Tp, wflags);
         }
         rc = check_launch("split_w_l16_kernel");
         if (rc) return rc;
@@ -693,7 +742,7 @@ int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, co
     Params P;
     P.DB = pl.DB; P.nks_last = pl.nks_last; P.NT = pl.NT; P.n_mtiles = pl.n_mtiles; P.NA = pl.NA; P.NB = pl.NB;
     P.K_pad = pl.K_pad; P.rows = n; P.unit_offset = unit_offset; P.out_idx = out_idx; P.out_rd = out_rd;
-    P.x = x; P.g = g; P.scale = scale; P.stage = stage;
+    P.x = x; P.g = g; P.scale = scale; P.stage = stage; P.wflags = wflags;
 
     typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const Params);
     // [elem][merged][cg - 1], elem = ELEM_F32 / ELEM_F16 / ELEM_BF16
@@ -704,15 +753,24 @@ int launch_bmu_tc_l16(const void* x, int elem, const Geom& g, const float* W, co
         bmu_tc_l16_kernel<1, true, __half>, bmu_tc_l16_kernel<2, true, __half>,
         bmu_tc_l16_kernel<1, false, __nv_bfloat16>, bmu_tc_l16_kernel<2, false, __nv_bfloat16>,
         bmu_tc_l16_kernel<1, true, __nv_bfloat16>, bmu_tc_l16_kernel<2, true, __nv_bfloat16>};
-    static PerDeviceFlag attr_done;
-    rc = smem_opt_in(attr_done, kernels, 12, (int)SMEM_BYTES, "bmu(tc f16)");
+    static const KernelFn kernels_w16[12] = {
+        bmu_tc_l16_kernel<1, false, float, true>, bmu_tc_l16_kernel<2, false, float, true>,
+        bmu_tc_l16_kernel<1, true, float, true>, bmu_tc_l16_kernel<2, true, float, true>,
+        bmu_tc_l16_kernel<1, false, __half, true>, bmu_tc_l16_kernel<2, false, __half, true>,
+        bmu_tc_l16_kernel<1, true, __half, true>, bmu_tc_l16_kernel<2, true, __half, true>,
+        bmu_tc_l16_kernel<1, false, __nv_bfloat16, true>, bmu_tc_l16_kernel<2, false, __nv_bfloat16, true>,
+        bmu_tc_l16_kernel<1, true, __nv_bfloat16, true>, bmu_tc_l16_kernel<2, true, __nv_bfloat16, true>};
+    static PerDeviceFlag attr_done, attr_done_w16;
+    rc = w16 ? smem_opt_in(attr_done_w16, kernels_w16, 12, (int)SMEM_BYTES_W16, "bmu(tc f16)")
+             : smem_opt_in(attr_done, kernels, 12, (int)SMEM_BYTES, "bmu(tc f16)");
     if (rc) return rc;
     const int n_jobs = (pl.n_mtiles + pl.cg - 1) / pl.cg;
     const int max_groups = sm_count() / pl.cg;
     const int groups = n_jobs < max_groups ? n_jobs : max_groups;
     // a cluster of cg CTAs, and PDL (see som_common.cuh: pdl_begin)
-    cudaError_t le = launch_kernel(kernels[4 * elem + 2 * pl.merged + pl.cg - 1], (unsigned)(groups * pl.cg), NUM_THREADS,
-                                   SMEM_BYTES, st, (unsigned)pl.cg, true, map_b, map_t, P);
+    const int ki = 4 * elem + 2 * pl.merged + pl.cg - 1;
+    cudaError_t le = launch_kernel(w16 ? kernels_w16[ki] : kernels[ki], (unsigned)(groups * pl.cg), NUM_THREADS,
+                                   w16 ? SMEM_BYTES_W16 : SMEM_BYTES, st, (unsigned)pl.cg, true, map_b, map_t, P);
     if (le != cudaSuccess) { set_error("bmu_tc_l16_kernel: launch: %s", cudaGetErrorString(le)); return (int)le; }
     return check_launch("bmu_tc_l16_kernel");
 }

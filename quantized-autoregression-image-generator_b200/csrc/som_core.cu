@@ -97,8 +97,14 @@ int make_geom(Geom* g, const void* x, int64_t n_img, int C, int H, int W, int pH
 // original order (a masked element contributes fma(0, 0, s) = s), so the result is bit-identical to the
 // one-warp-per-unit, lane-strided order.  A warp owns (32 / G) * U consecutive units and has U * J loads in flight
 // per lane (short rows were latency-bound at 10-26 % of the HBM copy rate with one load in flight).
-template <int G, int U, int J>
-__global__ void __launch_bounds__(256) norm2_kernel(const float* __restrict__ W, int K, int D,
+// T = __half / __nv_bfloat16 (16-bit codebooks): each element is widened exactly and summed in the same order, so the
+// norms equal those of the codebook's fp32 copy bit for bit.
+__device__ __forceinline__ float ld_widen(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_widen(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ float ld_widen(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+
+template <int G, int U, int J, typename T = float>
+__global__ void __launch_bounds__(256) norm2_kernel(const T* __restrict__ W, int K, int D,
                                                     float* __restrict__ out) {
     pdl_begin();
     trace_stamp(s_trace_buf, 5);
@@ -118,7 +124,7 @@ __global__ void __launch_bounds__(256) norm2_kernel(const float* __restrict__ W,
             for (int k = 0; k < U; ++k)
 #pragma unroll
                 for (int j = 0; j < J; ++j)
-                    v[k][j] = (r[k] < K && d0 + 32 * j < D) ? __ldg(W + r[k] * D + d0 + 32 * j) : 0.f;
+                    v[k][j] = (r[k] < K && d0 + 32 * j < D) ? ld_widen(W + r[k] * D + d0 + 32 * j) : 0.f;
 #pragma unroll
             for (int k = 0; k < U; ++k)
 #pragma unroll
@@ -137,16 +143,17 @@ __global__ void __launch_bounds__(256) norm2_kernel(const float* __restrict__ W,
 // per four units leaves most SMs without work (C3: 128 warps, 16 us for 8 MB).  Thread t adds d = t, t + 256, ... in
 // order (four loads in flight), then a warp butterfly and the eight warp sums in warp order: fixed order, and the
 // rule depends on D only, so a unit's norm does not depend on how many units the launch (or the shard) holds.
-__global__ void __launch_bounds__(256) norm2_long_kernel(const float* __restrict__ W, int D, float* __restrict__ out) {
+template <typename T = float>
+__global__ void __launch_bounds__(256) norm2_long_kernel(const T* __restrict__ W, int D, float* __restrict__ out) {
     pdl_begin();
     trace_stamp(s_trace_buf, 5);
     __shared__ float part[8];
-    const float* row = W + (int64_t)blockIdx.x * D;
+    const T* row = W + (int64_t)blockIdx.x * D;
     float s = 0.f;
     for (int d0 = threadIdx.x; d0 < D; d0 += 4 * 256) {
         float v[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) v[j] = (d0 + 256 * j < D) ? __ldg(row + d0 + 256 * j) : 0.f;
+        for (int j = 0; j < 4; ++j) v[j] = (d0 + 256 * j < D) ? ld_widen(row + d0 + 256 * j) : 0.f;
 #pragma unroll
         for (int j = 0; j < 4; ++j) s = fmaf(v[j], v[j], s);
     }
@@ -332,12 +339,14 @@ __global__ void __launch_bounds__(256) assemble_tokens_kernel(const int64_t* __r
 
 // ---------------------------------------------------------------------------------------------
 // quantise: out[offset(p, d)] = table[idx[p]][d]   (gather + fused unpatchify)
-// one thread per VEC-wide run; consecutive threads walk d fastest inside a patch
+// one thread per VEC-wide run; consecutive threads walk d fastest inside a patch.  T: float, or a 16-bit element
+// (any format: the values are copied as bit patterns)
 // ---------------------------------------------------------------------------------------------
-template <int VEC>
+template <int VEC, typename T = float>
 __global__ void __launch_bounds__(256) quantize_kernel(const int64_t* __restrict__ idx,
-                                                       const float* __restrict__ table, int K,
-                                                       Geom g, float* __restrict__ out) {
+                                                       const T* __restrict__ table, int K,
+                                                       Geom g, T* __restrict__ out) {
+    constexpr int RUN = VEC * (int)sizeof(T);             // bytes per run
     const int dv = g.D / VEC;
     int64_t total = g.n_patches * dv;
     int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -347,10 +356,11 @@ __global__ void __launch_bounds__(256) quantize_kernel(const int64_t* __restrict
         int64_t u = idx[p];
         if (u < 0) u = 0;
         if (u >= K) u = K - 1;
-        const float* src = table + u * (int64_t)g.D + d;
-        float* dst = out + patch_base(g, p) + feat_off(g, d);
-        if (VEC == 4) *reinterpret_cast<float4*>(dst) = *reinterpret_cast<const float4*>(src);
-        else if (VEC == 2) *reinterpret_cast<float2*>(dst) = *reinterpret_cast<const float2*>(src);
+        const T* src = table + u * (int64_t)g.D + d;
+        T* dst = out + patch_base(g, p) + feat_off(g, d);
+        if (RUN == 16) *reinterpret_cast<float4*>(dst) = *reinterpret_cast<const float4*>(src);
+        else if (RUN == 8) *reinterpret_cast<float2*>(dst) = *reinterpret_cast<const float2*>(src);
+        else if (RUN == 4) *reinterpret_cast<float*>(dst) = *reinterpret_cast<const float*>(src);
         else *dst = *src;
     }
 }
@@ -361,13 +371,15 @@ __global__ void __launch_bounds__(256) quantize_kernel(const int64_t* __restrict
 // then walks images, so the loop has no integer division (the first output-ordered version spent its time there:
 // ~300 instructions per run).  Per image a thread loads its U (2U for pW = 2) indices, then the table rows from L2,
 // then issues streaming stores.  The patch-ordered kernel above reached 21-36 % of the HBM copy rate.
-template <bool PW2>
+// A run holds V = 16 / sizeof(T) values: 4 floats, or 8 16-bit values (then PW2 means pW == 4).
+template <bool PW2, typename T = float>
 __global__ void __launch_bounds__(256, 4) quantize_out_kernel(const int64_t* __restrict__ idx,
-                                                           const float* __restrict__ table, int K,
-                                                           Geom g, float* __restrict__ out) {
+                                                           const T* __restrict__ table, int K,
+                                                           Geom g, T* __restrict__ out) {
     constexpr int U = 4;
-    const int wq = g.W >> 2;                              // 16-byte runs per image row
-    const int quads_img = (int)(g.img_stride >> 2);
+    constexpr int LV = sizeof(T) == 4 ? 2 : 3;            // log2 V
+    const int wq = g.W >> LV;                             // 16-byte runs per image row
+    const int quads_img = (int)(g.img_stride >> LV);
     int slot[U], d[U], r[U];
 #pragma unroll
     for (int k = 0; k < U; ++k) {
@@ -375,7 +387,7 @@ __global__ void __launch_bounds__(256, 4) quantize_out_kernel(const int64_t* __r
         slot[k] = -1; d[k] = 0;
         if (r[k] < quads_img) {
             const int row = r[k] / wq;                    // c * H + h
-            const int w = (r[k] - row * wq) << 2;
+            const int w = (r[k] - row * wq) << LV;
             const int c = row / g.H;
             const int h = row - c * g.H;
             const int ph = h / g.pH;
@@ -519,9 +531,10 @@ __global__ void __launch_bounds__(256) adam_dp_kernel(float* __restrict__ W, flo
     }
 }
 
-__global__ void __launch_bounds__(256) gather_rows_kernel(const float* __restrict__ W, int D,
+template <typename T = float>
+__global__ void __launch_bounds__(256) gather_rows_kernel(const T* __restrict__ W, int D,
                                                           const int64_t* __restrict__ keep,
-                                                          int64_t n_keep, float* __restrict__ out) {
+                                                          int64_t n_keep, T* __restrict__ out) {
     int64_t total = n_keep * D;
     int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < total; t += stride) {
@@ -531,7 +544,8 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const float* __restric
     }
 }
 
-// D % 4 == 0, 16-byte aligned rows: one 16-byte run per thread, four in flight
+// 16-byte aligned rows of a multiple of 16 bytes (4 floats, 8 16-bit values): one 16-byte run per thread, four in
+// flight
 __global__ void __launch_bounds__(256) gather_rows4_kernel(const float4* __restrict__ W, int D4,
                                                            const int64_t* __restrict__ keep,
                                                            int64_t n_keep, float4* __restrict__ out) {
@@ -611,6 +625,82 @@ static int convert_16_f32(const char* who, const void* in, int64_t n, float* out
     return check_launch("convert_16_f32_kernel");
 }
 
+template <typename T>
+static int prepare_codebook(const T* W, int K, int D, float* c_norm2, void* stream) {
+    SOM_REQUIRE(W && c_norm2, SOM_E_BADARG, "prepare_codebook: null pointer");
+    SOM_REQUIRE(K > 0 && D > 0, SOM_E_BADARG, "prepare_codebook: K=%d D=%d", K, D);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (D >= 2048) {
+        launch_pdl(norm2_long_kernel<T>, (unsigned)K, 256, 0, st, W, D, c_norm2);
+        return check_launch("norm2_long_kernel");
+    }
+    if (D > 16) {            // 4 units x 4 row segments in flight per lane
+        int blocks = grid_for(ceil_div64(K, 4) * 32, 256, 8);
+        launch_pdl(norm2_kernel<32, 4, 4, T>, blocks, 256, 0, st, W, K, D, c_norm2);
+    } else if (D > 8) {      // 2 x 8 units per warp
+        int blocks = grid_for(ceil_div64(K, 16) * 32, 256, 8);
+        launch_pdl(norm2_kernel<16, 8, 1, T>, blocks, 256, 0, st, W, K, D, c_norm2);
+    } else {                 // 4 x 8 units per warp
+        int blocks = grid_for(ceil_div64(K, 32) * 32, 256, 8);
+        launch_pdl(norm2_kernel<8, 8, 1, T>, blocks, 256, 0, st, W, K, D, c_norm2);
+    }
+    return check_launch("norm2_kernel");
+}
+
+// V = values per 16-byte run: 4 floats or 8 16-bit values
+template <typename T>
+static int quantize_nchw(const int64_t* idx, const T* table, int K, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                         T* out, void* stream) {
+    constexpr int ES = (int)sizeof(T), V = 16 / ES;
+    SOM_REQUIRE(table && ((idx && out) || n_img == 0), SOM_E_BADARG, "quantize: null pointer");
+    SOM_REQUIRE(K > 0, SOM_E_BADARG, "quantize: K=%d", K);
+    Geom g;
+    int rc = make_geom(&g, out, n_img, C, H, Wd, pH, pW, ES);
+    if (rc) return rc;
+    if (g.n_patches == 0) return SOM_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    const bool pw4 = (pW % V == 0), pw2 = (pW == V / 2);
+    if (Wd % V == 0 && ((uintptr_t)out & 15) == 0 && (pw4 || pw2) && g.img_stride >= 256 * V &&
+        g.img_stride / (256 * V) < 65535 &&
+        ((uintptr_t)table & (pw4 ? 15 : 7)) == 0) {
+        const int64_t quads_img = g.img_stride / V;
+        const int gy = (int)ceil_div64(quads_img, 256 * 4);
+        int gx = sm_count() * 8 / gy;
+        if (gx < 1) gx = 1;
+        if (gx > g.n_img) gx = (int)g.n_img;
+        dim3 blocks((unsigned)gx, (unsigned)gy);
+        if (pw2) quantize_out_kernel<true, T><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
+        else quantize_out_kernel<false, T><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
+        return check_launch("quantize_out_kernel");
+    }
+    int vec = g.vec;
+    if (((uintptr_t)table & (4 * ES - 1)) != 0 || g.D % 4 != 0) vec = (vec == 4) ? 1 : vec;
+    if (vec == 2 && (((uintptr_t)table & (2 * ES - 1)) != 0 || g.D % 2 != 0)) vec = 1;
+    int64_t items = g.n_patches * (g.D / vec);
+    int blocks = grid_for(items, 256, 16);
+    if (vec == 4) quantize_kernel<4, T><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
+    else if (vec == 2) quantize_kernel<2, T><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
+    else quantize_kernel<1, T><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
+    return check_launch("quantize_kernel");
+}
+
+template <typename T>
+static int gather_rows(const T* W, int D, const int64_t* keep, int64_t n_keep, T* out, void* stream) {
+    constexpr int V = 16 / (int)sizeof(T);
+    SOM_REQUIRE(W && keep && out, SOM_E_BADARG, "gather_rows: null pointer");
+    SOM_REQUIRE(D > 0 && n_keep >= 0, SOM_E_BADARG, "gather_rows: D=%d n_keep=%lld", D, (long long)n_keep);
+    if (n_keep == 0) return SOM_OK;
+    if (D % V == 0 && (((uintptr_t)W | (uintptr_t)out) & 15) == 0) {
+        int blocks = grid_for(n_keep * (D / V), 256 * 4, 8);
+        gather_rows4_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const float4*>(W), D / V, keep,
+                                                                      n_keep, reinterpret_cast<float4*>(out));
+        return check_launch("gather_rows4_kernel");
+    }
+    int blocks = grid_for(n_keep * D, 256, 16);
+    gather_rows_kernel<T><<<blocks, 256, 0, (cudaStream_t)stream>>>(W, D, keep, n_keep, out);
+    return check_launch("gather_rows_kernel");
+}
+
 }  // namespace som
 
 using namespace som;
@@ -658,26 +748,6 @@ int som_device_info(int* sm, int* major, int* minor) {
     return SOM_OK;
 }
 
-int som_prepare_codebook_f32(const float* W, int K, int D, float* c_norm2, void* stream) {
-    SOM_REQUIRE(W && c_norm2, SOM_E_BADARG, "prepare_codebook: null pointer");
-    SOM_REQUIRE(K > 0 && D > 0, SOM_E_BADARG, "prepare_codebook: K=%d D=%d", K, D);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (D >= 2048) {
-        launch_pdl(norm2_long_kernel, (unsigned)K, 256, 0, st, W, D, c_norm2);
-        return check_launch("norm2_long_kernel");
-    }
-    if (D > 16) {            // 4 units x 4 row segments in flight per lane
-        int blocks = grid_for(ceil_div64(K, 4) * 32, 256, 8);
-        launch_pdl(norm2_kernel<32, 4, 4>, blocks, 256, 0, st, W, K, D, c_norm2);
-    } else if (D > 8) {      // 2 x 8 units per warp
-        int blocks = grid_for(ceil_div64(K, 16) * 32, 256, 8);
-        launch_pdl(norm2_kernel<16, 8, 1>, blocks, 256, 0, st, W, K, D, c_norm2);
-    } else {                 // 4 x 8 units per warp
-        int blocks = grid_for(ceil_div64(K, 32) * 32, 256, 8);
-        launch_pdl(norm2_kernel<8, 8, 1>, blocks, 256, 0, st, W, K, D, c_norm2);
-    }
-    return check_launch("norm2_kernel");
-}
 
 int som_merge_candidates(const float* rd, const int64_t* idx, int R, int64_t n,
                          int64_t* out_idx, float* out_rd, void* stream) {
@@ -728,40 +798,6 @@ int som_histogram_i64(const int64_t* idx, int64_t n, int K, int64_t* counts, voi
     return check_launch("hist_global_kernel");
 }
 
-int som_quantize_nchw_f32(const int64_t* idx, const float* table, int K,
-                          int64_t n_img, int C, int H, int Wd, int pH, int pW,
-                          float* out, void* stream) {
-    SOM_REQUIRE(table && ((idx && out) || n_img == 0), SOM_E_BADARG, "quantize: null pointer");
-    SOM_REQUIRE(K > 0, SOM_E_BADARG, "quantize: K=%d", K);
-    Geom g;
-    int rc = make_geom(&g, out, n_img, C, H, Wd, pH, pW);
-    if (rc) return rc;
-    if (g.n_patches == 0) return SOM_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    const bool pw4 = (pW % 4 == 0), pw2 = (pW == 2);
-    if (Wd % 4 == 0 && ((uintptr_t)out & 15) == 0 && (pw4 || pw2) && g.img_stride >= 1024 &&
-        g.img_stride / 1024 < 65535 &&
-        ((uintptr_t)table & (pw4 ? 15 : 7)) == 0) {
-        const int64_t quads_img = g.img_stride / 4;
-        const int gy = (int)ceil_div64(quads_img, 256 * 4);
-        int gx = sm_count() * 8 / gy;
-        if (gx < 1) gx = 1;
-        if (gx > g.n_img) gx = (int)g.n_img;
-        dim3 blocks((unsigned)gx, (unsigned)gy);
-        if (pw2) quantize_out_kernel<true><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
-        else quantize_out_kernel<false><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
-        return check_launch("quantize_out_kernel");
-    }
-    int vec = g.vec;
-    if (((uintptr_t)table & 15) != 0 || g.D % 4 != 0) vec = (vec == 4) ? 1 : vec;
-    if (vec == 2 && (((uintptr_t)table & 7) != 0 || g.D % 2 != 0)) vec = 1;
-    int64_t items = g.n_patches * (g.D / vec);
-    int blocks = grid_for(items, 256, 16);
-    if (vec == 4) quantize_kernel<4><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
-    else if (vec == 2) quantize_kernel<2><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
-    else quantize_kernel<1><<<blocks, 256, 0, s>>>(idx, table, K, g, out);
-    return check_launch("quantize_kernel");
-}
 
 int som_assemble_tokens_i64(const int64_t* lr_idx, const int64_t* hr_idx, int64_t n, int lr_seq, int hr_seq,
                             int64_t lr_K, int64_t hr_K, int base_model, int64_t* hr_input, int64_t* hr_target,
@@ -829,20 +865,36 @@ int som_convert_bf16_f32(const void* in, int64_t n, float* out, void* stream) {
     return convert_16_f32<__nv_bfloat16>("convert_bf16_f32", in, n, out, stream);
 }
 
-int som_gather_rows_f32(const float* W, int D, const int64_t* keep, int64_t n_keep,
-                        float* out, void* stream) {
-    SOM_REQUIRE(W && keep && out, SOM_E_BADARG, "gather_rows: null pointer");
-    SOM_REQUIRE(D > 0 && n_keep >= 0, SOM_E_BADARG, "gather_rows: D=%d n_keep=%lld", D, (long long)n_keep);
-    if (n_keep == 0) return SOM_OK;
-    if (D % 4 == 0 && (((uintptr_t)W | (uintptr_t)out) & 15) == 0) {
-        int blocks = grid_for(n_keep * (D / 4), 256 * 4, 8);
-        gather_rows4_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const float4*>(W), D / 4, keep,
-                                                                      n_keep, reinterpret_cast<float4*>(out));
-        return check_launch("gather_rows4_kernel");
-    }
-    int blocks = grid_for(n_keep * D, 256, 16);
-    gather_rows_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(W, D, keep, n_keep, out);
-    return check_launch("gather_rows_kernel");
+
+int som_prepare_codebook_f32(const float* W, int K, int D, float* c_norm2, void* stream) {
+    return prepare_codebook(W, K, D, c_norm2, stream);
+}
+
+int som_prepare_codebook_w16(const void* W, int w_dtype, int K, int D, float* c_norm2, void* stream) {
+    SOM_REQUIRE(w_dtype == ELEM_F16 || w_dtype == ELEM_BF16, SOM_E_BADARG, "prepare_codebook: w_dtype=%d", w_dtype);
+    SOM_REQUIRE(((uintptr_t)W & 1) == 0, SOM_E_BADARG, "prepare_codebook: W is not 2-byte aligned");
+    if (w_dtype == ELEM_F16) return prepare_codebook((const __half*)W, K, D, c_norm2, stream);
+    return prepare_codebook((const __nv_bfloat16*)W, K, D, c_norm2, stream);
+}
+
+int som_quantize_nchw_f32(const int64_t* idx, const float* table, int K, int64_t n_img, int C, int H, int Wd, int pH,
+                          int pW, float* out, void* stream) {
+    return quantize_nchw(idx, table, K, n_img, C, H, Wd, pH, pW, out, stream);
+}
+
+int som_quantize_nchw_b16(const int64_t* idx, const void* table, int K, int64_t n_img, int C, int H, int Wd, int pH,
+                          int pW, void* out, void* stream) {
+    SOM_REQUIRE((((uintptr_t)table | (uintptr_t)out) & 1) == 0, SOM_E_BADARG, "quantize: 16-bit buffer misaligned");
+    return quantize_nchw(idx, (const uint16_t*)table, K, n_img, C, H, Wd, pH, pW, (uint16_t*)out, stream);
+}
+
+int som_gather_rows_f32(const float* W, int D, const int64_t* keep, int64_t n_keep, float* out, void* stream) {
+    return gather_rows(W, D, keep, n_keep, out, stream);
+}
+
+int som_gather_rows_b16(const void* W, int D, const int64_t* keep, int64_t n_keep, void* out, void* stream) {
+    SOM_REQUIRE((((uintptr_t)W | (uintptr_t)out) & 1) == 0, SOM_E_BADARG, "gather_rows: 16-bit buffer misaligned");
+    return gather_rows((const uint16_t*)W, D, keep, n_keep, (uint16_t*)out, stream);
 }
 
 }  // extern "C"

@@ -19,6 +19,7 @@ SIGNATURES = {
     "som_launch_count": (ctypes.c_uint64, []),
     "som_device_info": (c_int, [POINTER(c_int), POINTER(c_int), POINTER(c_int)]),
     "som_prepare_codebook_f32": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "som_prepare_codebook_w16": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "som_bmu_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int]),
     "som_bmu_pick_variant": (c_int, [c_int64, c_int, c_int]),
     "som_bmu_split_mode": (c_int, [c_int64, c_int, c_int]),
@@ -38,6 +39,9 @@ SIGNATURES = {
                                         c_void_p, c_size_t, c_int, c_void_p]),
     "som_convert_f16_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "som_convert_bf16_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
+    "som_bmu_w16_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int]),
+    "som_bmu_w16_nchw": (c_int, [c_void_p, c_int, c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int,
+                                 c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_void_p]),
     "som_bmu_flat_f32": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p,
                                  c_void_p, c_size_t, c_int, c_void_p]),
     "som_backward_nchw_f32": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int,
@@ -75,11 +79,14 @@ SIGNATURES = {
                                         c_int, c_int, c_void_p, c_int, c_void_p]),
     "som_quantize_nchw_f32": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_int, c_int,
                                       c_int, c_int, c_void_p, c_void_p]),
+    "som_quantize_nchw_b16": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int, c_int, c_int,
+                                      c_int, c_int, c_void_p, c_void_p]),
     "som_adam_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_double, c_double,
                              c_double, c_double, c_int64, c_void_p]),
     "som_adam_devstep_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_double, c_double,
                                      c_double, c_double, c_void_p, c_void_p]),
     "som_gather_rows_f32": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_void_p, c_void_p]),
+    "som_gather_rows_b16": (c_int, [c_void_p, c_int, c_void_p, c_int64, c_void_p, c_void_p]),
     "som_assemble_tokens_i64": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int64, c_int64, c_int,
                                         c_void_p, c_void_p, c_void_p]),
 }

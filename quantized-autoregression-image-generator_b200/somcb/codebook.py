@@ -13,6 +13,11 @@ train_quantized_transformer.py run unchanged.  The arithmetic runs in libsomcb:
   backward (autograd)    -> som_accumulate_nchw_f32 + som_filter_f32
   get_quantized_image    -> som_quantize_nchw_f32             (:138-154)
 
+After ``cb.half()`` or ``cb.to(torch.bfloat16)`` the inference methods keep working -- ``get_patches_bmu`` (results as
+for the fp32 module on ``weight.float()``) and ``get_quantized_image`` (detached output in the weight's dtype, as
+``nn.Embedding`` gives) -- and so do ``bmu_histogram``, ``prune_codebook`` and the tokenisers; ``forward`` and
+``get_quantized_patches`` (the training / autograd path) need fp32 weights.
+
 There is no CPU path: CPU inputs raise.
 """
 import torch
@@ -104,6 +109,7 @@ class Codebook(nn.Module):
         return idx
 
     def get_quantized_patches(self, x, use_gaussian=True):
+        self._require_fp32_weights("get_quantized_patches")
         x, geom = self._input(x)
         idx = ops.bmu(x, geom, self._weight(), self._norms(), variant=self.bmu_variant)
         n_patches = idx.numel()
@@ -112,25 +118,40 @@ class Codebook(nn.Module):
         return _GatherFn.apply(table, idx, flat, (x.shape[0], -1, self.embedding_dim))
 
     def get_quantized_image(self, indices, unpatchify_input=True):
+        """Codebook rows of ``indices`` (N, Seq), unpatchified to (N, C, H, W) or as (N, Seq, D).  With fp16 / bf16
+        weights the result is in that dtype and detached (no autograd through a 16-bit codebook)."""
         n, seq = indices.shape
         idx = self._indices(indices)
+        w = self.codebook.weight
+        gather = _GatherFn.apply
+        if w.dtype in ops.HALF_DTYPES:
+            w = w.detach()
+
+            def gather(table, i, geom, shape):
+                return ops.quantize(i, table, geom).view(shape)
         if unpatchify_input:
             c = self.embedding_dim // (self.patch_dim[0] * self.patch_dim[1])
             geom = ops.geometry((n, c, self.image_dim[0], self.image_dim[1]), self.patch_dim)
             if ops.n_patches_of(geom) != idx.numel():
                 raise Exception("indices do not match image_dim / patch_dim.")
-            return _GatherFn.apply(self.codebook.weight, idx, geom,
-                                   (n, c, self.image_dim[0], self.image_dim[1]))
+            return gather(w, idx, geom, (n, c, self.image_dim[0], self.image_dim[1]))
         flat = ops.flat_geometry(idx.numel(), self.embedding_dim)
-        return _GatherFn.apply(self.codebook.weight, idx, flat, (n, seq, self.embedding_dim))
+        return gather(w, idx, flat, (n, seq, self.embedding_dim))
 
     def forward(self, x, use_gaussian=True):
+        self._require_fp32_weights("forward")
         x, geom = self._input(x)
         idx = ops.bmu(x, geom, self._weight(), self._norms(), variant=self.bmu_variant)
         table = self._table(use_gaussian)
         return _GatherFn.apply(table, idx, geom, tuple(x.shape))
 
     # ---- helpers ---------------------------------------------------------------------------
+    def _require_fp32_weights(self, what):
+        dt = self.codebook.weight.dtype
+        if dt != torch.float32:
+            raise TypeError(f"Codebook.{what}: the training / autograd path needs float32 weights, the codebook holds "
+                            f"{dt} (16-bit codebooks support get_patches_bmu and get_quantized_image)")
+
     def _weight(self):
         return self.codebook.weight.detach()
 

@@ -74,16 +74,31 @@ def device_info():
     return sm.value, major.value, minor.value
 
 
+# 16-bit codebook dtypes and their C dtype codes (include/somcb.h: w_dtype; also the feature-map shards' codes)
+_W16_CODES = {torch.float16: 1, torch.bfloat16: 2}
+
+
+def _req_weight(weight):
+    """A codebook: fp32, or fp16 / bf16 (inference only: the search, decoding and row compaction)."""
+    if isinstance(weight, torch.Tensor) and weight.dtype in _W16_CODES:
+        return _req(weight, weight.dtype, "weight")
+    return _req(weight, torch.float32, "weight")
+
+
 def prepare_codebook(weight, out=None):
-    """c_norm2[j] = ||W_j||^2  (K0)."""
+    """c_norm2[j] = ||W_j||^2  (K0).  A 16-bit ``weight`` gives the norms of ``weight.float()`` bit for bit."""
     lib = _lib.load()
-    w = _req(weight, torch.float32, "weight")
+    w = _req_weight(weight)
     k, d = w.shape
     if out is None:
         out = torch.empty(k, dtype=torch.float32, device=w.device)
     with torch.cuda.device(w.device):
-        check("som_prepare_codebook_f32",
-              lib.som_prepare_codebook_f32(_ptr(w), k, d, _ptr(out), _stream(w)))
+        if w.dtype in _W16_CODES:
+            check("som_prepare_codebook_w16",
+                  lib.som_prepare_codebook_w16(_ptr(w), _W16_CODES[w.dtype], k, d, _ptr(out), _stream(w)))
+        else:
+            check("som_prepare_codebook_f32",
+                  lib.som_prepare_codebook_f32(_ptr(w), k, d, _ptr(out), _stream(w)))
     return out
 
 
@@ -138,10 +153,13 @@ def bmu(x, geom, weight, c_norm2=None, unit_offset=0, want_rd=False, variant=SOM
 
     A 16-bit ``x`` gives exactly the results of the same call on ``x.float()``: the FP16-split kernel reads it
     directly where ``bmu_f16_native`` says so, other shapes search an fp32 copy made by ``upcast_f16`` /
-    ``upcast_bf16``."""
+    ``upcast_bf16``.  Likewise a 16-bit (fp16 / bf16) ``weight`` gives exactly the results of ``weight.float()``
+    (som_bmu_w16_nchw); it takes no ``stage``, which only the training step reads."""
     lib = _lib.load()
-    w = _req(weight, torch.float32, "weight")
+    w = _req_weight(weight)
     k, d = w.shape
+    if w.dtype in _W16_CODES and stage is not None:
+        raise ValueError("bmu: stage is not available with a 16-bit codebook (training needs fp32 weights)")
     if isinstance(x, torch.Tensor) and x.dtype in _HALF_ENTRIES:
         x = _req(x, x.dtype, "x")
         if not bmu_f16_native(geom, k, variant):
@@ -166,6 +184,13 @@ def bmu(x, geom, weight, c_norm2=None, unit_offset=0, want_rd=False, variant=SOM
         if stage.numel() != npat * d:
             raise ValueError("stage must hold n_patches x D floats")
     with torch.cuda.device(x.device):
+        if w.dtype in _W16_CODES:
+            x_code = _W16_CODES.get(x.dtype, 0)
+            ws, ws_bytes = _workspace(lib.som_bmu_w16_workspace_bytes(npat, d, k, variant), x.device)
+            check("som_bmu_w16_nchw",
+                  lib.som_bmu_w16_nchw(_ptr(x), x_code, *geom, _ptr(w), _W16_CODES[w.dtype], _ptr(c_norm2), k,
+                                       int(unit_offset), _ptr(out), _ptr(rd), _ptr(ws), ws_bytes, variant, _stream(x)))
+            return (out, rd) if want_rd else out
         ws, ws_bytes = _workspace(lib.som_bmu_workspace_bytes(npat, d, k, variant), x.device)
         check(entry, getattr(lib, entry)(_ptr(x), *geom, _ptr(w), _ptr(c_norm2), k, int(unit_offset),
                                          _ptr(out), _ptr(rd), _ptr(stage), _ptr(ws), ws_bytes, variant, _stream(x)))
@@ -293,19 +318,20 @@ def adam_step_dp(weight, m, v, grad, dim, lr, steps_done, tail, loss_out=None, b
 
 
 def quantize(idx, table, geom, out=None):
-    """Gather + fused unpatchify: returns the fp32 buffer described by ``geom``."""
+    """Gather + fused unpatchify: returns the buffer described by ``geom`` in the table's dtype (fp32, or fp16 / bf16:
+    the 16-bit values are copied exactly)."""
     lib = _lib.load()
     idx = _req(idx, torch.int64, "idx")
-    table = _req(table, torch.float32, "table")
+    table = _req_weight(table)
     k, d = table.shape
     if d != dim_of(geom) or idx.numel() != n_patches_of(geom):
         raise ValueError("idx/table do not match the geometry")
     n, c, h, w, _, _ = geom
     if out is None:
-        out = torch.empty(n, c, h, w, dtype=torch.float32, device=table.device)
+        out = torch.empty(n, c, h, w, dtype=table.dtype, device=table.device)
+    entry = "som_quantize_nchw_b16" if table.dtype in _W16_CODES else "som_quantize_nchw_f32"
     with torch.cuda.device(table.device):
-        check("som_quantize_nchw_f32",
-              lib.som_quantize_nchw_f32(_ptr(idx), _ptr(table), k, *geom, _ptr(out), _stream(table)))
+        check(entry, getattr(lib, entry)(_ptr(idx), _ptr(table), k, *geom, _ptr(out), _stream(table)))
     return out
 
 
@@ -365,13 +391,14 @@ def step_small(x, geom, weight, m, v, neighbourhood_range, lr, steps_done, betas
 
 
 def gather_rows(weight, keep):
+    """out[r] = weight[keep[r]] in the weight's dtype (fp32, fp16 or bf16)."""
     lib = _lib.load()
-    w = _req(weight, torch.float32, "weight")
+    w = _req_weight(weight)
     keep = _req(keep, torch.int64, "keep")
-    out = torch.empty(keep.numel(), w.shape[1], dtype=torch.float32, device=w.device)
+    out = torch.empty(keep.numel(), w.shape[1], dtype=w.dtype, device=w.device)
+    entry = "som_gather_rows_b16" if w.dtype in _W16_CODES else "som_gather_rows_f32"
     with torch.cuda.device(w.device):
-        check("som_gather_rows_f32",
-              lib.som_gather_rows_f32(_ptr(w), w.shape[1], _ptr(keep), keep.numel(), _ptr(out), _stream(w)))
+        check(entry, getattr(lib, entry)(_ptr(w), w.shape[1], _ptr(keep), keep.numel(), _ptr(out), _stream(w)))
     return out
 
 

@@ -245,7 +245,8 @@ def bmu_histogram(codebook, batches, counts=None, ops=None):
 @torch.no_grad()
 def prune_codebook(codebook, counts, prune_threshold, image_channel=None, global_steps=0, ops=None):
     """Keep units with count >= threshold in ascending index order and build the smaller
-    codebook + the reference's checkpoint dict (prune_codebook.py:144-178)."""
+    codebook + the reference's checkpoint dict (prune_codebook.py:144-178).  The pruned codebook keeps the weights'
+    dtype (fp32, or fp16 / bf16 for a 16-bit codebook)."""
     from .codebook import Codebook
     ops = ops or _default_ops
     keep = torch.nonzero(counts >= prune_threshold).flatten().to(torch.int64)
@@ -254,7 +255,7 @@ def prune_codebook(codebook, counts, prune_threshold, image_channel=None, global
         image_channel = codebook.embedding_dim // (codebook.patch_dim[0] * codebook.patch_dim[1])
     new_cb = Codebook(patch_dim=codebook.patch_dim, image_dim=codebook.image_dim,
                       image_channel=image_channel, num_embeddings=int(keep.numel()),
-                      init_neighbour_range=codebook.neighbourhood_range).to(rows.device)
+                      init_neighbour_range=codebook.neighbourhood_range).to(device=rows.device, dtype=rows.dtype)
     new_cb.codebook.weight.data.copy_(rows)
     ck = {"patch_dim": codebook.patch_dim, "image_dim": codebook.image_dim, "image_C": image_channel,
           "num_embeddings": int(keep.numel()), "neighbourhood_range": codebook.neighbourhood_range,
