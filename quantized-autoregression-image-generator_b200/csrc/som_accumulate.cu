@@ -717,6 +717,24 @@ static int launch_levels(const float* x, const Geom& g, const AccumPlan& pl, con
     return SOM_OK;
 }
 
+// Which path and vector width accumulate_impl runs, from the shape, the batch's own vector width and the alignment of
+// Wt and Rbar.  Scan path (static rule on the shape): tiny batches, where the eight launches of the sorted path are the
+// cost; a CTA's run time grows with its unit's hit count, so skewed large batches stay on the sorted path (measured at
+// C3, 4096 patches: 71 us sorted vs 135 us scanned).  Sorted paths: the library's counting sort where the plan has sort
+// blocks, cub's radix sort otherwise (n = 0 sorts nothing and takes that branch for the offsets alone).
+struct AccumRoute { int path, vec, n_slices; };
+static AccumRoute accumulate_route(const Geom& g, const AccumPlan& pl, const float* Wt, const float* Rbar) {
+    const int64_t n = g.n_patches;
+    int vec = g.vec;
+    if (Wt != nullptr && ((uintptr_t)Wt & 15) != 0) vec = 1;
+    if (((uintptr_t)Rbar & 15) != 0) vec = 1;
+    if (n > 0 && n <= 2048 && n * (int64_t)pl.K <= (1ll << 26))
+        return {ACC_SCAN, vec, (int)ceil_div64(g.D, (int64_t)SCAN_THREADS * vec)};
+    // a warp covers 32 * vec features of one patch row: keep all lanes busy for short rows (C4, D = 64: vec 2)
+    while (vec > 1 && 32 * vec > g.D) vec >>= 1;
+    return {(n > 0 && pl.cs_blocks > 0) ? ACC_COUNTING : ACC_RADIX, vec, (int)ceil_div64(g.D, 32 * vec)};
+}
+
 }  // namespace som
 
 using namespace som;
@@ -754,15 +772,11 @@ static int accumulate_impl(const float* x, int64_t n_img, int C, int H, int Wd, 
     double* sse_part = (double*)(base + pl.off_sse);
     void* cub_tmp = base + pl.off_cub;
     const int64_t n = g.n_patches;
+    const AccumRoute route = accumulate_route(g, pl, Wt, Rbar);
+    const int vec = route.vec;
 
-    if (n > 0 && n <= 2048 && n * (int64_t)K <= (1ll << 26)) {
-        // scan path (static rule on the shape): tiny batches, where the eight launches of the sorted path are the
-        // cost; a CTA's run time grows with its unit's hit count, so skewed large batches stay on the sorted path
-        // (measured at C3, 4096 patches: 71 us sorted vs 135 us scanned)
-        int vec = g.vec;
-        if (Wt != nullptr && ((uintptr_t)Wt & 15) != 0) vec = 1;
-        if (((uintptr_t)Rbar & 15) != 0) vec = 1;
-        const int n_slices = (int)ceil_div64(g.D, (int64_t)SCAN_THREADS * vec);
+    if (route.path == ACC_SCAN) {
+        const int n_slices = route.n_slices;
         dim3 grid((unsigned)K, (unsigned)n_slices);
         double* sp = ((sse || tail) && Wt) ? sse_part : nullptr;
         if (vec == 4) launch_pdl(acc_scan_kernel<4>, grid, SCAN_THREADS, 0, st, x, g, bmu, K, Wt, Rbar, counts, sp, n_slices);
@@ -779,7 +793,7 @@ static int accumulate_impl(const float* x, int64_t n_img, int C, int H, int Wd, 
 
     const int* skey = keys_a;
     const int* sid = vals_a;
-    if (n > 0 && pl.cs_blocks > 0) {
+    if (route.path == ACC_COUNTING) {
         int* hist = (int*)(base + pl.off_hist);
         int* total = hist + (size_t)pl.cs_blocks * K;
         const size_t bins = (size_t)K * sizeof(int);
@@ -816,14 +830,33 @@ static int accumulate_impl(const float* x, int64_t n_img, int C, int H, int Wd, 
     if (rc) return rc;
     }
 
-    int vec = g.vec;
-    if (Wt != nullptr && ((uintptr_t)Wt & 15) != 0) vec = 1;
-    if (((uintptr_t)Rbar & 15) != 0) vec = 1;
-    // a warp covers 32 * vec features of one patch row: keep all lanes busy for short rows (C4, D = 64: vec 2)
-    while (vec > 1 && 32 * vec > g.D) vec >>= 1;
     if (vec == 4) return launch_levels<4>(x, g, pl, skey, sid, offsets, Wt, Rbar, counts, sse, tail, partial, sse_part, st);
     if (vec == 2) return launch_levels<2>(x, g, pl, skey, sid, offsets, Wt, Rbar, counts, sse, tail, partial, sse_part, st);
     return launch_levels<1>(x, g, pl, skey, sid, offsets, Wt, Rbar, counts, sse, tail, partial, sse_part, st);
+}
+
+// debug: the plan of an accumulation, as APF_COUNT int64 fields (som_common.cuh: AccumPlanField, -1 where a field does
+// not apply); the first n_out are written.  x, Wt and Rbar are the pointers a call would pass (Wt may be null); only
+// their alignment is read.  The answers come from the rules accumulate_impl uses.  Not in somcb.h: a test hook.
+extern "C" SOM_API int som_debug_accumulate_plan(const float* x, int64_t n_img, int C, int H, int Wd, int pH, int pW,
+                                                 const float* Wt, int K, const float* Rbar, int64_t* out, int n_out) {
+    SOM_REQUIRE(K > 0 && out != nullptr && n_out >= 0, SOM_E_BADARG, "accumulate plan: K=%d, output", K);
+    Geom g;
+    int rc = make_geom(&g, x, n_img, C, H, Wd, pH, pW);
+    if (rc) return rc;
+    AccumPlan pl;
+    rc = make_plan(&pl, g.n_patches, g.D, K, false);
+    if (rc) return rc;
+    const AccumRoute r = accumulate_route(g, pl, Wt, Rbar);
+    int64_t f[APF_COUNT];
+    for (int i = 0; i < APF_COUNT; ++i) f[i] = -1;
+    f[APF_PATH] = r.path;
+    f[APF_VEC] = r.vec;
+    f[APF_N_SLICES] = r.n_slices;
+    if (r.path != ACC_SCAN) { f[APF_S] = pl.S; f[APF_N_CHUNKS] = pl.n_chunks; }
+    if (r.path == ACC_COUNTING) { f[APF_CS_PER] = pl.cs_per; f[APF_CS_BLOCKS] = pl.cs_blocks; }
+    for (int i = 0; i < n_out && i < APF_COUNT; ++i) out[i] = f[i];
+    return SOM_OK;
 }
 
 extern "C" int som_accumulate_nchw_f32(const float* x, int64_t n_img, int C, int H, int Wd, int pH,

@@ -69,6 +69,32 @@ enum PlanField : int {
     PF_COUNT
 };
 
+// The update path's plans, the same way: som_debug_filter_plan (som_filter.cu), som_debug_accumulate_plan
+// (som_accumulate.cu) and som_debug_step_small_plan (som_step_small.cu).
+enum FilterKernel : int { FK_SCALAR = 0, FK_TILE64 = 1, FK_TILE128 = 2, FK_TC64 = 3, FK_TC128 = 4 };
+enum FilterPlanField : int {
+    FPF_KERNEL,         // FilterKernel
+    FPF_H,              // band half-width
+    FPF_SMEM,           // dynamic shared memory of the main kernel (bytes)
+    FPF_NKB,            // tensor cores: 32-row k-blocks per unit tile
+    FPF_Q,              // tensor cores: k-blocks per accumulation chain
+    FPF_NA,             // tensor cores: accumulation chains
+    FPF_KS,             // tensor cores: CTAs per tile (k-split, then filter_reduce_kernel) or 1
+    FPF_KP,             // tensor cores: padded inner length of the transposed operand
+    FPF_COUNT
+};
+enum AccumPath : int { ACC_SCAN = 0, ACC_COUNTING = 1, ACC_RADIX = 2 };
+enum AccumPlanField : int {
+    APF_PATH,           // AccumPath
+    APF_VEC,            // floats per lane access
+    APF_S,              // sorted paths: positions per level-1 chunk
+    APF_N_CHUNKS,       // sorted paths: level-1 chunks
+    APF_N_SLICES,       // feature slices (32 * VEC wide sorted, 256 * VEC on the scan path)
+    APF_CS_PER,         // counting sort: patches per sort block
+    APF_CS_BLOCKS,      // counting sort: sort blocks
+    APF_COUNT
+};
+
 // elem_bytes: 4 for an fp32 batch, 2 for a 16-bit one (fp16 or bf16; vec then counts 16-bit elements)
 int make_geom(Geom* g, const void* x, int64_t n_img, int C, int H, int W, int pH, int pW, int elem_bytes = 4);
 

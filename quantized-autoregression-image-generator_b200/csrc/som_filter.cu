@@ -206,8 +206,26 @@ filter_tile_kernel(const float* __restrict__ in, float* __restrict__ out, int K,
 // som_filter_tc.cu
 bool filter_tc_applicable(int K, int D, int h);
 size_t filter_tc_workspace_bytes(int K, int D, int h);
+void filter_tc_plan_fields(int K, int D, int h, int64_t* f);
 int launch_filter_tc(const float* in, float* out, int K, int D, float two_var, int h, float scale, void* ws,
                      size_t ws_bytes, cudaStream_t st);
+
+// The kernel som_filter_f32 runs (FilterPlanField::FPF_KERNEL) and its dynamic shared memory.  The tile kernels take
+// D % 4 == 0, D >= 48 and 16-byte aligned `in` and `out` while their table and chunk ring fit in 200 KB; the scalar kernel
+// takes every other shape while its table fits (h <= 25 583), also the tile kernels' shapes with a wider band than
+// theirs.  False where no kernel fits.
+static bool filter_ffma_route(int D, int h, bool aligned16, int* kernel, size_t* smem) {
+    if ((D & 3) == 0 && D >= 48 && aligned16) {
+        const int td = D >= 128 ? 128 : 64;
+        const size_t tab_n = (size_t)(2 * (h + FT_PAD) + 1);
+        *smem = ((tab_n + 3) & ~(size_t)3) * sizeof(float) + 2 * (size_t)FT_JC * td * sizeof(float);
+        *kernel = td == 128 ? FK_TILE128 : FK_TILE64;
+        if (*smem <= 200 * 1024) return true;
+    }
+    *smem = (size_t)(2 * (h + FILT_PAD) + 1) * sizeof(float);
+    *kernel = FK_SCALAR;
+    return *smem <= 200 * 1024;
+}
 
 }  // namespace som
 
@@ -248,29 +266,55 @@ extern "C" int som_filter_f32(const float* in, float* out, int K, int D,
                 neighbourhood_range);
     const float two_var = filter_two_var(neighbourhood_range);
     const int h = filter_band_half_width(two_var, K);
-    size_t smem = (size_t)(2 * (h + FILT_PAD) + 1) * sizeof(float);
-    SOM_REQUIRE(smem <= 200 * 1024, SOM_E_SHAPE, "filter: band half-width %d too large", h);
+    int kern;
+    size_t smem;
+    SOM_REQUIRE(filter_ffma_route(D, h, (((uintptr_t)in | (uintptr_t)out) & 15) == 0, &kern, &smem), SOM_E_SHAPE,
+                "filter: band half-width %d too large", h);
     typedef void (*FilterFn)(const float*, float*, int, int, float, int, float);
+    if (kern != FK_SCALAR) {
+        const int td = kern == FK_TILE128 ? 128 : 64;
+        static const FilterFn tile_kernels[2] = {filter_tile_kernel<128, 2>, filter_tile_kernel<64, 4>};
+        static PerDeviceFlag attr_done;
+        const int rc = smem_opt_in(attr_done, tile_kernels, 2, 200 * 1024, "filter");
+        if (rc) return rc;
+        dim3 gt((unsigned)ceil_div64(K, 32), (unsigned)ceil_div64(D, td));      // 32 units per CTA in both shapes
+        launch_pdl(tile_kernels[td == 64], gt, FT_THREADS, smem, (cudaStream_t)stream, in, out, K, D, two_var, h, scale);
+        return check_launch("filter_tile_kernel");
+    }
     if (smem > 48 * 1024) {
         static PerDeviceFlag attr_done;
         const FilterFn kernel = filter_kernel;
         const int rc = smem_opt_in(attr_done, &kernel, 1, 200 * 1024, "filter");
         if (rc) return rc;
     }
-    if ((D & 3) == 0 && D >= 48 && (((uintptr_t)in | (uintptr_t)out) & 15) == 0) {
-        const int td = D >= 128 ? 128 : 64;
-        const size_t tab_n = (size_t)(2 * (h + FT_PAD) + 1);
-        const size_t smem_t = ((tab_n + 3) & ~(size_t)3) * sizeof(float) + 2 * (size_t)FT_JC * td * sizeof(float);
-        SOM_REQUIRE(smem_t <= 200 * 1024, SOM_E_SHAPE, "filter: band half-width %d too large", h);
-        static const FilterFn tile_kernels[2] = {filter_tile_kernel<128, 2>, filter_tile_kernel<64, 4>};
-        static PerDeviceFlag attr_done;
-        const int rc = smem_opt_in(attr_done, tile_kernels, 2, 200 * 1024, "filter");
-        if (rc) return rc;
-        dim3 gt((unsigned)ceil_div64(K, 32), (unsigned)ceil_div64(D, td));      // 32 units per CTA in both shapes
-        launch_pdl(tile_kernels[td == 64], gt, FT_THREADS, smem_t, (cudaStream_t)stream, in, out, K, D, two_var, h, scale);
-        return check_launch("filter_tile_kernel");
-    }
     dim3 grid((unsigned)ceil_div64(K, FILT_WARPS * FILT_TA), (unsigned)ceil_div64(D, 32));
     launch_pdl(filter_kernel, grid, FILT_WARPS * 32, smem, (cudaStream_t)stream, in, out, K, D, two_var, h, scale);
     return check_launch("filter_kernel");
+}
+
+// debug: the plan of a filter call, as FPF_COUNT int64 fields (som_common.cuh: FilterPlanField, -1 where a field does
+// not apply); the first n_out are written.  with_ws: som_filter_ws_f32 with a workspace (else som_filter_f32, or
+// som_filter_ws_f32 without one); aligned16: `in` and `out` are both 16-byte aligned.  The answers come from the rules the
+// launchers use.  Not in somcb.h: a test hook, not part of the ABI.
+extern "C" SOM_API int som_debug_filter_plan(int K, int D, double neighbourhood_range, int with_ws, int aligned16,
+                                             int64_t* out, int n_out) {
+    SOM_REQUIRE(K > 0 && D > 0 && neighbourhood_range > 0.0, SOM_E_BADARG, "filter plan: K=%d D=%d range=%g", K, D,
+                neighbourhood_range);
+    SOM_REQUIRE(out != nullptr && n_out >= 0, SOM_E_BADARG, "filter plan: output");
+    int64_t f[FPF_COUNT];
+    for (int i = 0; i < FPF_COUNT; ++i) f[i] = -1;
+    const int h = filter_band_half_width(filter_two_var(neighbourhood_range), K);
+    if (with_ws && filter_tc_applicable(K, D, h)) {
+        filter_tc_plan_fields(K, D, h, f);
+    } else {
+        int kern;
+        size_t smem;
+        SOM_REQUIRE(filter_ffma_route(D, h, aligned16 != 0, &kern, &smem), SOM_E_SHAPE,
+                    "filter: band half-width %d too large", h);
+        f[FPF_KERNEL] = kern;
+        f[FPF_SMEM] = (int64_t)smem;
+    }
+    f[FPF_H] = h;
+    for (int i = 0; i < n_out && i < FPF_COUNT; ++i) out[i] = f[i];
+    return SOM_OK;
 }

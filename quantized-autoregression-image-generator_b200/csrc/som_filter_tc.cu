@@ -407,6 +407,19 @@ size_t filter_tc_workspace_bytes(int K, int D, int h) {
     return pl.total;
 }
 
+// the plan of launch_filter_tc for som_debug_filter_plan (f: FPF_COUNT fields)
+void filter_tc_plan_fields(int K, int D, int h, int64_t* f) {
+    ftc::Plan pl;
+    ftc::make_plan(&pl, K, D, h);
+    f[FPF_KERNEL] = pl.tnf == 128 ? FK_TC128 : FK_TC64;
+    f[FPF_SMEM] = (int64_t)ftc::smem_bytes(pl.tnf, h);
+    f[FPF_NKB] = pl.nkb;
+    f[FPF_Q] = pl.q;
+    f[FPF_NA] = pl.na;
+    f[FPF_KS] = pl.ks;
+    f[FPF_KP] = pl.Kp;
+}
+
 // pin != nullptr: `in` is a multicast address, read with the in-switch reduction (see split_in_t_kernel)
 int launch_filter_tc_in(const float* in, float* out, int K, int D, float two_var, int h, float scale, void* ws,
                         size_t ws_bytes, cudaStream_t st, const ftc::PeerIn* pin) {

@@ -421,6 +421,9 @@ static bool make_plan(Plan* pl, int64_t n, int D, int K, double range) {
     return true;
 }
 
+// the RBCAP slot of step_small_kernel<D, RBCAP> for RB output rows per thread: RBCAP = 2, 8 or 32
+static int rb_slot(int RB) { return RB <= 2 ? 0 : (RB <= 8 ? 1 : 2); }
+
 }  // namespace sstep
 }  // namespace som
 
@@ -469,7 +472,7 @@ extern "C" int som_step_small_f32(const float* x, int64_t n_img, int C, int H, i
         {step_small_kernel<128, 2>, step_small_kernel<128, 8>, step_small_kernel<128, 32>},
         {step_small_kernel<256, 2>, step_small_kernel<256, 8>, step_small_kernel<256, 32>}};
     const int dslot = g.D == 16 ? 0 : g.D == 32 ? 1 : g.D == 64 ? 2 : g.D == 128 ? 3 : 4;
-    const int rslot = pl.RB <= 2 ? 0 : (pl.RB <= 8 ? 1 : 2);
+    const int rslot = rb_slot(pl.RB);
     KernelFn fn = fns[dslot][rslot];
     const size_t smem = smem_bytes();
     static PerDeviceFlag attr_done[15];
@@ -480,6 +483,22 @@ extern "C" int som_step_small_f32(const float* x, int64_t n_img, int C, int H, i
                                                  (cudaStream_t)stream);
     if (le != cudaSuccess) { set_error("step_small_kernel: launch: %s", cudaGetErrorString(le)); return (int)le; }
     return check_launch("step_small_kernel");
+}
+
+// debug: the plan of som_step_small_f32 for n patches of dimension D, K units and a range, as 8 int64 fields: grid, R,
+// RB, the RBCAP slot (0, 1, 2: RBCAP = 2, 8, 32), UC, PG, PPG, h; all -1 where the one-kernel step does not cover the
+// shape.  The first n_out are written.  Not in somcb.h: a test hook, not part of the ABI.
+extern "C" SOM_API int som_debug_step_small_plan(int64_t n_patches, int D, int K, double neighbourhood_range,
+                                                 int64_t* out, int n_out) {
+    SOM_REQUIRE(out != nullptr && n_out >= 0, SOM_E_BADARG, "step_small plan: output");
+    int64_t f[8] = {-1, -1, -1, -1, -1, -1, -1, -1};
+    Plan pl;
+    if (make_plan(&pl, n_patches, D, K, neighbourhood_range)) {
+        const int64_t v[8] = {pl.grid, pl.R, pl.RB, rb_slot(pl.RB), pl.UC, pl.PG, pl.PPG, pl.h};
+        for (int i = 0; i < 8; ++i) f[i] = v[i];
+    }
+    for (int i = 0; i < n_out && i < 8; ++i) out[i] = f[i];
+    return SOM_OK;
 }
 
 // debug: CTA 0's globaltimer (ns) at the eight phase boundaries of the last launch

@@ -144,9 +144,16 @@ def check_bound(a, b):
     return worst
 
 
+def tf32_rna(v):
+    """cvt.rna.tf32.f32: round to 10 stored mantissa bits, ties away from zero (fp32 in, fp32 out)"""
+    u = v.contiguous().view(torch.int32)
+    return ((u + 0x1000) & ~0x1FFF).view(torch.float32)
+
+
 def to_float(ints, e, dtype=torch.float32):
-    """ints * 2^e, exactly (every |value| here is below 2^24)."""
-    return torch.ldexp(ints.to(torch.float64), torch.tensor(float(e), dtype=torch.float64)).to(dtype)
+    """ints * 2^e, exactly (every |value| here is below 2^24).  A multiply by the Python float 2^e, not torch.ldexp:
+    on CUDA tensors ldexp computes 2^e with pow and is 1 ulp off for negative e."""
+    return (ints.to(torch.float64) * 2.0 ** e).to(dtype)
 
 
 def unpatchify(rows, c, ph, pw, gh, gw):

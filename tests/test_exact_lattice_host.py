@@ -25,10 +25,7 @@ def _rd64(x, w):
     return torch.cat([rd for _, rd in L.fp64_rd(x, w)])
 
 
-def _tf32_rna(v):
-    """cvt.rna.tf32.f32: round to 10 stored mantissa bits, ties away from zero (fp32 in, fp32 out)"""
-    u = v.contiguous().view(torch.int32)
-    return ((u + 0x1000) & ~0x1FFF).view(torch.float32)
+_tf32_rna = L.tf32_rna
 
 
 def _3xtf32_terms(x, w):
