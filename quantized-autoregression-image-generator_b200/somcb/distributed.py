@@ -208,6 +208,32 @@ class DataParallelSom(SomTrainer):
         self.last_bmu = bmu
         return loss
 
+    def _full_moments(self):
+        """On the peer tail a rank's Adam step updates only its own rows [lo, hi) of m and v; the other rows are stale
+        there.  One all-gather of every rank's rows (padded to the largest slice) makes the saved moments complete and
+        identical on every rank.  ``state_dict`` is therefore collective: call it on every rank."""
+        if self.peer is None:
+            return self.m, self.v
+        k, d = self.cb.num_embeddings, self.cb.embedding_dim
+        spans = [shard_bounds(k, self.peer.world, r) for r in range(self.peer.world)]
+        rows = max(hi - lo for lo, hi in spans)
+        lo, hi = spans[self.peer.rank]
+        send = torch.zeros(2, rows, d, dtype=torch.float32, device=self.m.device)
+        send[0, :hi - lo] = self.m[lo:hi]
+        send[1, :hi - lo] = self.v[lo:hi]
+        recv = torch.empty(len(spans), 2, rows, d, dtype=torch.float32, device=self.m.device)
+        dist.all_gather_into_tensor(recv, send, group=self.group)
+        return tuple(torch.cat([recv[r, i, :b - a] for r, (a, b) in enumerate(spans)]) for i in (0, 1))
+
+    def load_state_dict(self, state):
+        """``SomTrainer.load_state_dict`` on every rank: each copies the full moments (on the peer tail it then uses only
+        its own rows), then a barrier, so that no rank starts a step, whose tail writes into every rank's codebook, before
+        every rank has loaded.  A state saved at any world size, on either tail, loads at any other.  Collective: call it
+        (or ``resume``) on every rank."""
+        super().load_state_dict(state)
+        if self.world_size > 1:
+            dist.barrier(group=self.group)
+
     def broadcast_weights(self, src=0):
         """Make every replica start from rank ``src``'s codebook."""
         dist.broadcast(self.cb.codebook.weight.data, src=src, group=self.group)

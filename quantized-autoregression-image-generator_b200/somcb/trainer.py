@@ -36,8 +36,8 @@ class SomTrainer:
         flag the step is captured once per (batch shape, neighbourhood range, lr) into a CUDA graph and
         replayed: the batch is copied into a static buffer first.  ``use_cuda_graph="alias"`` captures on
         the caller's own input buffer instead (one graph per distinct buffer address, at most MAX_GRAPHS
-        kept): for loops that refill a few device staging buffers.  The first step always runs eagerly
-        (one-time kernel attribute set-up and NCCL communicator creation must not happen during capture).
+        kept): for loops that refill a few device staging buffers.  The first step of a trainer always runs eagerly, also
+        after a resume (one-time kernel attribute set-up and NCCL communicator creation must not happen during capture).
 
         ``check_nan``: the reference's ``NaN encountered during training`` guard (train_codebook.py:237-238);
         it reads the loss back, i.e. one host synchronisation per step, so it is off by default.
@@ -63,7 +63,7 @@ class SomTrainer:
         self._side = None                                   # side stream of the W~ filter
         self._wt_side = None                                # its output (kept: written on one stream, read on another)
         w = codebook.codebook.weight
-        # the reference does not checkpoint Adam state: a resume restarts the moments at zero
+        # Adam's moments; ``state_dict`` / ``load_state_dict`` save and restore them with the step count and schedule
         self.m = torch.zeros_like(w, requires_grad=False)
         self.v = torch.zeros_like(w, requires_grad=False)
         self.t = 0
@@ -74,6 +74,7 @@ class SomTrainer:
         self.use_cuda_graph = bool(use_cuda_graph)
         self._graph_alias = use_cuda_graph == "alias"
         self._graphs = {}             # key -> (CUDAGraph, x_static, loss_static)
+        self._warm = False            # an eager step has run in this trainer (a resumed t >= 1 does not say so)
 
     @torch.no_grad()
     def step(self, feature_map, bmu=None):
@@ -81,7 +82,7 @@ class SomTrainer:
         tensor (global mean squared error, as F.mse_loss over the global batch).  Under ``use_cuda_graph`` the
         tensor is the captured graph's own output buffer: read it (``float(loss)``, ``.clone()``) before the same
         graph is replayed again."""
-        if self.use_cuda_graph and bmu is None and self.t >= 1 and feature_map.is_cuda:
+        if self.use_cuda_graph and bmu is None and self._warm and feature_map.is_cuda:
             loss = self._graph_step(feature_map)
         else:
             loss = self._eager_step(feature_map, bmu)
@@ -130,6 +131,7 @@ class SomTrainer:
 
     def _eager_step(self, feature_map, bmu=None):
         loss = self._device_step(feature_map, bmu)
+        self._warm = True
         self.t += 1
         self._bookkeeping()
         return loss.reshape(())
@@ -221,12 +223,110 @@ class SomTrainer:
             return bmu, stage, ops.flat_geometry(npat, d)
         return ops.bmu(x, geom, w, cn, variant=cb.bmu_variant), x, geom
 
-    def checkpoint_dict(self, image_channel):
-        """The reference's checkpoint layout (train_codebook.py:271-278)."""
+    STATE_KEYS = ("num_embeddings", "embedding_dim", "m", "v", "t", "t_dev", "lr", "global_steps", "lr_step",
+                  "neighbourhood_step", "betas", "eps", "neighbourhood_range")
+
+    def _sync(self):
+        w = self.cb.codebook.weight
+        if w.is_cuda:
+            torch.cuda.synchronize(w.device)
+
+    def _full_moments(self):
+        """(m, v) with every row current (``DataParallelSom``'s sharded tail gathers them)."""
+        return self.m, self.v
+
+    @torch.no_grad()
+    def state_dict(self):
+        """Everything a run needs to continue exactly where it stopped, except the weights (those are the codebook's own
+        ``state_dict``; ``checkpoint_dict(..., with_state=True)`` holds both): Adam's moments ``m`` and ``v`` (CPU fp32,
+        (K, D)), the host step count ``t`` and the device one ``t_dev``, the schedule (``lr`` as halved so far,
+        ``global_steps``, ``lr_step``, ``neighbourhood_step`` and the codebook's ``neighbourhood_range``), ``betas``,
+        ``eps``, and ``num_embeddings`` / ``embedding_dim`` to check against on load.
+
+        Synchronises the device before it reads anything, so it may be called while steps are still in flight, from any
+        stream: e.g. right after ``HostTrainer.step`` calls whose losses are still pending."""
         cb = self.cb
-        return {"patch_dim": cb.patch_dim, "image_dim": cb.image_dim, "image_C": image_channel,
-                "num_embeddings": cb.num_embeddings, "neighbourhood_range": cb.neighbourhood_range,
-                "global_steps": self.global_steps, "checkpoint": cb.state_dict()}
+        self._sync()
+        m, v = self._full_moments()
+        return {"num_embeddings": cb.num_embeddings, "embedding_dim": cb.embedding_dim,
+                "m": m.detach().to("cpu", torch.float32, copy=True), "v": v.detach().to("cpu", torch.float32, copy=True),
+                "t": self.t, "t_dev": int(self.t_dev[0]), "lr": self.lr, "global_steps": self.global_steps,
+                "lr_step": self.lr_step, "neighbourhood_step": self.neighbourhood_step, "betas": tuple(self.betas),
+                "eps": self.eps, "neighbourhood_range": cb.neighbourhood_range}
+
+    def _check_state(self, state):
+        missing = [key for key in self.STATE_KEYS if key not in state]
+        if missing:
+            raise ValueError(f"SomTrainer state: missing {', '.join(missing)}")
+        k, d = self.cb.num_embeddings, self.cb.embedding_dim
+        if (state["num_embeddings"], state["embedding_dim"]) != (k, d):
+            raise ValueError(f"SomTrainer state of a codebook with K = {state['num_embeddings']}, "
+                             f"D = {state['embedding_dim']}; this trainer's codebook has K = {k}, D = {d}")
+        for name in ("m", "v"):
+            if tuple(state[name].shape) != (k, d):
+                raise ValueError(f"SomTrainer state: {name} has shape {tuple(state[name].shape)}, expected ({k}, {d})")
+
+    @torch.no_grad()
+    def load_state_dict(self, state):
+        """Restore a ``state_dict``.  Copies in place into the existing ``m``, ``v`` and ``t_dev``, never rebinding them,
+        so the CUDA graphs this trainer has captured stay valid and their next replay runs on the loaded state.  A graph
+        is keyed by batch shape, neighbourhood range and lr: a loaded range or lr that no graph was captured for selects
+        another graph or captures a new one at the next step.  The weights are not part of the state: ``resume`` copies
+        them into the codebook, in place as well.  Raises ValueError, having changed nothing, when a key is missing or
+        K, D or the moments' shapes do not match this trainer's codebook."""
+        self._check_state(state)
+        self._sync()                          # no step still in flight reads or writes what is overwritten
+        self.m.copy_(state["m"])
+        self.v.copy_(state["v"])
+        self.t_dev.copy_(torch.tensor([int(state["t_dev"]), 0], dtype=torch.int64))
+        betas, eps = tuple(state["betas"]), state["eps"]
+        if (betas, eps) != (tuple(self.betas), self.eps):
+            self._graphs.clear()              # captured graphs hold betas and eps as kernel arguments
+        self.betas, self.eps = betas, eps
+        self.t = int(state["t"])
+        self.lr = state["lr"]
+        self.global_steps = int(state["global_steps"])
+        self.lr_step = int(state["lr_step"])
+        self.neighbourhood_step = int(state["neighbourhood_step"])
+        self.cb.neighbourhood_range = state["neighbourhood_range"]
+        self._sync()
+
+    @torch.no_grad()
+    def resume(self, checkpoint):
+        """Continue a run from a dict of the ``checkpoint_dict`` layout (e.g. ``torch.load`` of a saved one): copies the
+        weights into the codebook in place, then loads the ``"trainer"`` state (``load_state_dict``), after which the
+        run continues exactly as if it had not been interrupted.  A checkpoint without ``"trainer"`` (the reference's
+        own layout) resumes as the reference does: Adam's moments and step count at zero, ``global_steps`` and the
+        neighbourhood range from the checkpoint, lr and schedule as this trainer holds them.  Raises ValueError, having
+        changed nothing, when the weights or the state do not match this trainer's codebook."""
+        w = self.cb.codebook.weight.data
+        w_new = checkpoint["checkpoint"]["codebook.weight"]
+        if tuple(w_new.shape) != tuple(w.shape):
+            raise ValueError(f"checkpoint weights have shape {tuple(w_new.shape)}, this trainer's codebook "
+                             f"{tuple(w.shape)}")
+        state = checkpoint.get("trainer")
+        if state is None:
+            k, d = w.shape
+            state = {"num_embeddings": k, "embedding_dim": d, "m": torch.zeros(k, d), "v": torch.zeros(k, d), "t": 0,
+                     "t_dev": 0, "lr": self.lr, "global_steps": checkpoint["global_steps"], "lr_step": self.lr_step,
+                     "neighbourhood_step": self.neighbourhood_step, "betas": self.betas, "eps": self.eps,
+                     "neighbourhood_range": checkpoint["neighbourhood_range"]}
+        self._check_state(state)
+        self._sync()
+        w.copy_(w_new)
+        self.load_state_dict(state)
+
+    def checkpoint_dict(self, image_channel, with_state=False):
+        """The reference's checkpoint layout (train_codebook.py:271-278).  ``with_state=True`` adds one key,
+        ``"trainer"`` = ``state_dict()``, for ``resume``; the other keys stay exactly as without it, and the reference's
+        loader, which reads only those, still loads the file."""
+        cb = self.cb
+        ck = {"patch_dim": cb.patch_dim, "image_dim": cb.image_dim, "image_C": image_channel,
+              "num_embeddings": cb.num_embeddings, "neighbourhood_range": cb.neighbourhood_range,
+              "global_steps": self.global_steps, "checkpoint": cb.state_dict()}
+        if with_state:
+            ck["trainer"] = self.state_dict()
+        return ck
 
 
 @torch.no_grad()
