@@ -249,7 +249,8 @@ SOM_API int som_adam_devstep_f32(float* W, float* m, float* v, const float* g, i
 /* Data-parallel tail of the step: `g` is the UNSCALED gradient T @ Rbar_global (som_filter_ws_f32 with scale 1 on
  * the all-reduced accumulators) and `tail` the all-reduced 4-float tail of som_accumulate_packed_nchw_f32.  Applies
  * g * (float)(2 / numel), numel = D * n_global (F.mse_loss's mean, train_codebook.py:233-235) and the Adam rule of
- * som_adam_devstep_f32; writes loss = sse / numel to loss_out (device double, may be NULL).  Everything the host
+ * som_adam_devstep_f32; writes loss = sse / numel to loss_out (device double, may be NULL) -- except at n == 0,
+ * where only the step count advances and loss_out is left as it was.  Everything the host
  * would have to wait for stays on the device, so the whole step can be captured in a CUDA graph.
  * steps_done points to TWO int64: [0] the number of completed steps (t = steps_done[0] + 1 is used, then it is
  * incremented by the kernel itself), [1] a scratch word the kernel uses as its block-arrival counter: zero it once,
